@@ -33,6 +33,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True          # the tree may be read-only: no __pycache__ next to the sources it imports
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -492,11 +493,12 @@ def run_own(args, rank, world, local_rank):
         """n_steps steps (24 windows each) over the PCM already resident in each context's HBM buffer.  The windows are
         cut into equally sized generate calls exactly as the chunk scheduler cuts a job (`balanced_microbatch`: as few
         calls as keep every context busy, at most MB windows each); the contexts take the calls round-robin on their
-        own streams.  Returns per-context end events and the rows of the last call."""
+        own streams.  Returns per-context end events and the rows of every call, in call order."""
         ends, errs = [None] * len(engines), []
         n_win = n_steps * B
         mb = balanced_microbatch(n_win, len(engines), MB)
         calls = [min(mb, n_win - a) for a in range(0, n_win, mb)]
+        rows = [None] * len(calls)
 
         def work(ci):
             try:
@@ -504,7 +506,7 @@ def run_own(args, rank, world, local_rank):
                 with torch.cuda.stream(eng.stream) if eng.stream is not None else torch.cuda.stream(torch.cuda.current_stream()):
                     for k in range(ci, len(calls), len(engines)):
                         eng.features(calls[k])
-                        work.rows = eng.generate(calls[k])
+                        rows[k] = eng.generate(calls[k])
                     ev = torch.cuda.Event(enable_timing=True)
                     ev.record()
                     ends[ci] = ev
@@ -517,7 +519,7 @@ def run_own(args, rank, world, local_rank):
             t.join()
         if errs:
             raise errs[0]
-        return ends, getattr(work, "rows", None)
+        return ends, rows
 
     # ---- device-resident leg ("value")
     res_clips = clips * (MB // B)
@@ -564,7 +566,8 @@ def run_own(args, rank, world, local_rank):
         with torch.cuda.stream(engines[0].stream):
             single = engines[0].generate_from_pcm(clips)
     rows_ok = len(e2e_rows) == K * B and all(e2e_rows[i] == single[i % B] for i in range(len(e2e_rows)))
-    resident_ok = rows is not None and all(rows[i] == single[i % B] for i in range(len(rows)))
+    # window i of every call decodes clips[i % B] (the resident buffer holds the 24 clips repeated)
+    resident_ok = all(r[i] == single[i % B] for r in rows for i in range(len(r)))
 
     # ---- rooflines of the dominant kernels, measured live
     pk = peaks()
@@ -663,6 +666,9 @@ def run_own(args, rank, world, local_rank):
     if rank == 0:
         if world == 1 and not args.no_cpu_baseline:
             line["cpu_baseline"] = cpu_baseline_subprocess(args.reference_budget_s)
+        if args.dump_outputs:
+            # the timed region's last step: its last B windows, in the order the calls cover them
+            dump_outputs(args.dump_outputs, [r for call in rows for r in call][-B:])
         emit(line)
     if world > 1:
         dist.destroy_process_group()
@@ -807,6 +813,19 @@ def extra_config5(dev, pipe, dims, pk):
     return rec
 
 
+def dump_outputs(out_dir: str, rows) -> None:
+    """What the timed path's generate calls returned for the windows of its last step, so that two builds can be compared
+    output for output: token_ids.npy [windows, longest row] (-1 after the end of a row) and token_counts.npy [windows],
+    float32 (every id below 2**24 is exact)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    ids = np.full((len(rows), max((len(r) for r in rows), default=0)), -1, dtype=np.float32)
+    for b, r in enumerate(rows):
+        ids[b, :len(r)] = r
+    np.save(os.path.join(out_dir, "token_ids.npy"), ids)
+    np.save(os.path.join(out_dir, "token_counts.npy"), np.array([len(r) for r in rows], dtype=np.float32))
+
+
 _RESULT_FD = None
 
 
@@ -845,6 +864,9 @@ def main():
                     help="reference arm: skip the extra call in the reference's literal num_beams = 5 mode")
     ap.add_argument("--reference-budget-s", type=float, default=480.0,
                     help="reference arm: stop after the call that crosses this wall-clock budget (steps reports the calls made)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="own arm: after the timed steps, write the token ids of the last timed step's windows (rank 0) "
+                         "as DIR/*.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

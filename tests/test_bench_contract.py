@@ -41,3 +41,19 @@ def test_both_arms_name_the_same_workload_and_the_traffic_keys_exist():
     assert 1.0 <= t["decode_attn_kernel"] / (24 * 7.68e6) < 1.05
     assert 1.0 <= t["decode_attn_kernel_96_rows"] / (96 * 7.68e6) < 1.05
     json.dumps(t)
+
+
+def test_dump_outputs_writes_the_rows_as_float_arrays(tmp_path):
+    """--dump-outputs: one row of token ids per window of the last timed step, -1 after its end, plus the row lengths;
+    a run that cannot happen (no GPU) writes nothing."""
+    import numpy as np
+    r = _run(["--steps", "1", "--no-extras", "--no-cpu-baseline", "--dump-outputs", str(tmp_path / "none")])
+    assert r.returncode != 0 and not (tmp_path / "none").exists()
+    sys.path.insert(0, ROOT)
+    import bench
+    rows = [[50258, 50259, 50360, 50365, 51865, 50414], [50258, 50259, 50360]]
+    bench.dump_outputs(str(tmp_path / "out"), rows)
+    ids, counts = np.load(tmp_path / "out" / "token_ids.npy"), np.load(tmp_path / "out" / "token_counts.npy")
+    assert ids.dtype == counts.dtype == np.float32 and ids.shape == (2, 6) and counts.tolist() == [6, 3]
+    assert [row[:int(n)].astype(np.int64).tolist() for row, n in zip(ids, counts)] == rows
+    assert (ids[1, 3:] == -1).all()

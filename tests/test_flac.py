@@ -1,11 +1,8 @@
 """CPU tests of the native FLAC reader (csrc/flac.cpp behind tw_flac_decode; SURVEY.md §8f rank 2) against streams
 written by the test-side encoder (tests/flac_writer.py): bit-exact PCM for every subframe type, Rice variant, stereo
 mode, bit depth and block-size / sample-rate coding the format has, ragged last blocks, unknown stream length, an ID3
-prefix, trailing garbage; corrupted bytes are rejected through the frame CRCs and the STREAMINFO MD5.  When the
-reference tree is present, its own example input (ref:examples/Test1/ChrisAndAlexDiTest.flac) must decode to PCM whose
-MD5 equals the signature in its header."""
+prefix, trailing garbage; corrupted bytes are rejected through the frame CRCs and the STREAMINFO MD5."""
 import ctypes as C
-import os
 
 import numpy as np
 import pytest
@@ -110,15 +107,3 @@ def test_corruption_is_detected():
     assert lib.tw_flac_decode(None, 0, None, 0, C.byref(n)) != 0 and b"tw_flac_decode" in lib.tw_last_error()
     buf = np.frombuffer(b"fLaCxxxx", dtype=np.uint8)
     assert lib.tw_flac_decode(buf.ctypes.data_as(C.c_void_p), 8, None, 0, C.byref(n)) != 0
-
-
-REF_FLAC = "/root/reference/examples/Test1/ChrisAndAlexDiTest.flac"
-
-
-@pytest.mark.skipif(not os.path.exists(REF_FLAC), reason="reference tree not present (GPU box)")
-def test_reference_example_file_decodes_to_its_md5():
-    """The reference's own example input: 19.73 s, 192 kHz, mono, 16 bit, encoded by a real FLAC encoder (LPC
-    subframes, Rice partitions).  _read_flac verifies the STREAMINFO MD5 of the decoded samples."""
-    x, sr = _read_flac(open(REF_FLAC, "rb").read())
-    assert sr == 192000 and x.dtype == np.int16 and x.shape == (3788416, 1)
-    assert abs(x.shape[0] / sr - 19.74) < 0.02        # ref:examples/Test1/output.json ends at 19.74 s

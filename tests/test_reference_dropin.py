@@ -1,90 +1,32 @@
-"""CPU drop-in test at the reference's own entry point (SURVEY.md §8b / §8c recipe): when the reference tree is mounted
-(/root/reference — absent on the GPU box, where this test is skipped), its unmodified
-`vocalis.core.audio_pipeline.AudioProcessingPipeline.process_audio(path, task="transcribe")` runs with
-`transcription_model` set to a `B200WhisperPipeline` (the binding INTEGRATION.md §1 shows) and must return exactly what
-it returned with the transformers pipeline object (tests/golden/pipeline_tiny.json, `reference_process_audio_varied`).
-The GPU engines are replaced by the oracle scheduler of tests/test_pipeline_host_golden.py, so the comparison is exact and
-covers the reference-facing contract: call signature, keyword arguments the reference passes (chunk_length_s=60,
-batch_size, stride_length_s=5, generate_kwargs={"task": ...}, return_timestamps=True), the output dict it consumes
-(`text`, `chunks` -> its `segments`) and its error convention (exceptions become {"error": ...})."""
+"""CPU drop-in test at the reference's model construction (SURVEY.md §8b / §8c recipe): `install()` patches the
+`transformers.pipeline` factory, and the call the reference's `load_transcription_model` makes
+(`pipeline("automatic-speech-recognition", model=model_name, device=device, torch_dtype=...)`,
+ref:vocalis/core/audio_pipeline.py:187-200, quoted in turbo-whisper-workspace_b200/install.py) returns a
+`B200WhisperPipeline`.  Called the way the reference's `transcribe()` calls it (chunk_length_s=60, batch_size=32,
+stride_length_s=5, generate_kwargs={"task": ...}, return_timestamps=True; ref:vocalis/core/audio_pipeline.py:351-358),
+that object must return the text and segments the reference's own `process_audio` returned with the transformers
+pipeline object (stored in tests/golden/pipeline_tiny.json, `reference_process_audio_varied`, by
+tests/golden/make_golden.py).  The GPU engines are replaced by the oracle scheduler of tests/test_pipeline_host_golden.py,
+so the comparison is exact."""
 import json
 import os
-import sys
-import types
 
 import numpy as np
-import pytest
+import torch
 
 import helpers
 from test_pipeline_host_golden import GOLD, OracleScheduler
 from turbo_whisper_workspace_b200.config import WhisperDims
 from turbo_whisper_workspace_b200.pipeline import B200WhisperPipeline
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "vocalis")), reason="reference tree not mounted")
 
-
-@pytest.fixture(scope="module")
-def ap():
-    # import what transformers resolves lazily BEFORE stubbing the optional audio modules (its availability probes
-    # call importlib.util.find_spec on them)
-    import transformers
-    from transformers import pipeline, WhisperForConditionalGeneration, WhisperTokenizer  # noqa: F401
-    import importlib.machinery
-    for m in ("librosa", "soundfile", "sherpa_onnx", "pydub"):
-        if m not in sys.modules:
-            stub = types.ModuleType(m)
-            stub.__spec__ = importlib.machinery.ModuleSpec(m, None)
-            sys.modules[m] = stub
-    if not hasattr(sys.modules["pydub"], "AudioSegment"):
-        sys.modules["pydub"].AudioSegment = type("AudioSegment", (), {})
-    if REF not in sys.path:
-        sys.path.insert(0, REF)
-    import vocalis.core.audio_pipeline as mod
-    mod.LLM_AVAILABLE = False
-    return mod
-
-
-def test_process_audio_with_the_b200_pipeline_object(ap, tmp_path):
-    gold = json.load(open(os.path.join(GOLD, "pipeline_tiny.json")))["reference_process_audio_varied"]
-    pcm = np.concatenate([helpers.synth_clip(0), helpers.synth_clip(1, kind="mod"),
-                          helpers.synth_clip(2, seconds=11.3, kind="mod")])
-    wav = tmp_path / "golden_71s.wav"
-    helpers.write_wav16(wav, pcm)
-    pipe = B200WhisperPipeline(None, WhisperDims(**helpers.TINY), helpers.build_tokenizer(),
-                               scheduler=OracleScheduler("varied"))
-    seen = {}
-    call = pipe.__call__
-
-    class Spy:          # records the keyword arguments the reference passes (ref:vocalis/core/audio_pipeline.py:351-358)
-        def __call__(self, inputs, **kw):
-            seen.update(kw, inputs=inputs)
-            return call(inputs, **kw)
-    p = ap.AudioProcessingPipeline()
-    p.transcription_model = Spy()
-    p.diarize = lambda *a, **k: []
-    res = p.process_audio(str(wav), task="transcribe")
-    assert "error" not in res, res
-    assert sorted(res.keys()) == gold["keys"]
-    assert res["text"] == gold["text"]
-    assert [{"timestamp": list(c["timestamp"]), "text": c["text"]} for c in res["segments"]] == gold["segments"]
-    assert seen["inputs"] == str(wav) and seen["chunk_length_s"] == 60 and seen["stride_length_s"] == 5
-    assert seen["generate_kwargs"] == {"task": "transcribe"} and seen["return_timestamps"] is True
-    assert seen["batch_size"] in (32, 512)
-
-    # error convention: an exception inside the model call becomes the reference's {"error": ...} dict
-    class Boom:
-        def __call__(self, *a, **k):
-            raise RuntimeError("engine failure")
-    p.transcription_model = Boom()
-    res = p.process_audio(str(wav), task="transcribe")
-    assert "error" in res and "engine failure" in res["error"]
-
-
-def test_zero_touch_install_through_load_transcription_model(ap, tmp_path, monkeypatch):
-    """INTEGRATION.md §1 option (ii): `install()` patches `transformers.pipeline`, and the reference's UNMODIFIED
-    `load_transcription_model` (ref:vocalis/core/audio_pipeline.py:171-208) — reached through `process_audio` ->
-    `transcribe` with no model loaded — ends up holding the B200 pipeline object; other tasks are forwarded."""
+def test_zero_touch_install_through_load_transcription_model(tmp_path, monkeypatch):
+    """INTEGRATION.md §1 option (ii): with `install()` in place, the reference's model construction (default model name
+    "openai/whisper-large-v3") yields the B200 pipeline object, other tasks / models are forwarded to the original factory,
+    and `uninstall()` puts the original back."""
+    # importing `pipeline` from transformers the first time replaces its lazy top-level module in sys.modules: do it
+    # before binding the module object that gets patched
+    from transformers import pipeline  # noqa: F401
     import transformers
     import turbo_whisper_workspace_b200.install as twb
     gold = json.load(open(os.path.join(GOLD, "pipeline_tiny.json")))["reference_process_audio_varied"]
@@ -103,21 +45,21 @@ def test_zero_touch_install_through_load_transcription_model(ap, tmp_path, monke
     def builder(hf_model, tokenizer):
         assert hf_model == "hf-model-stand-in"
         return B200WhisperPipeline(None, WhisperDims(**helpers.TINY), tokenizer, scheduler=OracleScheduler("varied"))
-    monkeypatch.setitem(ap._PIPELINE_CACHE, "transcription_model", None)
     twb.install(devices=["cuda:0"], loader=loader, builder=builder)
     try:
         assert transformers.pipeline("text-classification", model="bert") == "lib" and forwarded == [("text-classification", "bert")]
         assert transformers.pipeline("automatic-speech-recognition", model="facebook/wav2vec2-base") == "lib"
-        p = ap.AudioProcessingPipeline()
-        assert p.transcription_model is None
-        p.diarize = lambda *a, **k: []
-        res = p.process_audio(str(wav), task="transcribe")
-        assert "error" not in res, res
-        assert isinstance(p.transcription_model, B200WhisperPipeline)
-        assert ap._PIPELINE_CACHE["transcription_model"] is p.transcription_model
+        # the reference's load_transcription_model: `from transformers import pipeline` at call time, then this call
+        from transformers import pipeline
+        model = pipeline("automatic-speech-recognition", model="openai/whisper-large-v3", device="cpu",
+                         torch_dtype=torch.float32)
+        assert isinstance(model, B200WhisperPipeline)
         assert loaded == ["openai/whisper-large-v3"]            # the reference's default model name
+        # the reference's transcribe() call
+        res = model(str(wav), chunk_length_s=60, batch_size=32, stride_length_s=5,
+                    generate_kwargs={"task": "transcribe"}, return_timestamps=True)
         assert res["text"] == gold["text"]
-        assert [{"timestamp": list(c["timestamp"]), "text": c["text"]} for c in res["segments"]] == gold["segments"]
+        assert [{"timestamp": list(c["timestamp"]), "text": c["text"]} for c in res["chunks"]] == gold["segments"]
     finally:
         twb.uninstall()
     assert transformers.pipeline("x", model="y") == "lib"       # the original factory is back
