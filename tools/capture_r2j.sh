@@ -6,7 +6,3 @@ step() { echo "== $1" >&2; }
 step "decode probe: stats late (default) vs early"
 python tools/probe_decode_tail.py 2>/dev/null | grep "^{" | sed 's/^{/{"stats": "late", /' | tee gpurun_out/${T}_decode_probe.jsonl
 TWB200_LIB=$PWD/turbo-whisper-workspace_b200/variants/libtwb200_lnearly.so python tools/probe_decode_tail.py 2>/dev/null | grep "^{" | sed 's/^{/{"stats": "early", /' | tee -a gpurun_out/${T}_decode_probe.jsonl
-step "attention: default vs v3 (+ parity test with v3)"
-timeout 120 python tools/bench_kernels.py 24 attention 2>/dev/null | grep '^{' | sed 's/^{/{"variant": "default", /' | tee gpurun_out/${T}_attn.jsonl | cut -c1-330
-TWB200_ATTN=v3 timeout 120 python tools/bench_kernels.py 24 attention 2>&1 | grep -E '^\{|rror' | sed 's/^{/{"variant": "v3", /' | tee -a gpurun_out/${T}_attn.jsonl | cut -c1-330
-TWB200_ATTN=v3 timeout 300 python -m pytest tests/test_gpu_ops.py -m gpu -x -q -k "attention" 2>&1 | tail -3

@@ -16,7 +16,3 @@ print(json.dumps({'ln':'$mode','value':round(d['value'],1),'e2e':round(d['e2e'][
   done
 done
 unset TWB200_NO_LN_FOLD
-echo "== attention persist" >&2
-timeout 120 python tools/bench_kernels.py 24 attention 2>/dev/null | grep '^{' | sed 's/^{/{"variant": "default", /' | tee gpurun_out/${T}_attn.jsonl | cut -c1-200
-TWB200_ATTN=persist timeout 120 python tools/bench_kernels.py 24 attention 2>&1 | grep -E '^\{|rror' | sed 's/^{/{"variant": "persist", /' | tee -a gpurun_out/${T}_attn.jsonl | cut -c1-330
-TWB200_ATTN=persist timeout 300 python -m pytest tests/test_gpu_ops.py -m gpu -x -q -k "attention" 2>&1 | tail -3

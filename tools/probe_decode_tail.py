@@ -1,6 +1,4 @@
-"""Decode-step time of one context alone (graph replays, B = 24, large-v3-turbo and large-v3 dims).  Run twice:
-plain, and with TWB200_PROBE_NO_LN=1 (LayerNorm tails skipped: WRONG results, timing only) to bound what a
-restructured LayerNorm could save."""
+"""Decode-step time of one context alone (graph replays, B = 24, large-v3-turbo and large-v3 dims)."""
 import json, os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -18,7 +16,7 @@ for name, dims, B in cases:
     eng.features(B)
     eng.encode(B)
     us, nbytes = bench.decode_step_probe(eng, B)
-    print(json.dumps({"model": name, "B": B, "no_ln_probe": bool(os.environ.get("TWB200_PROBE_NO_LN")), "us_per_step": round(us, 1),
+    print(json.dumps({"model": name, "B": B, "us_per_step": round(us, 1),
                       "floor_us": round(nbytes / 6458.7e3, 1), "launches": eng.launches_per_step}), flush=True)
     del eng
     torch.cuda.empty_cache()

@@ -6,57 +6,47 @@
 // which is exact for a power of two).
 //
 // Input is the fused QKV projection output [B*T, 3*D] bf16 (q | k | v, head h at columns 64h..).
-// One CTA = one (batch, head) and NT 128-query tiles (template parameter; default NT = 1: 320 threads, 256 TMEM
-// columns, TWO independent CTAs per SM that overlap each other's prologue / epilogue; NT = 2: 576 threads, all 512
-// columns, K/V tiles shared by both query tiles, one CTA per SM).  Warp 0 TMA producer, warp 1 MMA issuer (whole
-// warp converged, one elected lane issues from uniform registers), 8 softmax warps per tile with TWO threads per
-// query row (64 keys each).
-//   S  = Q K_j^T      tcgen05.mma 128x128x64 (SS)  -> TMEM S_g (128 fp32 columns)
-//   P  = exp2(S - m)  softmax threads: S_g -> registers -> bf16 pairs -> TMEM P_g (64 columns)
-//   O += P V_j        tcgen05.mma 128x64x128 (TS: A = P_g from tensor memory, B = V_j MN-major straight from its
-//                     TMA tile) accumulating in TMEM O_g across all kv tiles
+// One CTA = one (batch, head) and one 128-query tile: 320 threads, 256 TMEM columns, TWO independent CTAs per SM
+// that overlap each other's prologue / epilogue.  Warp 0 TMA producer, warp 1 MMA issuer (whole warp converged,
+// one elected lane issues from uniform registers), 8 softmax warps with TWO threads per query row (64 keys each).
+//   S  = Q K_j^T      tcgen05.mma 128x128x64 (SS)  -> TMEM S (128 fp32 columns)
+//   P  = exp2(S - m)  softmax threads: S -> registers -> bf16 pairs -> TMEM P (64 columns)
+//   O += P V_j        tcgen05.mma 128x64x128 (TS: A = P from tensor memory, B = V_j MN-major straight from its
+//                     TMA tile) accumulating in TMEM O across all kv tiles
 // The exponentials are the co-limiter of this head size (MUFU: 16 results/clk/SM = 2048 cycles per kv step
-// for both tiles, the MMAs need ~600), so the schedule is built around the softmax warps:
-//   * S_g is released (s_free) as soon as every thread has copied its keys to registers, so S_g(j+1) is
-//     computed WHILE softmax(j) runs; P has its own TMEM columns, so PV_g(j) runs while softmax(j+1) runs,
-//     and the wait for PV_g(j-1) sits after the exponentials, just before P_g is overwritten;
+// for the two CTAs of an SM, the MMAs need ~600), so the schedule is built around the softmax warps:
+//   * S is released (s_free) as soon as every thread has copied its keys to registers, so S(j+1) is
+//     computed WHILE softmax(j) runs; P has its own TMEM columns, so PV(j) runs while softmax(j+1) runs,
+//     and the wait for PV(j-1) sits after the exponentials, just before P is overwritten;
 //   * four softmax warps per SM sub-partition: a warp issues in order and each MUFU.EX2 holds the XU port for
 //     8 cycles, so with fewer warps the MUFU idles during every load / row-max / store phase;
 //   * optionally (ATTN_POLY_EVERY) a share of the exponentials runs as a degree-3 polynomial on the FMA pipe;
 //   * scale/shift FMA and row-sum ADD are packed f32x2; row sums stay in registers; the softmax reference
 //     point only moves when the running maximum grows by more than 2^8 (lazy rescale of O in TMEM).
-// TMEM per tile: S (128 fp32 columns) | P (64) | O (64); 80 KB smem per CTA at NT = 1.
+// TMEM: S (128 fp32 columns) | P (64) | O (64); 80 KB of smem tiles per CTA.
 // Measured history (B=24, T=1500, H=20, per layer): 0.61 ms with P aliased on S and one thread per row,
-// 0.50-0.52 ms with two threads per row (NT = 2), 0.46-0.49 ms with NT = 1 / two CTAs per SM (torch SDPA 0.35 ms); tools/probes/ holds the MUFU / instruction-mix probes behind the numbers.
-#include <cstdlib>
+// 0.50-0.52 ms with two threads per row and two query tiles per CTA, 0.46-0.49 ms with one tile / two CTAs per SM
+// (torch SDPA 0.35 ms); tools/probes/ holds the MUFU / instruction-mix probes behind the numbers.  DESIGN.md §3 lists
+// the layouts tried since and rejected.
 #include "common.cuh"
 #include "twb200_internal.h"
 
 namespace tw {
 namespace attn {
 
-constexpr int BQ = 128;   // query rows per tile; a CTA owns two tiles (A, B) that ping-pong
+constexpr int BQ = 128;   // query rows per CTA
 constexpr int BKV = 128;  // keys per iteration
 constexpr int DH = 64;
-constexpr int GROUP_THREADS = 256;         // softmax threads per query tile: two per row (64 keys each)
+constexpr int GROUP_THREADS = 256;         // softmax threads: two per row (64 keys each)
+constexpr int NUM_THREADS = 64 + GROUP_THREADS;   // TMA warp, MMA warp, 8 softmax warps
 constexpr int TILE_BYTES = 128 * DH * 2;   // 16 KB: Q, K, V tiles and each half of P
-// A CTA owns NT query tiles (template parameter): NT = 2 -> 576 threads, all 512 TMEM columns, K/V tiles shared by both
-// query tiles, one CTA per SM; NT = 1 -> 320 threads, 256 TMEM columns, two independent CTAs per SM (each overlaps the
-// other's prologue / epilogue).  TMEM map: S_g at g*128 (fp32 scores) | P_g at NT*128 + g*64 (bf16 probabilities, two
-// keys per column) | O_g at NT*192 + g*64 (fp32 output accumulators).  smem tiles: Q_0..Q_{NT-1} | K0 K1 | V0 V1.
+// TMEM map (256 columns): S at 0 (fp32 scores) | P at 128 (bf16 probabilities, two keys per column) | O at 192 (fp32
+// output accumulators).  smem: Q | K0 K1 | V0 V1 | exchange | barriers.
 // P never touches shared memory: tcgen05.mma reads it from tensor memory.
-constexpr int XCH_BYTES = 2 * 2 * 2 * 128 * 4;   // row-max / row-sum exchange between the two threads of a row: [parity][tile][half][row]
-constexpr int smem_bytes(int nt) { return (nt + 4) * TILE_BYTES + XCH_BYTES + 1024 + 256; }
-// -DATTN_MERGED_ISSUE=1: ONE warp issues both the TMA loads and the MMAs (both are single-lane jobs driven by the same
-// event loop), a CTA is then 9 warps.  Measured (profiles/r2e_attn_variants.jsonl): 0.464 ms vs 0.466 ms for the default
-// two-warp layout — no gain, because ptxas derives the register cap of __launch_bounds__(288, 2) as for 10 warps (96
-// registers either way; the ~90 bytes of loop spills stay), and stating the cap directly (__maxnreg__(112), which cannot
-// be combined with __launch_bounds__) loses the second CTA per SM: 0.636 ms.  Kept as a build option.
-#ifndef ATTN_MERGED_ISSUE
-#define ATTN_MERGED_ISSUE 0
-#endif
-constexpr int ISSUE_WARPS = ATTN_MERGED_ISSUE ? 1 : 2;
-constexpr int num_threads(int nt) { return 32 * ISSUE_WARPS + nt * GROUP_THREADS; }   // issue warp(s), 8 softmax warps per tile
+constexpr int TMEM_COLS = 256;
+constexpr int S_COL = 0, P_COL = 128, O_COL = 192;
+constexpr int XCH_BYTES = 2 * 2 * 2 * 128 * 4;   // row-max / row-sum exchange between the two threads of a row: [parity][grp][half][row]
+constexpr int SMEM_BYTES = 5 * TILE_BYTES + XCH_BYTES + 1024 + 256;
 constexpr float LOG2E = 1.4426950408889634f;
 // One pair of exponentials in POLY_EVERY takes the FMA-pipe polynomial path (1000 = none).  Measured on one box:
 // none 0.526 ms, every 4th 0.476 ms, every 3rd 0.470 ms, every 2nd 0.484 ms per layer.  It is OFF by default: the
@@ -68,22 +58,14 @@ constexpr float LOG2E = 1.4426950408889634f;
 #endif
 constexpr int POLY_EVERY = ATTN_POLY_EVERY;
 
-// single-instruction exp2 (MUFU.EX2, flush-to-zero): arguments here are <= 0, so the slow path of exp2f()
-// (denormal-input scaling, 4 extra instructions per element) is never needed
-// two exponentials per MUFU op on bf16 pairs: the result is directly the packed bf16 P operand.  The argument
-// is rounded to bf16 first (|error| <= 2^-9 |x| in the exponent, below the bf16 rounding of P itself for the
-// entries that carry weight).
-TW_DEVINL uint32_t ex2_bf16x2(uint32_t x) {
-    uint32_t y;
-    asm("ex2.approx.ftz.bf16x2 %0, %1;" : "=r"(y) : "r"(x));
-    return y;
-}
 // three-input maximum (FMNMX3, sm_100): halves the instruction count of the row-maximum pass
 TW_DEVINL float max3(float a, float b, float c) {
     float d;
     asm("max.f32 %0, %1, %2, %3;" : "=f"(d) : "f"(a), "f"(b), "f"(c));
     return d;
 }
+// single-instruction exp2 (MUFU.EX2, flush-to-zero): arguments here are <= 0, so the slow path of exp2f()
+// (denormal-input scaling, 4 extra instructions per element) is never needed
 TW_DEVINL float ex2_approx(float x) {
     float y;
     asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
@@ -130,42 +112,38 @@ TW_DEVINL void exp2_poly_x2(uint64_t a2, float& p0, float& p1) {
     p1 = __int_as_float(__float_as_int(q1) + (__float_as_int(r1) << 23));
 }
 
-// named barriers 1 / 2: the MUFU turn of tile A / B (see the softmax loop)
+// named barriers 1-4: the two softmax warps that share a TMEM lane quarter (see the softmax loop)
 TW_DEVINL void named_bar_sync(int id, int count) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(count) : "memory"); }
-TW_DEVINL void named_bar_arrive(int id, int count) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(count) : "memory"); }
 
 struct Params {
     int T, H, D;        // sequence length, heads, model width (H*64)
     long long out_ld;   // elements
     __nv_bfloat16* out;
-    long long* dbg;   // optional clock64 trace of CTA (0,0,0): [0..63] MMA thread, [64..] softmax A row 0
+    long long* dbg;   // optional clock64 trace of CTA (0,0,0): [0..63] MMA thread, [64..] softmax row 0
 };
 
-template <int NT>
-__global__ void __launch_bounds__(num_threads(NT), NT == 1 ? 2 : 1)
+__global__ void __launch_bounds__(NUM_THREADS, 2)
 attention_enc_kernel(const __grid_constant__ CUtensorMap tmQKV, const Params p) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-    constexpr int TMEM_COLS = NT * 256;
-    constexpr int S_COL = 0, P_COL = NT * 128, O_COL = NT * 192;
-    uint8_t* sQ = smem;                              // NT tiles
-    uint8_t* sK = smem + NT * TILE_BYTES;            // 2 stages
-    uint8_t* sV = smem + (NT + 2) * TILE_BYTES;      // 2 stages
-    float* xch = reinterpret_cast<float*>(smem + (NT + 4) * TILE_BYTES);
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + (NT + 4) * TILE_BYTES + XCH_BYTES);
+    uint8_t* sQ = smem;
+    uint8_t* sK = smem + TILE_BYTES;                 // 2 stages
+    uint8_t* sV = smem + 3 * TILE_BYTES;             // 2 stages
+    float* xch = reinterpret_cast<float*>(smem + 5 * TILE_BYTES);
+    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + 5 * TILE_BYTES + XCH_BYTES);
     uint64_t* q_full = bars + 0;
     uint64_t* k_full = bars + 1;   // [2]
     uint64_t* k_empty = bars + 3;  // [2]
     uint64_t* v_full = bars + 5;   // [2]
     uint64_t* v_empty = bars + 7;  // [2]
-    uint64_t* s_full = bars + 9;   // [2] per group
-    uint64_t* p_full = bars + 11;  // [2] per group
-    uint64_t* o_full = bars + 13;  // [2] per group
-    uint64_t* s_free = bars + 15;  // [2] per group: every thread of the group holds its S row in registers
+    uint64_t* s_full = bars + 9;   // [2] indexed by grp (see the softmax warps)
+    uint64_t* p_full = bars + 11;  // [2] indexed by grp
+    uint64_t* o_full = bars + 13;  // [2] indexed by grp
+    uint64_t* s_free = bars + 15;  // [2] indexed by grp: every softmax thread holds its S row in registers
     uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(bars + 17);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int q0 = blockIdx.x * (NT * BQ), h = blockIdx.y, b = blockIdx.z;
+    const int q0 = blockIdx.x * BQ, h = blockIdx.y, b = blockIdx.z;
     const int nkv = (p.T + BKV - 1) / BKV;
     const bool trace = p.dbg && blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0;
     int ti = 0;
@@ -186,8 +164,7 @@ attention_enc_kernel(const __grid_constant__ CUtensorMap tmQKV, const Params p) 
         }
         fence_barrier_init();
     }
-    constexpr int MMA_WARP = ISSUE_WARPS - 1;   // the warp that issues the MMAs (and owns the TMEM allocation)
-    if (warp == MMA_WARP) {
+    if (warp == 1) {   // the MMA warp owns the TMEM allocation
         tmem_alloc(tmem_ptr_smem, TMEM_COLS);
         tmem_relinquish();
     }
@@ -196,11 +173,10 @@ attention_enc_kernel(const __grid_constant__ CUtensorMap tmQKV, const Params p) 
     tcgen05_fence_after();
     const uint32_t tmem_base = *tmem_ptr_smem;
 
-    if (!ATTN_MERGED_ISSUE && warp == 0) {
+    if (warp == 0) {
         if (lane == 0) {
-            mbar_arrive_expect_tx(q_full, NT * TILE_BYTES);
-#pragma unroll
-            for (int g = 0; g < NT; ++g) tma_load_3d(&tmQKV, q_full, sQ + g * TILE_BYTES, h * DH, q0 + g * BQ, b);
+            mbar_arrive_expect_tx(q_full, TILE_BYTES);
+            tma_load_3d(&tmQKV, q_full, sQ, h * DH, q0, b);
             for (int j = 0; j < nkv; ++j) {
                 const int s = j & 1;
                 const uint32_t ph = (j >> 1) & 1;
@@ -212,37 +188,37 @@ attention_enc_kernel(const __grid_constant__ CUtensorMap tmQKV, const Params p) 
                 tma_load_3d(&tmQKV, &v_full[s], sV + s * TILE_BYTES, 2 * p.D + h * DH, j * BKV, b);
             }
         }
-    } else if (warp == MMA_WARP) {
+    } else if (warp == 1) {
         // The whole warp runs this loop converged and one elected lane issues: every operand of tcgen05.mma is
         // then warp-uniform (uniform registers), so an issue costs ~3 instructions.  (With a single divergent
         // thread and descriptor arrays in local memory each issue cost ~110 cycles - more than the 32-64
         // cycles the MMAs themselves last - and the issuing thread, not the tensor pipe or the MUFU, set the pace.)
         constexpr uint32_t idesc_s = umma_idesc_bf16(BQ, BKV, 0, 0);
         constexpr uint32_t idesc_o = umma_idesc_bf16(BQ, DH, 0, 1);  // B = V is MN-major
-        const uint64_t dq0 = umma_desc_sw128(smem_u32(sQ), 16, 1024);
+        const uint64_t dq = umma_desc_sw128(smem_u32(sQ), 16, 1024);
         const uint64_t dk0 = umma_desc_sw128(smem_u32(sK), 16, 1024);
         // V: one 64-wide MN atom (the head dim), 16 key rows x 128 B per K step, 8-row groups 1024 B apart
         const uint64_t dv0 = umma_desc_sw128(smem_u32(sV), 1024, 1024);
         constexpr uint64_t TILE_D = TILE_BYTES >> 4;   // descriptor address field is in 16-byte units
-        auto issue_s = [&](int g, int j) {   // S_g = Q_g K_j^T
-            const uint64_t a = dq0 + (uint64_t)g * TILE_D, bd = dk0 + (uint64_t)(j & 1) * TILE_D;
+        auto issue_s = [&](int j) {   // S = Q K_j^T
+            const uint64_t bd = dk0 + (uint64_t)(j & 1) * TILE_D;
             if (elect_one_sync()) {
 #pragma unroll
                 for (int k = 0; k < DH / 16; ++k)
-                    tcgen05_mma_f16(tmem_base + S_COL + g * BKV, a + k * 2, bd + k * 2, idesc_s, k != 0);
-                tcgen05_commit(&s_full[g]);
+                    tcgen05_mma_f16(tmem_base + S_COL, dq + k * 2, bd + k * 2, idesc_s, k != 0);
+                tcgen05_commit(s_full);
             }
             __syncwarp();
         };
-        auto issue_pv = [&](int g, int j) {  // O_g += P_g V_j   (A = P from TMEM)
+        auto issue_pv = [&](int j) {  // O += P V_j   (A = P from TMEM)
             const uint64_t bd = dv0 + (uint64_t)(j & 1) * TILE_D;
-            const uint32_t p_tmem = tmem_base + P_COL + g * (BKV / 2);
+            const uint32_t p_tmem = tmem_base + P_COL;
             const uint32_t acc0 = j != 0;
             if (elect_one_sync()) {
 #pragma unroll
                 for (int k = 0; k < BKV / 16; ++k)
-                    tcgen05_mma_f16_ts(tmem_base + O_COL + g * DH, p_tmem + k * 8, bd + k * 128, idesc_o, k != 0 ? 1u : acc0);
-                tcgen05_commit(&o_full[g]);
+                    tcgen05_mma_f16_ts(tmem_base + O_COL, p_tmem + k * 8, bd + k * 128, idesc_o, k != 0 ? 1u : acc0);
+                tcgen05_commit(o_full);
             }
             __syncwarp();
         };
@@ -250,97 +226,53 @@ attention_enc_kernel(const __grid_constant__ CUtensorMap tmQKV, const Params p) 
             if (elect_one_sync()) tcgen05_commit(bar);
             __syncwarp();
         };
-        // merged layout: this warp is also the TMA producer.  Q and the first two K / V stages go out at once; later
-        // stages are (re)filled from the event loop below as soon as their consumers release them.
-        int jk = 0, jv = 0;   // next K / V tile to load
-        auto load_k = [&](int j) {
-            if (elect_one_sync()) {
-                mbar_arrive_expect_tx(&k_full[j & 1], TILE_BYTES);
-                tma_load_3d(&tmQKV, &k_full[j & 1], sK + (j & 1) * TILE_BYTES, p.D + h * DH, j * BKV, b);
-            }
-            __syncwarp();
-        };
-        auto load_v = [&](int j) {
-            if (elect_one_sync()) {
-                mbar_arrive_expect_tx(&v_full[j & 1], TILE_BYTES);
-                tma_load_3d(&tmQKV, &v_full[j & 1], sV + (j & 1) * TILE_BYTES, 2 * p.D + h * DH, j * BKV, b);
-            }
-            __syncwarp();
-        };
-        if (ATTN_MERGED_ISSUE) {
-            if (elect_one_sync()) {
-                mbar_arrive_expect_tx(q_full, NT * TILE_BYTES);
-#pragma unroll
-                for (int g = 0; g < NT; ++g) tma_load_3d(&tmQKV, q_full, sQ + g * TILE_BYTES, h * DH, q0 + g * BQ, b);
-            }
-            __syncwarp();
-            for (; jk < 2 && jk < nkv; ++jk) load_k(jk);
-            for (; jv < 2 && jv < nkv; ++jv) load_v(jv);
-        }
         if (lane == 0) TRACE(0);
         mbar_wait(q_full, 0);
         mbar_wait(&k_full[0], 0);
         if (lane == 0) TRACE(0);
         tcgen05_fence_after();
-#pragma unroll
-        for (int g = 0; g < NT; ++g) issue_s(g, 0);
+        issue_s(0);
         release(&k_empty[0]);
-        // Event loop over the things that can become issuable, polled without blocking so that no tile ever delays
-        // another:  S_g(j) once the group has copied S_g(j-1) to registers (s_free) and K_j has landed;  PV_g(j)
-        // once P_g(j) is stored (p_full) and V_j has landed.  A K/V stage is handed back to the producer by
-        // whichever tile issues the last MMA that reads it.
-        int js[NT], jp[NT];   // next S / PV index per tile (constant indices after unrolling: registers)
-#pragma unroll
-        for (int g = 0; g < NT; ++g) { js[g] = 1; jp[g] = 0; }
-        auto pending = [&]() { bool any = false;
-#pragma unroll
-            for (int g = 0; g < NT; ++g) any = any || jp[g] < nkv;
-            return any; };
+        // Event loop over the two things that can become issuable, polled without blocking so that neither delays
+        // the other:  S(j) once the softmax threads have copied S(j-1) to registers (s_free) and K_j has landed;
+        // PV(j) once P(j) is stored (p_full) and V_j has landed.  Each MMA hands its K / V stage back to the producer.
+        int js = 1, jp = 0;   // next S / PV index
+        // The exit test is a one-trip loop on purpose.  Written as a plain `while (jp < nkv)`, the loop is compiled with
+        // nkv reloaded from a local-memory spill slot at loop entry (spill loads 96 -> 100 bytes); this form compiles to
+        // the instructions the kernel was measured with.
+        auto pending = [&]() {
+            bool more = false;
+            for (int once = 0; once < 1; ++once) more = jp < nkv;
+            return more;
+        };
         while (pending()) {
-            if (ATTN_MERGED_ISSUE) {
-                // a stage is free again once the MMAs that read its previous tile have completed (k_empty / v_empty are
-                // armed by tcgen05.commit); tile j reuses the stage of tile j - 2
-                if (jk < nkv && __any_sync(0xffffffffu, mbar_test_wait(&k_empty[jk & 1], ((jk >> 1) & 1) ^ 1))) { load_k(jk); ++jk; }
-                if (jv < nkv && __any_sync(0xffffffffu, mbar_test_wait(&v_empty[jv & 1], ((jv >> 1) & 1) ^ 1))) { load_v(jv); ++jv; }
+            if (js < nkv && __any_sync(0xffffffffu, mbar_test_wait(s_free, (js - 1) & 1) &&
+                                                       mbar_test_wait(&k_full[js & 1], (js >> 1) & 1))) {
+                tcgen05_fence_after();
+                issue_s(js);
+                release(&k_empty[js & 1]);
+                ++js;
             }
-#pragma unroll
-            for (int g = 0; g < NT; ++g) {
-                // (K_j / V_j are part of the non-blocking condition: a tile that runs two kv tiles ahead of the other
-                // needs a stage the slower tile has not released yet, and only this warp can make it release it)
-                if (js[g] < nkv && __any_sync(0xffffffffu, mbar_test_wait(&s_free[g], (js[g] - 1) & 1) &&
-                                                               mbar_test_wait(&k_full[js[g] & 1], (js[g] >> 1) & 1))) {
-                    const int j = js[g];
-                    tcgen05_fence_after();
-                    issue_s(g, j);
-                    bool last_reader = true;
-#pragma unroll
-                    for (int o = 0; o < NT; ++o) if (o != g) last_reader = last_reader && js[o] > j;
-                    if (last_reader) release(&k_empty[j & 1]);
-                    js[g] = j + 1;
-                }
-                if (jp[g] < nkv && __any_sync(0xffffffffu, mbar_test_wait(&p_full[g], jp[g] & 1) &&
-                                                               mbar_test_wait(&v_full[jp[g] & 1], (jp[g] >> 1) & 1))) {
-                    const int j = jp[g];
-                    tcgen05_fence_after();
-                    issue_pv(g, j);
-                    bool last_reader = true;
-#pragma unroll
-                    for (int o = 0; o < NT; ++o) if (o != g) last_reader = last_reader && jp[o] > j;
-                    if (last_reader) release(&v_empty[j & 1]);
-                    jp[g] = j + 1;
-                }
+            if (__any_sync(0xffffffffu, mbar_test_wait(p_full, jp & 1) && mbar_test_wait(&v_full[jp & 1], (jp >> 1) & 1))) {
+                tcgen05_fence_after();
+                issue_pv(jp);
+                release(&v_empty[jp & 1]);
+                ++jp;
             }
             // (backing off with nanosleep when nothing fired was measured slower at every setting: the latency of
             // picking up an event is on the critical path, the issue slots this warp burns are not)
         }
     } else {
         // Two threads per query row (64 keys each): four softmax warps per SM sub-partition.  A warp issues in order
-        // and every MUFU.EX2 holds the XU port for 8 cycles, so one warp per tile per sub-partition leaves the MUFU
-        // idle during its TMEM load / row-max / store phases and the FMA pipe idle during its exp phase; with four
-        // warps in different phases both stay busy.  Warps w and w+4 of a tile share a TMEM lane quarter (w % 4) and
-        // split the columns; they agree on the row maximum through shared memory (named barrier per warp pair).
-        const int ws = warp - ISSUE_WARPS;  // softmax warp index
-        const int grp = ws >> 3;            // 0: tile A, 1: tile B
+        // and every MUFU.EX2 holds the XU port for 8 cycles, so one warp per sub-partition leaves the MUFU idle
+        // during its TMEM load / row-max / store phases and the FMA pipe idle during its exp phase; with four
+        // warps in different phases both stay busy.  Warps w and w+4 share a TMEM lane quarter (w % 4) and split the
+        // columns; they agree on the row maximum through shared memory (named barrier per warp pair).
+        const int ws = warp - 2;            // softmax warp index
+        // grp is 0 for all eight softmax warps, but the compiler cannot prove it (it does not bound the warp index).
+        // Folding it away shifts this kernel's register allocation (spills 52/96 -> 56/116 bytes stored/loaded), so
+        // it stays a run-time value until a change to the softmax pipeline measures that.
+        const int grp = ws >> 3;
         const int quarter = warp & 3;       // TMEM lane quarter this warp may access (hardware: warp id % 4)
         const int hf = (ws >> 2) & 1;       // which 64 keys of the tile (and which 32 output columns) this thread owns
         const int r = quarter * 32 + lane;  // query row within the tile == TMEM lane
@@ -371,7 +303,7 @@ attention_enc_kernel(const __grid_constant__ CUtensorMap tmQKV, const Params p) 
                 tmem_ld_32x32b_x16(tmem_base + t_lane + s_col + c * 16, *reinterpret_cast<uint32_t(*)[16]>(&v[c * 16]));
             tmem_ld_wait();
             tcgen05_fence_before();
-            mbar_arrive(&s_free[grp]);          // the tensor core may now overwrite S_g with S_g(j+1)
+            mbar_arrive(&s_free[grp]);          // the tensor core may now overwrite S with S(j+1)
             if (tr) TRACE(64);
             float mx = -INFINITY;
             if (full) {
@@ -447,8 +379,8 @@ attention_enc_kernel(const __grid_constant__ CUtensorMap tmQKV, const Params p) 
                     }
                 }
             }
-            // PV_g(j-1) must be complete before P_g is overwritten and before O_g may be rescaled.  It is issued only
-            // when the slowest warp of the tile has stored its part of P(j-1), so the wait sits AFTER the exponentials
+            // PV(j-1) must be complete before P is overwritten and before O may be rescaled.  It is issued only
+            // when the slowest softmax warp has stored its part of P(j-1), so the wait sits AFTER the exponentials
             // (which only need registers): a fast warp overlaps it with useful work instead of stalling up front.
             if (j > 0) {
                 mbar_wait(&o_full[grp], (j - 1) & 1);
@@ -505,598 +437,16 @@ attention_enc_kernel(const __grid_constant__ CUtensorMap tmQKV, const Params p) 
     }
     tcgen05_fence_before();
     __syncthreads();
-    if (warp == MMA_WARP) {
-        tcgen05_fence_after();
-        tmem_dealloc(tmem_base, TMEM_COLS);
-    }
-}
-
-
-// ================================================================================================================
-// Variant "v3" (round 2, TWB200_ATTN=v3): THREE query tiles per CTA, kv tiles of 64 keys, ONE thread per query row.
-// The stall profile of the kernel above (profiles/r2d_attn_stalls.txt) shows the MUFU only 60 % busy although it is
-// the binding pipe: a CTA's two softmax warps per SM sub-partition move in lock-step (same S tile, row maximum
-// exchanged through a named barrier), so an SM holds just two independent "agents" per sub-partition, and whenever both
-// sit in their TMEM-load / row-max / exchange / store phase the MUFU idles.  Here a thread owns a whole row of a
-// 64-key tile (the same 64 exponentials per thread and kv step, but no exchange and no pair barrier), a tile needs one
-// warp per sub-partition, and THREE tiles share one CTA: three independent agents per sub-partition over one K / V
-// stream (K / V smem traffic per query row drops 3x), 448 threads, 144 registers per thread (no spills), one CTA per
-// SM.  TMEM: S_g 64 | P_g 32 | O_g 64 columns per tile = 480 of 512.
-// ================================================================================================================
-namespace v3 {
-constexpr int NT3 = 3;
-constexpr int BKV3 = 64;
-constexpr int STAGES = 4;
-constexpr int Q_BYTES = BQ * DH * 2;      // 16 KB
-constexpr int KV_BYTES = BKV3 * DH * 2;   // 8 KB
-constexpr int THREADS = 64 + NT3 * 128;
-constexpr int SMEM = NT3 * Q_BYTES + 2 * STAGES * KV_BYTES + 1024 + 512;
-constexpr int TMEM_COLS = 512;
-constexpr int S_COL = 0, P_COL = NT3 * 64, O_COL = NT3 * 96;
-
-__global__ void __launch_bounds__(THREADS, 1)
-attention_enc_v3_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmKV, const Params p) {
-    extern __shared__ uint8_t smem_raw[];
-    uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-    uint8_t* sQ = smem;
-    uint8_t* sK = smem + NT3 * Q_BYTES;
-    uint8_t* sV = sK + STAGES * KV_BYTES;
-    uint64_t* bars = reinterpret_cast<uint64_t*>(sV + STAGES * KV_BYTES);
-    uint64_t* q_full = bars + 0;
-    uint64_t* k_full = bars + 1;                  // [STAGES]
-    uint64_t* k_empty = k_full + STAGES;
-    uint64_t* v_full = k_empty + STAGES;
-    uint64_t* v_empty = v_full + STAGES;
-    uint64_t* s_full = v_empty + STAGES;          // [NT3]
-    uint64_t* p_full = s_full + NT3;
-    uint64_t* o_full = p_full + NT3;
-    uint64_t* s_free = o_full + NT3;
-    uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(s_free + NT3);
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int q0 = blockIdx.x * (NT3 * BQ), h = blockIdx.y, b = blockIdx.z;
-    const int nkv = (p.T + BKV3 - 1) / BKV3;
-
-    if (warp == 0 && lane == 0) {
-        tma_prefetch_desc(&tmQ);
-        tma_prefetch_desc(&tmKV);
-        mbar_init(q_full, 1);
-        for (int i = 0; i < STAGES; ++i) {
-            mbar_init(&k_full[i], 1); mbar_init(&k_empty[i], 1);
-            mbar_init(&v_full[i], 1); mbar_init(&v_empty[i], 1);
-        }
-        for (int g = 0; g < NT3; ++g) {
-            mbar_init(&s_full[g], 1); mbar_init(&p_full[g], 128); mbar_init(&o_full[g], 1); mbar_init(&s_free[g], 128);
-        }
-        fence_barrier_init();
-    }
-    if (warp == 1) {
-        tmem_alloc(tmem_ptr_smem, TMEM_COLS);
-        tmem_relinquish();
-    }
-    tcgen05_fence_before();
-    __syncthreads();
-    tcgen05_fence_after();
-    const uint32_t tmem_base = *tmem_ptr_smem;
-
-    if (warp == 0) {
-        if (lane == 0) {
-            mbar_arrive_expect_tx(q_full, NT3 * Q_BYTES);
-#pragma unroll
-            for (int g = 0; g < NT3; ++g) tma_load_3d(&tmQ, q_full, sQ + g * Q_BYTES, h * DH, q0 + g * BQ, b);
-            for (int j = 0; j < nkv; ++j) {
-                const int s = j % STAGES;
-                const uint32_t ph = (j / STAGES) & 1;
-                mbar_wait(&k_empty[s], ph ^ 1);
-                mbar_arrive_expect_tx(&k_full[s], KV_BYTES);
-                tma_load_3d(&tmKV, &k_full[s], sK + s * KV_BYTES, p.D + h * DH, j * BKV3, b);
-                mbar_wait(&v_empty[s], ph ^ 1);
-                mbar_arrive_expect_tx(&v_full[s], KV_BYTES);
-                tma_load_3d(&tmKV, &v_full[s], sV + s * KV_BYTES, 2 * p.D + h * DH, j * BKV3, b);
-            }
-        }
-    } else if (warp == 1) {
-        constexpr uint32_t idesc_s = umma_idesc_bf16(BQ, BKV3, 0, 0);
-        constexpr uint32_t idesc_o = umma_idesc_bf16(BQ, DH, 0, 1);   // B = V is MN-major
-        const uint64_t dq0 = umma_desc_sw128(smem_u32(sQ), 16, 1024);
-        const uint64_t dk0 = umma_desc_sw128(smem_u32(sK), 16, 1024);
-        const uint64_t dv0 = umma_desc_sw128(smem_u32(sV), 1024, 1024);
-        constexpr uint64_t Q_D = Q_BYTES >> 4, KV_D = KV_BYTES >> 4;
-        auto issue_s = [&](int g, int j) {   // S_g = Q_g K_j^T   (128 x 64 x 64)
-            const uint64_t a = dq0 + (uint64_t)g * Q_D, bd = dk0 + (uint64_t)(j % STAGES) * KV_D;
-            if (elect_one_sync()) {
-#pragma unroll
-                for (int k = 0; k < DH / 16; ++k)
-                    tcgen05_mma_f16(tmem_base + S_COL + g * BKV3, a + k * 2, bd + k * 2, idesc_s, k != 0);
-                tcgen05_commit(&s_full[g]);
-            }
-            __syncwarp();
-        };
-        auto issue_pv = [&](int g, int j) {  // O_g += P_g V_j   (128 x 64 x 64, A = P from TMEM)
-            const uint64_t bd = dv0 + (uint64_t)(j % STAGES) * KV_D;
-            const uint32_t p_tmem = tmem_base + P_COL + g * (BKV3 / 2);
-            const uint32_t acc0 = j != 0;
-            if (elect_one_sync()) {
-#pragma unroll
-                for (int k = 0; k < BKV3 / 16; ++k)
-                    tcgen05_mma_f16_ts(tmem_base + O_COL + g * DH, p_tmem + k * 8, bd + k * 128, idesc_o, k != 0 ? 1u : acc0);
-                tcgen05_commit(&o_full[g]);
-            }
-            __syncwarp();
-        };
-        auto release = [&](uint64_t* bar) {
-            if (elect_one_sync()) tcgen05_commit(bar);
-            __syncwarp();
-        };
-        mbar_wait(q_full, 0);
-        mbar_wait(&k_full[0], 0);
-        tcgen05_fence_after();
-#pragma unroll
-        for (int g = 0; g < NT3; ++g) issue_s(g, 0);
-        release(&k_empty[0]);
-        int js[NT3], jp[NT3];
-#pragma unroll
-        for (int g = 0; g < NT3; ++g) { js[g] = 1; jp[g] = 0; }
-        auto pending = [&]() { bool any = false;
-#pragma unroll
-            for (int g = 0; g < NT3; ++g) any = any || jp[g] < nkv;
-            return any; };
-        while (pending()) {
-#pragma unroll
-            for (int g = 0; g < NT3; ++g) {
-                if (js[g] < nkv && __any_sync(0xffffffffu, mbar_test_wait(&s_free[g], (js[g] - 1) & 1) &&
-                                                               mbar_test_wait(&k_full[js[g] % STAGES], (js[g] / STAGES) & 1))) {
-                    const int j = js[g];
-                    tcgen05_fence_after();
-                    issue_s(g, j);
-                    bool last_reader = true;
-#pragma unroll
-                    for (int o = 0; o < NT3; ++o) if (o != g) last_reader = last_reader && js[o] > j;
-                    if (last_reader) release(&k_empty[j % STAGES]);
-                    js[g] = j + 1;
-                }
-                if (jp[g] < nkv && __any_sync(0xffffffffu, mbar_test_wait(&p_full[g], jp[g] & 1) &&
-                                                               mbar_test_wait(&v_full[jp[g] % STAGES], (jp[g] / STAGES) & 1))) {
-                    const int j = jp[g];
-                    tcgen05_fence_after();
-                    issue_pv(g, j);
-                    bool last_reader = true;
-#pragma unroll
-                    for (int o = 0; o < NT3; ++o) if (o != g) last_reader = last_reader && jp[o] > j;
-                    if (last_reader) release(&v_empty[j % STAGES]);
-                    jp[g] = j + 1;
-                }
-            }
-        }
-    } else {
-        const int ws = warp - 2;
-        const int grp = ws >> 2;            // query tile of this warp
-        const int quarter = warp & 3;       // TMEM lane quarter this warp may access
-        const int r = quarter * 32 + lane;  // query row within the tile == TMEM lane
-        const uint32_t t_lane = (uint32_t)(quarter * 32) << 16;
-        const uint32_t s_col = S_COL + grp * BKV3, p_col = P_COL + grp * (BKV3 / 2), o_col = O_COL + grp * DH;
-        constexpr float RESCALE_LOG2 = 8.0f;
-        float m_used = -INFINITY, l_sum = 0.0f;
-        for (int j = 0; j < nkv; ++j) {
-            const uint32_t ph = j & 1;
-            const int kvalid = p.T - j * BKV3;
-            const bool full = kvalid >= BKV3;
-            mbar_wait(&s_full[grp], ph);
-            tcgen05_fence_after();
-            uint32_t v[BKV3];
-#pragma unroll
-            for (int c = 0; c < BKV3 / 16; ++c)
-                tmem_ld_32x32b_x16(tmem_base + t_lane + s_col + c * 16, *reinterpret_cast<uint32_t(*)[16]>(&v[c * 16]));
-            tmem_ld_wait();
-            tcgen05_fence_before();
-            mbar_arrive(&s_free[grp]);
-            float mx = -INFINITY;
-            if (full) {
-                float m4[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
-#pragma unroll
-                for (int i = 0; i < BKV3; i += 4) {
-                    m4[0] = fmaxf(m4[0], __uint_as_float(v[i]));
-                    m4[1] = fmaxf(m4[1], __uint_as_float(v[i + 1]));
-                    m4[2] = fmaxf(m4[2], __uint_as_float(v[i + 2]));
-                    m4[3] = fmaxf(m4[3], __uint_as_float(v[i + 3]));
-                }
-                mx = fmaxf(fmaxf(m4[0], m4[1]), fmaxf(m4[2], m4[3]));
-            } else {
-#pragma unroll
-                for (int i = 0; i < BKV3; ++i)
-                    if (i < kvalid) mx = fmaxf(mx, __uint_as_float(v[i]));
-            }
-            const float mx2 = mx * LOG2E;
-            const bool move = mx2 > m_used + RESCALE_LOG2;
-            const float alpha = move ? ex2_approx(m_used - mx2) : 1.0f;
-            if (move) m_used = mx2;
-            const float mb = m_used;
-            const uint64_t sc2 = pack_f32x2(LOG2E, LOG2E), mb2 = pack_f32x2(-mb, -mb);
-            uint64_t sum2[2] = {0ull, 0ull};
-            uint32_t pk[BKV3 / 2];
-            if (full) {
-#pragma unroll
-                for (int i = 0; i < BKV3 / 2; ++i) {
-                    const uint64_t a2 = fma_f32x2(pack_f32x2(__uint_as_float(v[2 * i]), __uint_as_float(v[2 * i + 1])), sc2, mb2);
-                    float p0, p1;
-                    if ((i % POLY_EVERY) == POLY_EVERY - 1) {
-                        exp2_poly_x2(a2, p0, p1);
-                    } else {
-                        float a0, a1;
-                        unpack_f32x2(a2, a0, a1);
-                        p0 = ex2_approx(a0);
-                        p1 = ex2_approx(a1);
-                    }
-                    sum2[i & 1] = add_f32x2(sum2[i & 1], pack_f32x2(p0, p1));
-                    pk[i] = pack_bf16x2(p0, p1);
-                }
-            } else {
-#pragma unroll
-                for (int i = 0; i < BKV3 / 2; ++i) {
-                    const int k0 = 2 * i;
-                    const float p0 = (k0 < kvalid) ? ex2_approx(fmaf(__uint_as_float(v[k0]), LOG2E, -mb)) : 0.0f;
-                    const float p1 = (k0 + 1 < kvalid) ? ex2_approx(fmaf(__uint_as_float(v[k0 + 1]), LOG2E, -mb)) : 0.0f;
-                    sum2[i & 1] = add_f32x2(sum2[i & 1], pack_f32x2(p0, p1));
-                    pk[i] = pack_bf16x2(p0, p1);
-                }
-            }
-            if (j > 0) {
-                mbar_wait(&o_full[grp], (j - 1) & 1);
-                tcgen05_fence_after();
-                if (__any_sync(0xffffffffu, move)) {
-#pragma unroll 1
-                    for (int c = 0; c < DH; c += 8) {
-                        uint32_t o[8];
-                        tmem_ld_32x32b_x8(tmem_base + t_lane + o_col + c, o);
-                        tmem_ld_wait();
-#pragma unroll
-                        for (int i = 0; i < 8; ++i) o[i] = __float_as_uint(__uint_as_float(o[i]) * alpha);
-                        tmem_st_32x32b_x8(tmem_base + t_lane + o_col + c, o);
-                    }
-                }
-            }
-            tmem_st_32x32b_x16(tmem_base + t_lane + p_col, *reinterpret_cast<uint32_t(*)[16]>(&pk[0]));
-            tmem_st_32x32b_x16(tmem_base + t_lane + p_col + 16, *reinterpret_cast<uint32_t(*)[16]>(&pk[16]));
-            float s0, s1, s2, s3;
-            unpack_f32x2(sum2[0], s0, s1);
-            unpack_f32x2(sum2[1], s2, s3);
-            l_sum = l_sum * alpha + ((s0 + s1) + (s2 + s3));
-            tmem_st_wait();
-            tcgen05_fence_before();
-            mbar_arrive(&p_full[grp]);
-        }
-        const float inv = 1.0f / l_sum;
-        mbar_wait(&o_full[grp], (nkv - 1) & 1);
-        tcgen05_fence_after();
-        const int q = q0 + grp * BQ + r;
-        __nv_bfloat16* o = p.out + ((size_t)b * p.T + q) * p.out_ld + h * DH;
-#pragma unroll
-        for (int half = 0; half < 2; ++half) {
-            uint32_t acc[32];
-            tmem_ld_32x32b_x32(tmem_base + t_lane + o_col + half * 32, acc);
-            tmem_ld_wait();
-            if (q < p.T) {
-#pragma unroll
-                for (int g = 0; g < 4; ++g) {
-                    uint4 w;
-                    w.x = pack_bf16x2(__uint_as_float(acc[g * 8 + 0]) * inv, __uint_as_float(acc[g * 8 + 1]) * inv);
-                    w.y = pack_bf16x2(__uint_as_float(acc[g * 8 + 2]) * inv, __uint_as_float(acc[g * 8 + 3]) * inv);
-                    w.z = pack_bf16x2(__uint_as_float(acc[g * 8 + 4]) * inv, __uint_as_float(acc[g * 8 + 5]) * inv);
-                    w.w = pack_bf16x2(__uint_as_float(acc[g * 8 + 6]) * inv, __uint_as_float(acc[g * 8 + 7]) * inv);
-                    reinterpret_cast<uint4*>(o + half * 32)[g] = w;
-                }
-            }
-        }
-        tcgen05_fence_before();
-    }
-    tcgen05_fence_before();
-    __syncthreads();
     if (warp == 1) {
         tcgen05_fence_after();
         tmem_dealloc(tmem_base, TMEM_COLS);
     }
 }
-}  // namespace v3
-
-
-// ================================================================================================================
-// Variant "persist" (round 2, TWB200_ATTN=persist): the default layout (one 128-query tile, two threads per row, two CTAs
-// per SM) as a PERSISTENT kernel.  Each CTA walks a strided list of (window, head, query tile) work items with running
-// barrier phases: TMEM, barriers and the tensor-map prefetch are set up once; the producer keeps streaming — the next
-// item's Q (double-buffered) and first K / V tiles land while the current item's last kv steps and epilogue run; the MMA
-// warp issues S(0) of the next item as soon as S is free, and only PV(0) waits for the epilogue to have read O (o_free).
-// Stall sampling attributed ~14 % of the default kernel's warp samples to per-CTA prologue / epilogue.
-// ================================================================================================================
-namespace persist {
-constexpr int THREADS = 64 + GROUP_THREADS;     // 320
-constexpr int SMEM = (2 + 4) * TILE_BYTES + XCH_BYTES + 1024 + 256;   // Q x2 | K x2 | V x2 | exchange | barriers
-constexpr int TMEM_COLS = 256;
-constexpr int S_COL = 0, P_COL = 128, O_COL = 192;
-
-__global__ void __launch_bounds__(THREADS, 2)
-attention_enc_persist_kernel(const __grid_constant__ CUtensorMap tmQKV, const Params p, const int n_items) {
-    extern __shared__ uint8_t smem_raw[];
-    uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-    uint8_t* sQ = smem;                              // 2 buffers
-    uint8_t* sK = smem + 2 * TILE_BYTES;             // 2 stages
-    uint8_t* sV = smem + 4 * TILE_BYTES;             // 2 stages
-    float* xch = reinterpret_cast<float*>(smem + 6 * TILE_BYTES);
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + 6 * TILE_BYTES + XCH_BYTES);
-    uint64_t* q_full = bars + 0;    // [2]
-    uint64_t* q_empty = bars + 2;   // [2]
-    uint64_t* k_full = bars + 4;    // [2]
-    uint64_t* k_empty = bars + 6;   // [2]
-    uint64_t* v_full = bars + 8;    // [2]
-    uint64_t* v_empty = bars + 10;  // [2]
-    uint64_t* s_full = bars + 12;
-    uint64_t* p_full = bars + 13;
-    uint64_t* o_full = bars + 14;
-    uint64_t* s_free = bars + 15;
-    uint64_t* o_free = bars + 16;
-    uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(bars + 17);
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int nkv = (p.T + BKV - 1) / BKV;
-    const int nq = (p.T + BQ - 1) / BQ;
-    const int stride = gridDim.x;
-
-    if (warp == 0 && lane == 0) {
-        tma_prefetch_desc(&tmQKV);
-        for (int i = 0; i < 2; ++i) {
-            mbar_init(&q_full[i], 1); mbar_init(&q_empty[i], 1);
-            mbar_init(&k_full[i], 1); mbar_init(&k_empty[i], 1);
-            mbar_init(&v_full[i], 1); mbar_init(&v_empty[i], 1);
-        }
-        mbar_init(s_full, 1); mbar_init(p_full, GROUP_THREADS); mbar_init(o_full, 1);
-        mbar_init(s_free, GROUP_THREADS); mbar_init(o_free, GROUP_THREADS);
-        fence_barrier_init();
-    }
-    if (warp == 1) {
-        tmem_alloc(tmem_ptr_smem, TMEM_COLS);
-        tmem_relinquish();
-    }
-    tcgen05_fence_before();
-    __syncthreads();
-    tcgen05_fence_after();
-    const uint32_t tmem_base = *tmem_ptr_smem;
-    // work item w -> (query tile, head, window): the tiles of one (window, head) are adjacent, so CTAs running at the same
-    // time share its K / V in L2
-    auto item = [&](int w, int& qt, int& h, int& b) { qt = w % nq; const int bh = w / nq; h = bh % p.H; b = bh / p.H; };
-
-    if (warp == 0) {
-        if (lane == 0) {
-            int it = 0;   // kv tiles loaded so far by this CTA (running stage / phase counter)
-            for (int w = blockIdx.x, t = 0; w < n_items; w += stride, ++t) {
-                int qt, h, b;
-                item(w, qt, h, b);
-                mbar_wait(&q_empty[t & 1], ((t >> 1) & 1) ^ 1);
-                mbar_arrive_expect_tx(&q_full[t & 1], TILE_BYTES);
-                tma_load_3d(&tmQKV, &q_full[t & 1], sQ + (t & 1) * TILE_BYTES, h * DH, qt * BQ, b);
-                for (int j = 0; j < nkv; ++j, ++it) {
-                    const int s = it & 1;
-                    const uint32_t ph = (it >> 1) & 1;
-                    mbar_wait(&k_empty[s], ph ^ 1);
-                    mbar_arrive_expect_tx(&k_full[s], TILE_BYTES);
-                    tma_load_3d(&tmQKV, &k_full[s], sK + s * TILE_BYTES, p.D + h * DH, j * BKV, b);
-                    mbar_wait(&v_empty[s], ph ^ 1);
-                    mbar_arrive_expect_tx(&v_full[s], TILE_BYTES);
-                    tma_load_3d(&tmQKV, &v_full[s], sV + s * TILE_BYTES, 2 * p.D + h * DH, j * BKV, b);
-                }
-            }
-        }
-    } else if (warp == 1) {
-        constexpr uint32_t idesc_s = umma_idesc_bf16(BQ, BKV, 0, 0);
-        constexpr uint32_t idesc_o = umma_idesc_bf16(BQ, DH, 0, 1);
-        const uint64_t dq0 = umma_desc_sw128(smem_u32(sQ), 16, 1024);
-        const uint64_t dk0 = umma_desc_sw128(smem_u32(sK), 16, 1024);
-        const uint64_t dv0 = umma_desc_sw128(smem_u32(sV), 1024, 1024);
-        constexpr uint64_t TILE_D = TILE_BYTES >> 4;
-        int n_mine = 0;
-        for (int w = blockIdx.x; w < n_items; w += stride) ++n_mine;
-        const int total = n_mine * nkv;       // kv iterations of this CTA over all its items
-        int gs = 0, gp = 0;                   // next S / PV iteration (global over the CTA's items)
-        while (gp < total) {
-            if (gs < total) {
-                const int t = gs / nkv, j = gs - t * nkv;
-                bool ready = (gs == 0 || mbar_test_wait(s_free, (gs - 1) & 1)) && mbar_test_wait(&k_full[gs & 1], (gs >> 1) & 1);
-                if (ready && j == 0) ready = mbar_test_wait(&q_full[t & 1], (t >> 1) & 1);
-                if (__any_sync(0xffffffffu, ready)) {
-                    tcgen05_fence_after();
-                    const uint64_t a = dq0 + (uint64_t)(t & 1) * TILE_D, bd = dk0 + (uint64_t)(gs & 1) * TILE_D;
-                    if (elect_one_sync()) {
-#pragma unroll
-                        for (int k = 0; k < DH / 16; ++k)
-                            tcgen05_mma_f16(tmem_base + S_COL, a + k * 2, bd + k * 2, idesc_s, k != 0);
-                        tcgen05_commit(s_full);
-                        tcgen05_commit(&k_empty[gs & 1]);
-                        if (j == nkv - 1) tcgen05_commit(&q_empty[t & 1]);   // last read of this item's Q
-                    }
-                    __syncwarp();
-                    ++gs;
-                }
-            }
-            {
-                const int t = gp / nkv, j = gp - t * nkv;
-                bool ready = gp < gs && mbar_test_wait(p_full, gp & 1) && mbar_test_wait(&v_full[gp & 1], (gp >> 1) & 1);
-                if (ready && j == 0 && t > 0) ready = mbar_test_wait(o_free, (t - 1) & 1);   // the previous item's O has been read
-                if (__any_sync(0xffffffffu, ready)) {
-                    tcgen05_fence_after();
-                    const uint64_t bd = dv0 + (uint64_t)(gp & 1) * TILE_D;
-                    const uint32_t acc0 = j != 0;
-                    if (elect_one_sync()) {
-#pragma unroll
-                        for (int k = 0; k < BKV / 16; ++k)
-                            tcgen05_mma_f16_ts(tmem_base + O_COL, tmem_base + P_COL + k * 8, bd + k * 128, idesc_o, k != 0 ? 1u : acc0);
-                        tcgen05_commit(o_full);
-                        tcgen05_commit(&v_empty[gp & 1]);
-                    }
-                    __syncwarp();
-                    ++gp;
-                }
-            }
-        }
-    } else {
-        const int quarter = warp & 3;
-        const int hf = ((warp - 2) >> 2) & 1;
-        const int r = quarter * 32 + lane;
-        const int pair_bar = 1 + quarter;
-        const uint32_t t_lane = (uint32_t)(quarter * 32) << 16;
-        const uint32_t s_col = S_COL + hf * (BKV / 2), p_col = P_COL + hf * (BKV / 4), o_col = O_COL + hf * (DH / 2);
-        constexpr int HK = BKV / 2;
-        constexpr float RESCALE_LOG2 = 8.0f;
-        int it = 0;   // kv iterations done so far (running phase counter)
-        for (int w = blockIdx.x, t = 0; w < n_items; w += stride, ++t) {
-            int qt, h, b;
-            item(w, qt, h, b);
-            float m_used = -INFINITY, l_sum = 0.0f;
-            for (int j = 0; j < nkv; ++j, ++it) {
-                const uint32_t ph = it & 1;
-                const int kvalid = p.T - j * BKV - hf * HK;
-                const bool full = kvalid >= HK;
-                mbar_wait(s_full, ph);
-                tcgen05_fence_after();
-                uint32_t v[HK];
-#pragma unroll
-                for (int c = 0; c < HK / 16; ++c)
-                    tmem_ld_32x32b_x16(tmem_base + t_lane + s_col + c * 16, *reinterpret_cast<uint32_t(*)[16]>(&v[c * 16]));
-                tmem_ld_wait();
-                tcgen05_fence_before();
-                mbar_arrive(s_free);
-                float mx = -INFINITY;
-                if (full) {
-                    float m4[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
-#pragma unroll
-                    for (int i = 0; i < HK; i += 4) {
-                        m4[0] = fmaxf(m4[0], __uint_as_float(v[i]));
-                        m4[1] = fmaxf(m4[1], __uint_as_float(v[i + 1]));
-                        m4[2] = fmaxf(m4[2], __uint_as_float(v[i + 2]));
-                        m4[3] = fmaxf(m4[3], __uint_as_float(v[i + 3]));
-                    }
-                    mx = fmaxf(fmaxf(m4[0], m4[1]), fmaxf(m4[2], m4[3]));
-                } else {
-#pragma unroll
-                    for (int i = 0; i < HK; ++i)
-                        if (i < kvalid) mx = fmaxf(mx, __uint_as_float(v[i]));
-                }
-                float* xm = xch + (ph * 2) * 128;
-                xm[hf * 128 + r] = mx;
-                named_bar_sync(pair_bar, 64);
-                mx = fmaxf(mx, xm[(hf ^ 1) * 128 + r]);
-                const float mx2 = mx * LOG2E;
-                const bool move = mx2 > m_used + RESCALE_LOG2;
-                const float alpha = move ? ex2_approx(m_used - mx2) : 1.0f;
-                if (move) m_used = mx2;
-                const float mb = m_used;
-                const uint64_t sc2 = pack_f32x2(LOG2E, LOG2E), mb2 = pack_f32x2(-mb, -mb);
-                uint64_t sum2[2] = {0ull, 0ull};
-                uint32_t pk[2][16];
-                if (full) {
-#pragma unroll
-                    for (int c = 0; c < HK / 32; ++c) {
-#pragma unroll
-                        for (int i = 0; i < 16; ++i) {
-                            const int k0 = c * 32 + 2 * i;
-                            const uint64_t a2 = fma_f32x2(pack_f32x2(__uint_as_float(v[k0]), __uint_as_float(v[k0 + 1])), sc2, mb2);
-                            float p0, p1;
-                            if ((i % POLY_EVERY) == POLY_EVERY - 1) {
-                                exp2_poly_x2(a2, p0, p1);
-                            } else {
-                                float a0, a1;
-                                unpack_f32x2(a2, a0, a1);
-                                p0 = ex2_approx(a0);
-                                p1 = ex2_approx(a1);
-                            }
-                            sum2[i & 1] = add_f32x2(sum2[i & 1], pack_f32x2(p0, p1));
-                            pk[c][i] = pack_bf16x2(p0, p1);
-                        }
-                    }
-                } else {
-#pragma unroll
-                    for (int c = 0; c < HK / 32; ++c) {
-#pragma unroll
-                        for (int i = 0; i < 16; ++i) {
-                            const int k0 = c * 32 + 2 * i;
-                            const float p0 = (k0 < kvalid) ? ex2_approx(fmaf(__uint_as_float(v[k0]), LOG2E, -mb)) : 0.0f;
-                            const float p1 = (k0 + 1 < kvalid) ? ex2_approx(fmaf(__uint_as_float(v[k0 + 1]), LOG2E, -mb)) : 0.0f;
-                            sum2[i & 1] = add_f32x2(sum2[i & 1], pack_f32x2(p0, p1));
-                            pk[c][i] = pack_bf16x2(p0, p1);
-                        }
-                    }
-                }
-                if (j > 0) {
-                    mbar_wait(o_full, (it - 1) & 1);
-                    tcgen05_fence_after();
-                    if (__any_sync(0xffffffffu, move)) {
-#pragma unroll 1
-                        for (int c = 0; c < DH / 2; c += 8) {
-                            uint32_t o[8];
-                            tmem_ld_32x32b_x8(tmem_base + t_lane + o_col + c, o);
-                            tmem_ld_wait();
-#pragma unroll
-                            for (int i = 0; i < 8; ++i) o[i] = __float_as_uint(__uint_as_float(o[i]) * alpha);
-                            tmem_st_32x32b_x8(tmem_base + t_lane + o_col + c, o);
-                        }
-                    }
-                }
-                tmem_st_32x32b_x16(tmem_base + t_lane + p_col, pk[0]);
-                tmem_st_32x32b_x16(tmem_base + t_lane + p_col + 16, pk[1]);
-                float s0, s1, s2, s3;
-                unpack_f32x2(sum2[0], s0, s1);
-                unpack_f32x2(sum2[1], s2, s3);
-                l_sum = l_sum * alpha + ((s0 + s1) + (s2 + s3));
-                tmem_st_wait();
-                tcgen05_fence_before();
-                mbar_arrive(p_full);
-            }
-            // total row sum = this thread's half + the partner's.  Its own slot: the two max-exchange slots are both in
-            // use around an item boundary (the partner may already be in the next item's first kv step)
-            float* xl = xch + 512;
-            xl[hf * 128 + r] = l_sum;
-            named_bar_sync(pair_bar, 64);
-            const float inv = 1.0f / (l_sum + xl[(hf ^ 1) * 128 + r]);
-            mbar_wait(o_full, (it - 1) & 1);
-            tcgen05_fence_after();
-            const int q = qt * BQ + r;
-            __nv_bfloat16* o = p.out + ((size_t)b * p.T + q) * p.out_ld + h * DH + hf * (DH / 2);
-            uint32_t acc[32];
-            tmem_ld_32x32b_x32(tmem_base + t_lane + o_col, acc);
-            tmem_ld_wait();
-            tcgen05_fence_before();
-            mbar_arrive(o_free);             // the next item's PV(0) may overwrite O now
-            if (q < p.T) {
-#pragma unroll
-                for (int g = 0; g < 4; ++g) {
-                    uint4 wv;
-                    wv.x = pack_bf16x2(__uint_as_float(acc[g * 8 + 0]) * inv, __uint_as_float(acc[g * 8 + 1]) * inv);
-                    wv.y = pack_bf16x2(__uint_as_float(acc[g * 8 + 2]) * inv, __uint_as_float(acc[g * 8 + 3]) * inv);
-                    wv.z = pack_bf16x2(__uint_as_float(acc[g * 8 + 4]) * inv, __uint_as_float(acc[g * 8 + 5]) * inv);
-                    wv.w = pack_bf16x2(__uint_as_float(acc[g * 8 + 6]) * inv, __uint_as_float(acc[g * 8 + 7]) * inv);
-                    reinterpret_cast<uint4*>(o)[g] = wv;
-                }
-            }
-            // the exchange slot written above is reused two kv steps later at the earliest (other parity first)
-        }
-    }
-    tcgen05_fence_before();
-    __syncthreads();
-    if (warp == 1) {
-        tcgen05_fence_after();
-        tmem_dealloc(tmem_base, TMEM_COLS);
-    }
-}
-}  // namespace persist
 
 }  // namespace attn
 }  // namespace tw
 
 static long long* g_attn_dbg = nullptr;
-// query tiles per CTA: 1 (two independent CTAs per SM: default, 16 % faster on the same box) or 2 (one CTA per SM, K/V shared);
-// TWB200_ATTN_TILES=2 selects the latter for comparison
-static int g_attn_tiles = [] { const char* e = getenv("TWB200_ATTN_TILES"); return (e && e[0] == '2') ? 2 : 1; }();
-// TWB200_ATTN=v3 selects the three-tile / 64-key / one-thread-per-row kernel (see namespace v3)
-static int g_attn_v3 = [] { const char* e = getenv("TWB200_ATTN"); return (e && e[0] == 'v' && e[1] == '3') ? 1 : 0; }();
-// TWB200_ATTN=persist selects the persistent form of the default layout (see namespace persist)
-static int g_attn_persist = [] { const char* e = getenv("TWB200_ATTN"); return (e && e[0] == 'p') ? 1 : 0; }();
 extern "C" int tw_attention_enc_set_trace(void* dev_buf_int64_x192) { g_attn_dbg = (long long*)dev_buf_int64_x192; return 0; }
 
 extern "C" int tw_attention_enc(const void* qkv_bf16, void* out_bf16, int32_t batch, int32_t seq,
@@ -1122,47 +472,11 @@ extern "C" int tw_attention_enc(const void* qkv_bf16, void* out_bf16, int32_t ba
     p.T = seq; p.H = heads; p.D = D; p.out_ld = out_ld; p.out = (__nv_bfloat16*)out_bf16; p.dbg = g_attn_dbg;
     static std::atomic<unsigned long long> attr_done{0};
     if (device_needs_setup(attr_done)) {
-        TW_CUDA_CHECK(cudaFuncSetAttribute(attention_enc_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes(1)));
-        TW_CUDA_CHECK(cudaFuncSetAttribute(attention_enc_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes(2)));
+        TW_CUDA_CHECK(cudaFuncSetAttribute(attention_enc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
         mark_device_done(attr_done);
     }
-    if (g_attn_persist) {
-        static std::atomic<unsigned long long> attrp_done{0};
-        if (device_needs_setup(attrp_done)) {
-            TW_CUDA_CHECK(cudaFuncSetAttribute(persist::attention_enc_persist_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                               persist::SMEM));
-            mark_device_done(attrp_done);
-        }
-        const int n_items = ((seq + BQ - 1) / BQ) * heads * batch;
-        const int sms = num_sms();
-        const int grid = n_items < 2 * sms ? n_items : 2 * sms;
-        persist::attention_enc_persist_kernel<<<grid, persist::THREADS, persist::SMEM, (cudaStream_t)stream>>>(tm, p, n_items);
-        TW_CUDA_CHECK(cudaGetLastError());
-        return 0;
-    }
-    if (g_attn_v3) {
-        CUtensorMap tmKV;
-        const uint32_t box_kv[3] = {DH, v3::BKV3, 1};
-        if (encode_tensor_map(&tmKV, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, qkv_bf16, dims, strides, box_kv,
-                              CU_TENSOR_MAP_SWIZZLE_128B))
-            return 1;
-        static std::atomic<unsigned long long> attr3_done{0};
-        if (device_needs_setup(attr3_done)) {
-            TW_CUDA_CHECK(cudaFuncSetAttribute(v3::attention_enc_v3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, v3::SMEM));
-            mark_device_done(attr3_done);
-        }
-        dim3 grid((seq + v3::NT3 * BQ - 1) / (v3::NT3 * BQ), heads, batch);
-        v3::attention_enc_v3_kernel<<<grid, v3::THREADS, v3::SMEM, (cudaStream_t)stream>>>(tm, tmKV, p);
-        TW_CUDA_CHECK(cudaGetLastError());
-        return 0;
-    }
-    if (g_attn_tiles == 1) {
-        dim3 grid((seq + BQ - 1) / BQ, heads, batch);
-        attention_enc_kernel<1><<<grid, num_threads(1), smem_bytes(1), (cudaStream_t)stream>>>(tm, p);
-    } else {
-        dim3 grid((seq + 2 * BQ - 1) / (2 * BQ), heads, batch);
-        attention_enc_kernel<2><<<grid, num_threads(2), smem_bytes(2), (cudaStream_t)stream>>>(tm, p);
-    }
+    dim3 grid((seq + BQ - 1) / BQ, heads, batch);
+    attention_enc_kernel<<<grid, NUM_THREADS, SMEM_BYTES, (cudaStream_t)stream>>>(tm, p);
     TW_CUDA_CHECK(cudaGetLastError());
     return 0;
 }

@@ -9,13 +9,10 @@
 // time-major activations, so im2col is never materialised
 // ($TF/models/whisper/modeling_whisper.py:619-620 conv1/conv2 + gelu).
 //
-// CTA = 320 threads: warp 0 TMA producer, warp 1 MMA issuer (+TMEM owner), warps 2-9 epilogue.
-// Two kernels share the epilogue design:
-//   gemm_bf16_2cta_kernel (default)  CTA pairs, cta_group::2, 256 x 256 x 64 tile per pair, 6-stage ring of 32 KB per CTA
-//   gemm_bf16_kernel                 one CTA per 128 x 256 x 64 tile, 4-stage ring of 48 KB (TWB200_GEMM_2CTA=0)
+// CTA = 320 threads: warp 0 TMA producer, warp 1 MMA issuer (+TMEM owner), warps 2-9 epilogue.  CTA pairs
+// (cta_group::2) own a 256 x 256 x 64 tile, 6-stage ring of 32 KB per CTA.
 // Two 256-column fp32 accumulators in TMEM per CTA so the epilogue of tile i overlaps the MMAs of tile i+1.
 // Grid = #SMs, static tile striding.
-#include <cstdlib>
 #include "common.cuh"
 #include "twb200_internal.h"
 
@@ -26,19 +23,15 @@ constexpr int BM = 128;
 constexpr int BN = 256;
 constexpr int BK = 64;
 constexpr int UMMA_K = 16;
-constexpr int STAGES = 4;
 constexpr int A_STAGE_BYTES = BM * BK * 2;  // 16 KB
-constexpr int B_STAGE_BYTES = BN * BK * 2;  // 32 KB
 constexpr int NUM_THREADS = 320;   // warp 0 TMA, warp 1 MMA, warps 2-9 epilogue (two warps per TMEM lane quarter)
 constexpr int TMEM_COLS = 512;
 constexpr int EPI_WARPS = 8;
 constexpr int EPI_STAGE_BYTES = EPI_WARPS * 32 * 32 * 4;  // one 32x32 fp32 tile per epilogue warp
-constexpr int SMEM_BYTES = STAGES * (A_STAGE_BYTES + B_STAGE_BYTES) + 1024 /*align*/ + 256 /*barriers*/ + EPI_STAGE_BYTES;
 
 struct Params {
     int rows, batches, N, K;
-    int m_tiles_per_batch, n_tiles, num_tiles, num_k_blocks;
-    int tile_m;   // rows per scheduled tile: BM (1-CTA kernel) or 2*BM (cta_group::2 kernel: one CTA pair per tile)
+    int m_tiles_per_batch, n_tiles, num_tiles, num_k_blocks;   // a tile is 2 * BM rows (one CTA pair) x BN columns
     const int* a_row_off;
     const float* bias;
     const float* resid;
@@ -59,211 +52,20 @@ TW_DEVINL TileCoord decode_tile(const Params& p, int tile) {
     const int nt = tile % p.n_tiles;
     const int mt_all = tile / p.n_tiles;
     t.b = mt_all / p.m_tiles_per_batch;
-    t.m0 = (mt_all - t.b * p.m_tiles_per_batch) * p.tile_m;
+    t.m0 = (mt_all - t.b * p.m_tiles_per_batch) * (2 * BM);
     t.n0 = nt * BN;
     return t;
 }
 
-// OUT_F32 / HAS_RESID / ACT are compile-time so the epilogue carries no per-element flag tests
-template <bool OUT_F32, bool HAS_RESID, int ACT>
-__global__ void __launch_bounds__(NUM_THREADS, 1)
-gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-                 const Params p) {
-    extern __shared__ uint8_t smem_raw[];
-    uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) &
-                                               ~uintptr_t(1023));
-    uint8_t* sA = smem;
-    uint8_t* sB = smem + STAGES * A_STAGE_BYTES;
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + STAGES * (A_STAGE_BYTES + B_STAGE_BYTES));
-    uint64_t* full_bar = bars;                    // [STAGES]
-    uint64_t* empty_bar = bars + STAGES;          // [STAGES]
-    uint64_t* tmem_full_bar = bars + 2 * STAGES;  // [2]
-    uint64_t* tmem_empty_bar = bars + 2 * STAGES + 2;  // [2]
-    uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(bars + 2 * STAGES + 4);
-
-    const int warp = threadIdx.x >> 5;
-    const int lane = threadIdx.x & 31;
-
-    if (warp == 0 && lane == 0) {
-        tma_prefetch_desc(&tmA);
-        tma_prefetch_desc(&tmB);
-        for (int s = 0; s < STAGES; ++s) {
-            mbar_init(&full_bar[s], 1);
-            mbar_init(&empty_bar[s], 1);
-        }
-        for (int s = 0; s < 2; ++s) {
-            mbar_init(&tmem_full_bar[s], 1);
-            mbar_init(&tmem_empty_bar[s], EPI_WARPS * 32);
-        }
-        fence_barrier_init();
-    }
-    if (warp == 1) {
-        tmem_alloc(tmem_ptr_smem, TMEM_COLS);
-        tmem_relinquish();
-    }
-    tcgen05_fence_before();
-    __syncthreads();
-    tcgen05_fence_after();
-    const uint32_t tmem_base = *tmem_ptr_smem;
-
-    if (warp == 0) {
-        if (lane == 0) {
-            // ===================== TMA producer =====================
-            int stage = 0;
-            uint32_t phase = 0;
-            for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x) {
-                const TileCoord t = decode_tile(p, tile);
-                const int row0 = t.m0 + (p.a_row_off ? p.a_row_off[t.b] : 0);
-                for (int kb = 0; kb < p.num_k_blocks; ++kb) {
-                    mbar_wait(&empty_bar[stage], phase ^ 1);
-                    mbar_arrive_expect_tx(&full_bar[stage], A_STAGE_BYTES + B_STAGE_BYTES);
-                    tma_load_3d(&tmA, &full_bar[stage], sA + stage * A_STAGE_BYTES, kb * BK, row0, t.b);
-                    tma_load_2d(&tmB, &full_bar[stage], sB + stage * B_STAGE_BYTES, kb * BK, t.n0);
-                    if (++stage == STAGES) { stage = 0; phase ^= 1; }
-                }
-            }
-        }
-    } else if (warp == 1) {
-        if (lane == 0) {
-            // ===================== MMA issuer =====================
-            constexpr uint32_t idesc = umma_idesc_bf16(BM, BN, 0, 0);
-            int stage = 0;
-            uint32_t phase = 0;
-            int acc = 0;
-            uint32_t acc_phase = 0;
-            for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x) {
-                mbar_wait(&tmem_empty_bar[acc], acc_phase ^ 1);
-                tcgen05_fence_after();
-                const uint32_t d_tmem = tmem_base + acc * BN;
-                for (int kb = 0; kb < p.num_k_blocks; ++kb) {
-                    mbar_wait(&full_bar[stage], phase);
-                    tcgen05_fence_after();
-                    const uint32_t a_addr = smem_u32(sA + stage * A_STAGE_BYTES);
-                    const uint32_t b_addr = smem_u32(sB + stage * B_STAGE_BYTES);
-#pragma unroll
-                    for (int k = 0; k < BK / UMMA_K; ++k) {
-                        const uint64_t adesc = umma_desc_sw128(a_addr + k * UMMA_K * 2, 16, 1024);
-                        const uint64_t bdesc = umma_desc_sw128(b_addr + k * UMMA_K * 2, 16, 1024);
-                        tcgen05_mma_f16(d_tmem, adesc, bdesc, idesc, (kb | k) != 0 ? 1u : 0u);
-                    }
-                    tcgen05_commit(&empty_bar[stage]);  // frees the smem slot when the MMAs retire
-                    if (++stage == STAGES) { stage = 0; phase ^= 1; }
-                }
-                tcgen05_commit(&tmem_full_bar[acc]);  // accumulator complete -> epilogue
-                if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-            }
-        }
-    } else {
-        // ===================== epilogue (warps 2..5) =====================
-        // Two phases per 32-column chunk so that every global access is coalesced:
-        //   A  thread = accumulator row: tcgen05.ld 32 fp32 -> its 128-byte row of the warp's smem tile
-        //      (16-byte chunks XOR-swizzled by row, conflict-free)
-        //   B  8 lanes = one 128-byte row segment: bias, activation, fp32 residual (coalesced 128 B
-        //      loads), store (128 B fp32 / 64 B bf16 per row per instruction)
-        const int quarter = warp & 3;       // TMEM lane quarter this warp may access
-        const int chalf = (warp - 2) >> 2;  // warps 2-5 take column chunks 0-3, warps 6-9 chunks 4-7 of the tile
-        float* stage = reinterpret_cast<float*>(smem + STAGES * (A_STAGE_BYTES + B_STAGE_BYTES) + 256) +
-                       (warp - 2) * (32 * 32);
-        const int sub = lane & 7;    // phase B: 16-byte column chunk within the 32-column chunk
-        const int rgrp = lane >> 3;  // phase B: row = rgrp + 4*i
-        int acc = 0;
-        uint32_t acc_phase = 0;
-        for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x) {
-            const TileCoord t = decode_tile(p, tile);
-            mbar_wait(&tmem_full_bar[acc], acc_phase);
-            tcgen05_fence_after();
-            const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + acc * BN;
-            const int row_base = t.m0 + quarter * 32;  // first row of this warp within the batch
-#pragma unroll 1
-            for (int c = chalf * (BN / 64); c < (chalf + 1) * (BN / 64); ++c) {
-                const int n_base = t.n0 + c * 32;
-                if (n_base >= p.N) break;  // warp-uniform
-                uint32_t v[32];
-                tmem_ld_32x32b_x32(taddr + c * 32, v);
-                tmem_ld_wait();
-                {
-                    float4* dst = reinterpret_cast<float4*>(stage + lane * 32);
-                    const int sw = lane & 7;
-#pragma unroll
-                    for (int g = 0; g < 8; ++g)
-                        dst[g ^ sw] = make_float4(__uint_as_float(v[4 * g]), __uint_as_float(v[4 * g + 1]),
-                                                  __uint_as_float(v[4 * g + 2]), __uint_as_float(v[4 * g + 3]));
-                }
-                __syncwarp();
-                const int n = n_base + sub * 4;
-                if (n < p.N) {
-                    float4 bias4 = make_float4(0.f, 0.f, 0.f, 0.f);
-                    if (p.bias) bias4 = __ldg(reinterpret_cast<const float4*>(p.bias + n));
-                    const int r0 = row_base + rgrp;  // this lane's rows are r0 + 4*i
-                    const float* rp = nullptr;
-                    if (HAS_RESID) rp = p.resid + ((size_t)t.b * p.resid_batch_rows + r0) * p.resid_ld + n;
-                    size_t o0 = ((size_t)t.b * p.out_batch_rows + p.out_row_off + r0) * p.out_ld + n;
-                    size_t out_ld = (size_t)p.out_ld;
-                    if (p.out_mode == 1) {  // element (b, r, n) -> [n / 64][b][r][n % 64]
-                        o0 = (((size_t)(n >> 6) * p.batches + t.b) * p.rows + r0) * 64 + (n & 63);
-                        out_ld = 64;
-                    }
-                    float* of = reinterpret_cast<float*>(p.out) + o0;
-                    __nv_bfloat16* ob = reinterpret_cast<__nv_bfloat16*>(p.out) + o0;
-                    const int nrows = p.rows - r0;  // rows r0 + 4*i with 4*i < nrows are valid
-                    float4 val[8];
-                    float4 res[8];
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) {
-                        const int rl = rgrp + 4 * i;
-                        val[i] = reinterpret_cast<const float4*>(stage + rl * 32)[sub ^ (rl & 7)];
-                        if (HAS_RESID) {
-                            res[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-                            if (4 * i < nrows) res[i] = *reinterpret_cast<const float4*>(rp + (size_t)(4 * i) * p.resid_ld);
-                        }
-                    }
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) {
-                        float4 f = val[i];
-                        f.x += bias4.x; f.y += bias4.y; f.z += bias4.z; f.w += bias4.w;
-                        if (ACT == 1) {
-                            gelu_erf_fast_x2(f.x, f.y);
-                            gelu_erf_fast_x2(f.z, f.w);
-                        }
-                        if (HAS_RESID) { f.x += res[i].x; f.y += res[i].y; f.z += res[i].z; f.w += res[i].w; }
-                        if (4 * i < nrows) {
-                            if (OUT_F32) {
-                                *reinterpret_cast<float4*>(of + (size_t)(4 * i) * out_ld) = f;
-                            } else {
-                                uint2 pk;
-                                pk.x = pack_bf16x2(f.x, f.y);
-                                pk.y = pack_bf16x2(f.z, f.w);
-                                *reinterpret_cast<uint2*>(ob + (size_t)(4 * i) * out_ld) = pk;
-                            }
-                        }
-                    }
-                }
-                __syncwarp();  // the staging tile is rewritten by the next chunk
-            }
-            tcgen05_fence_before();
-            mbar_arrive(&tmem_empty_bar[acc]);
-            if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-        }
-    }
-
-    tcgen05_fence_before();
-    __syncthreads();
-    if (warp == 1) {
-        tcgen05_fence_after();
-        tmem_dealloc(tmem_base, TMEM_COLS);
-    }
-}
-
-
 // ================================================================================================
-// cta_group::2 variant: a CLUSTER of two CTAs (one SM pair) owns a 256 x 256 output tile.
+// A CLUSTER of two CTAs (one SM pair) owns a 256 x 256 output tile.
 //
-// The 1-CTA kernel above moves (128 + 256) * K * 2 bytes into shared memory per 2 * 128 * 256 * K FLOP = 85 FLOP/B,
-// and at ~64 B/clk per SM of shared-memory fill that caps the chip near 1500 TFLOP/s (measured 1210-1330 on the
-// K = 1280 encoder shapes).  Here each CTA loads its own 128 rows of A and only HALF of the B tile (128 of the 256
+// One CTA per 128 x 256 tile would move (128 + 256) * K * 2 bytes into shared memory per 2 * 128 * 256 * K FLOP =
+// 85 FLOP/B, and at ~64 B/clk per SM of shared-memory fill that caps the chip near 1500 TFLOP/s (measured 1210-1330 on
+// the K = 1280 encoder shapes).  Here each CTA loads its own 128 rows of A and only HALF of the B tile (128 of the 256
 // output columns); tcgen05.mma.cta_group::2 (issued by the leader CTA only, M = 256) reads A and B from both CTAs'
 // shared memory: 128 FLOP/B.  Each CTA keeps the accumulator rows of its own 128 rows in its own TMEM and runs the
-// same epilogue as the 1-CTA kernel.
+// epilogue for them.
 //   * TMA loads of both CTAs complete on the LEADER's full barrier (shared::cluster address with the peer bit cleared);
 //   * tcgen05.commit multicasts to the empty / accumulator-full barriers of both CTAs;
 //   * the epilogue threads of both CTAs arrive on the leader's accumulator-empty barrier (remote mbarrier arrive).
@@ -325,6 +127,7 @@ TW_DEVINL void mbar_arrive_leader(uint64_t* bar) {   // arrive on the even CTA's
     asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(smem_u32(bar) & PEER_BIT_MASK) : "memory");
 }
 
+// OUT_F32 / HAS_RESID / ACT are compile-time so the epilogue carries no per-element flag tests
 template <bool OUT_F32, bool HAS_RESID, int ACT>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1)
 gemm_bf16_2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
@@ -374,7 +177,7 @@ gemm_bf16_2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
             int stage = 0;
             uint32_t phase = 0;
             for (int tile = cluster; tile < p.num_tiles; tile += n_clusters) {
-                const TileCoord t = decode_tile(p, tile);     // m0 in units of 2*BM rows (see the launcher)
+                const TileCoord t = decode_tile(p, tile);
                 const int row0 = t.m0 + (int)rank * BM + (p.a_row_off ? p.a_row_off[t.b] : 0);
                 for (int kb = 0; kb < p.num_k_blocks; ++kb) {
                     mbar_wait(&empty_bar[stage], phase ^ 1);
@@ -416,12 +219,17 @@ gemm_bf16_2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
             }
         }
     } else {
-        // ===================== epilogue (warps 2..9 of both CTAs; identical to the 1-CTA kernel) =====================
-        const int quarter = warp & 3;
-        const int chalf = (warp - 2) >> 2;
+        // ===================== epilogue (warps 2..9 of both CTAs) =====================
+        // Two phases per 32-column chunk so that every global access is coalesced:
+        //   A  thread = accumulator row: tcgen05.ld 32 fp32 -> its 128-byte row of the warp's smem tile
+        //      (16-byte chunks XOR-swizzled by row, conflict-free)
+        //   B  8 lanes = one 128-byte row segment: bias, activation, fp32 residual (coalesced 128 B
+        //      loads), store (128 B fp32 / 64 B bf16 per row per instruction)
+        const int quarter = warp & 3;       // TMEM lane quarter this warp may access
+        const int chalf = (warp - 2) >> 2;  // warps 2-5 take column chunks 0-3, warps 6-9 chunks 4-7 of the tile
         float* stage = reinterpret_cast<float*>(smem + STAGES2 * (A_STAGE_BYTES + B2_STAGE_BYTES) + 256) + (warp - 2) * (32 * 32);
-        const int sub = lane & 7;
-        const int rgrp = lane >> 3;
+        const int sub = lane & 7;    // phase B: 16-byte column chunk within the 32-column chunk
+        const int rgrp = lane >> 3;  // phase B: row = rgrp + 4*i
         int acc = 0;
         uint32_t acc_phase = 0;
         for (int tile = cluster; tile < p.num_tiles; tile += n_clusters) {
@@ -548,24 +356,20 @@ extern "C" int tw_gemm_bf16(const tw_gemm_args* a, void* stream) {
                               CU_TENSOR_MAP_SWIZZLE_128B))
             return 1;
     }
-    {
+    {   // each CTA of the pair loads 128 of the tile's 256 output columns
         const uint64_t dims[2] = {(uint64_t)a->k, (uint64_t)a->n};
         const uint64_t strides[1] = {(uint64_t)a->k * 2};
-        const uint32_t box[2] = {BK, BN};
+        const uint32_t box[2] = {BK, 128};
         if (encode_tensor_map(&tmB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, a->w, dims, strides, box,
                               CU_TENSOR_MAP_SWIZZLE_128B))
             return 1;
     }
-    // default: the cta_group::2 kernel (256 x 256 tile per CTA pair, +5-10 % on the encoder shapes); TWB200_GEMM_2CTA=0
-    // selects the 1-CTA kernel for comparison
-    static const bool use_2cta = [] { const char* e = getenv("TWB200_GEMM_2CTA"); return !(e && e[0] == '0'); }();
     Params p;
     p.rows = a->rows;
     p.batches = a->batches;
     p.N = a->n;
     p.K = a->k;
-    p.tile_m = use_2cta ? 2 * BM : BM;
-    p.m_tiles_per_batch = (a->rows + p.tile_m - 1) / p.tile_m;
+    p.m_tiles_per_batch = (a->rows + 2 * BM - 1) / (2 * BM);
     p.n_tiles = (a->n + BN - 1) / BN;
     p.num_tiles = p.m_tiles_per_batch * p.batches * p.n_tiles;
     p.num_k_blocks = (a->k + BK - 1) / BK;
@@ -584,44 +388,20 @@ extern "C" int tw_gemm_bf16(const tw_gemm_args* a, void* stream) {
 
     const int sms = num_sms();
     TW_REQUIRE(sms > 0, "tw_gemm_bf16: no CUDA device");
-    if (use_2cta) {
-        CUtensorMap tmB2;   // each CTA of the pair loads 128 of the tile's 256 output columns
-        const uint64_t dims[2] = {(uint64_t)a->k, (uint64_t)a->n};
-        const uint64_t strides[1] = {(uint64_t)a->k * 2};
-        const uint32_t box[2] = {BK, 128};
-        if (encode_tensor_map(&tmB2, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, a->w, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B))
-            return 1;
-        typedef void (*kern2_t)(const CUtensorMap, const CUtensorMap, const Params);
-        static const kern2_t kernels2[8] = {
-            gemm_bf16_2cta_kernel<false, false, 0>, gemm_bf16_2cta_kernel<false, false, 1>, gemm_bf16_2cta_kernel<false, true, 0>,
-            gemm_bf16_2cta_kernel<false, true, 1>,  gemm_bf16_2cta_kernel<true, false, 0>,  gemm_bf16_2cta_kernel<true, false, 1>,
-            gemm_bf16_2cta_kernel<true, true, 0>,   gemm_bf16_2cta_kernel<true, true, 1>};
-        static std::atomic<unsigned long long> attr2_done{0};
-        if (device_needs_setup(attr2_done)) {
-            for (int i = 0; i < 8; ++i)
-                TW_CUDA_CHECK(cudaFuncSetAttribute(kernels2[i], cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM2_BYTES));
-            mark_device_done(attr2_done);
-        }
-        const int clusters = p.num_tiles < sms / 2 ? p.num_tiles : sms / 2;
-        const kern2_t k2 = kernels2[(p.out_f32 ? 4 : 0) + (p.resid ? 2 : 0) + (p.act ? 1 : 0)];
-        k2<<<2 * clusters, NUM_THREADS, SMEM2_BYTES, (cudaStream_t)stream>>>(tmA, tmB2, p);
-        TW_CUDA_CHECK(cudaGetLastError());
-        return 0;
-    }
-    const int grid = p.num_tiles < sms ? p.num_tiles : sms;
     typedef void (*kern_t)(const CUtensorMap, const CUtensorMap, const Params);
     static const kern_t kernels[8] = {
-        gemm_bf16_kernel<false, false, 0>, gemm_bf16_kernel<false, false, 1>, gemm_bf16_kernel<false, true, 0>,
-        gemm_bf16_kernel<false, true, 1>,  gemm_bf16_kernel<true, false, 0>,  gemm_bf16_kernel<true, false, 1>,
-        gemm_bf16_kernel<true, true, 0>,   gemm_bf16_kernel<true, true, 1>};
+        gemm_bf16_2cta_kernel<false, false, 0>, gemm_bf16_2cta_kernel<false, false, 1>, gemm_bf16_2cta_kernel<false, true, 0>,
+        gemm_bf16_2cta_kernel<false, true, 1>,  gemm_bf16_2cta_kernel<true, false, 0>,  gemm_bf16_2cta_kernel<true, false, 1>,
+        gemm_bf16_2cta_kernel<true, true, 0>,   gemm_bf16_2cta_kernel<true, true, 1>};
     static std::atomic<unsigned long long> attr_done{0};
     if (device_needs_setup(attr_done)) {
         for (int i = 0; i < 8; ++i)
-            TW_CUDA_CHECK(cudaFuncSetAttribute(kernels[i], cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+            TW_CUDA_CHECK(cudaFuncSetAttribute(kernels[i], cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM2_BYTES));
         mark_device_done(attr_done);
     }
+    const int clusters = p.num_tiles < sms / 2 ? p.num_tiles : sms / 2;
     const kern_t k = kernels[(p.out_f32 ? 4 : 0) + (p.resid ? 2 : 0) + (p.act ? 1 : 0)];
-    k<<<grid, NUM_THREADS, SMEM_BYTES, (cudaStream_t)stream>>>(tmA, tmB, p);
+    k<<<2 * clusters, NUM_THREADS, SMEM2_BYTES, (cudaStream_t)stream>>>(tmA, tmB, p);
     TW_CUDA_CHECK(cudaGetLastError());
     return 0;
 }

@@ -26,9 +26,6 @@ from .config import N_FRAMES, N_SAMPLES, GenerationSettings, WhisperDims
 
 MAX_DECODE_BATCH = 96   # decode rows per engine context (projections: up to tw_dec_max_rows(); the LM head runs per 48-row chunk)
 LMHEAD_ROWS = 48
-# timing probe only (results are WRONG): skip the LayerNorm fused into the residual projections, to measure what the
-# last-CTA LayerNorm tails cost per decode step (tools/probe_decode_tail.py)
-_PROBE_NO_LN = bool(os.environ.get("TWB200_PROBE_NO_LN"))
 _CAPTURE_LOCK = threading.Lock()   # CUDA-graph capture is serialised across the engine contexts of a process
 PAGE = 64
 ROWSTATE_INTS = 8
@@ -481,7 +478,7 @@ class WhisperEngine:
         a.bias = None if bias is None else self.w[bias].data_ptr()
         # fragment-major weights are padded to 16 rows: the true N is the bias length (the LM head has N = vocab)
         a.batch, a.n, a.k = B, (self.dims.vocab if bias is None else self.w[bias].shape[0]), k
-        if ln is not None and not _PROBE_NO_LN:
+        if ln is not None:
             a.ln_gamma, a.ln_beta = self.w[ln + "_w"].data_ptr(), self.w[ln + "_b"].data_ptr()
             a.ln_out_bf16, a.ln_counter = self.dxn.data_ptr(), self.ln_cnt.data_ptr()
         if part_out:
