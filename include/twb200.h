@@ -40,7 +40,7 @@ int tw_abi_version(void);
  * Replaces WhisperFeatureExtractor._torch_extract_fbank_features
  * ($TF/models/whisper/feature_extraction_whisper.py:135-164) for clips already cut to <= 30 s:
  * zero-pad to 480000 samples, reflect-padded 400-point STFT at hop 160 (periodic Hann), power,
- * 128 slaney mel filters, log10(max(.,1e-10)), max(x, clipmax-8), (x+4)/4.
+ * 128 (or, through the *_n entry points, 80) slaney mel filters, log10(max(.,1e-10)), max(x, clipmax-8), (x+4)/4.
  * ---------------------------------------------------------------------------------------------- */
 size_t tw_logmel_tables_bytes(void);
 size_t tw_logmel_scratch_bytes(int32_t batch);
@@ -64,6 +64,18 @@ int tw_logmel(const void* tables_dev, const float* pcm, int64_t pcm_stride, cons
 int tw_logmel_long(const void* tables_dev, const float* pcm_long, int64_t hop_samples, int32_t n_windows,
                    const int32_t* frame_lo, const int32_t* frame_hi, const int32_t* out_row0, uint32_t* max_scratch,
                    void* out_bf16_t, int64_t total_frames, int32_t out_t_row_off, void* stream);
+/* The same three functions for a given mel-bin count: n_mels is 128 (the large-v3 family; what the functions above
+ * use) or 80 (large-v2 and older checkpoints, WhisperFeatureExtractor(feature_size=80)); any other count is an error.
+ * mel_filters_host is fp32 [201, n_mels]; every [.., 128] / [.., 128, ..] shape above has n_mels in place of 128, so an
+ * 80-bin frame is one 160-byte row of the time-major output.  The tables are laid out per count: launch with the count
+ * they were initialised for.  tw_logmel_tables_bytes() covers either layout. */
+int tw_logmel_init_n(void* tables_dev, const float* mel_filters_host, int32_t n_mels);
+int tw_logmel_n(const void* tables_dev, const float* pcm, int64_t pcm_stride, const int32_t* n_valid,
+                int32_t batch, void* scratch, float* out_f32, void* out_bf16_t,
+                int64_t out_t_bstride, int32_t out_t_row_off, int32_t n_mels, void* stream);
+int tw_logmel_long_n(const void* tables_dev, const float* pcm_long, int64_t hop_samples, int32_t n_windows,
+                     const int32_t* frame_lo, const int32_t* frame_hi, const int32_t* out_row0, uint32_t* max_scratch,
+                     void* out_bf16_t, int64_t total_frames, int32_t out_t_row_off, int32_t n_mels, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * K4  LayerNorm over the last dimension, fp32 in -> bf16 out (eps as nn.LayerNorm, 1e-5).

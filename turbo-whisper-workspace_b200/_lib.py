@@ -65,6 +65,11 @@ SIGNATURES = {
                             c_int64, c_int32, c_void_p]),
     "tw_logmel_long": (C.c_int, [c_void_p, c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                  c_int64, c_int32, c_void_p]),
+    "tw_logmel_init_n": (C.c_int, [c_void_p, c_void_p, c_int32]),
+    "tw_logmel_n": (C.c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int32, c_void_p, c_void_p, c_void_p,
+                              c_int64, c_int32, c_int32, c_void_p]),
+    "tw_logmel_long_n": (C.c_int, [c_void_p, c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                   c_int64, c_int32, c_int32, c_void_p]),
     "tw_layernorm": (C.c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_float, c_void_p]),
     "tw_gemm_bf16": (C.c_int, [C.POINTER(GemmArgs), c_void_p]),
     "tw_attention_enc": (C.c_int, [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int64, c_void_p]),

@@ -1,13 +1,16 @@
 """Model dimensions and generation settings of the Whisper checkpoints the path serves.
 
 Mirrors the fields of ``WhisperConfig`` / ``generation_config.json`` that the hot path reads
-(SURVEY.md §8: large-v3-turbo = 32 encoder / 4 decoder layers, large-v3 = 32 / 32)."""
+(SURVEY.md §8: large-v3-turbo = 32 encoder / 4 decoder layers, large-v3 = 32 / 32).  The 128-mel checkpoints
+(large-v3, large-v3-turbo, distil-large-v3) and the multilingual 80-mel ones (large-v2, distil-large-v2, medium, small,
+base) are served; ``n_mels`` carries the difference down to the log-mel kernels and the conv stem."""
 from __future__ import annotations
 
 from dataclasses import dataclass, field
 from typing import Dict, List, Optional
 
 N_SAMPLES = 480000   # 30 s at 16 kHz
+MEL_BINS = (80, 128)  # filterbank sizes the log-mel kernels are built for
 N_FRAMES = 3000      # mel frames per window
 SAMPLING_RATE = 16000
 
@@ -46,8 +49,10 @@ class WhisperDims:
             raise ValueError("turbo-whisper-workspace_b200 kernels are built for head_dim 64")
         if self.d_model % 256 or self.ffn % 256:
             raise ValueError("d_model and ffn must be multiples of 256")
-        if self.n_mels != 128 or self.max_source_positions != 1500:
-            raise ValueError("the log-mel / conv-stem kernels are built for 128 mel bins and 1500 source positions")
+        if self.n_mels not in MEL_BINS:
+            raise ValueError(f"the log-mel kernels are built for 80 or 128 mel bins, not {self.n_mels}")
+        if self.max_source_positions != 1500:
+            raise ValueError("the conv-stem kernels are built for 1500 source positions")
         if self.max_target_positions > 448:
             raise ValueError("max_target_positions > 448 is not supported")
 
@@ -58,6 +63,24 @@ class WhisperDims:
     @classmethod
     def large_v3(cls) -> "WhisperDims":
         return cls(dec_layers=32)
+
+    # the 80-mel checkpoints: openai/whisper-large-v2 (distil-whisper/distil-large-v2 is large_v2() with 2 decoder
+    # layers), openai/whisper-medium, -small and -base; their vocabulary has 51865 ids (no <|yue|>)
+    @classmethod
+    def large_v2(cls) -> "WhisperDims":
+        return cls(dec_layers=32, n_mels=80, vocab=51865)
+
+    @classmethod
+    def medium(cls) -> "WhisperDims":
+        return cls(d_model=1024, heads=16, ffn=4096, enc_layers=24, dec_layers=24, n_mels=80, vocab=51865)
+
+    @classmethod
+    def small(cls) -> "WhisperDims":
+        return cls(d_model=768, heads=12, ffn=3072, enc_layers=12, dec_layers=12, n_mels=80, vocab=51865)
+
+    @classmethod
+    def base(cls) -> "WhisperDims":
+        return cls(d_model=512, heads=8, ffn=2048, enc_layers=6, dec_layers=6, n_mels=80, vocab=51865)
 
     @classmethod
     def from_hf_config(cls, cfg) -> "WhisperDims":

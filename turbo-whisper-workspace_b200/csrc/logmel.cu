@@ -2,17 +2,19 @@
 //
 // Replaces WhisperFeatureExtractor._torch_extract_fbank_features
 // ($TF/models/whisper/feature_extraction_whisper.py:135-164): reflect-padded 400-point STFT at
-// hop 160 with a periodic Hann window, power spectrum, 128-bin slaney mel filterbank, log10 clamp
-// at 1e-10, per-clip `max - 8` floor and (x + 4) / 4.
+// hop 160 with a periodic Hann window, power spectrum, slaney mel filterbank, log10 clamp at 1e-10,
+// per-clip `max - 8` floor and (x + 4) / 4.  The bin count is a template parameter: 128 (large-v3 family) or 80
+// (large-v2 and older, WhisperFeatureExtractor(feature_size=80)); see MelLayout.
 //
 // logmel_kernel: a CTA owns FR = 32 consecutive frames of one clip.  The 5360 samples they touch are staged once in
 // shared memory (coalesced; reflect padding and the zero tail are index arithmetic), then every WARP works alone on
 // its 4 frames, one frame at a time, in a private shared-memory workspace — the 400-point real FFT as a 200-point
-// complex Stockham FFT (radix 8, 5, 5), the real post-process + power, the sparse (<= 12 taps) mel projection, log10 —
-// with __syncwarp between the phases and NO block-wide barrier in the loop (the previous version ran the phases
+// complex Stockham FFT (radix 8, 5, 5), the real post-process + power, the sparse (<= TAPS taps) mel projection,
+// log10 — with __syncwarp between the phases and NO block-wide barrier in the loop (the previous version ran the phases
 // CTA-wide behind six __syncthreads per 16 frames and was latency-bound at 0.07 of HBM).  Lane l owns mel bins
-// 4l..4l+3, so a frame's 128 bf16 values leave as one coalesced 256-byte row of the time-major layout the conv stem's
-// TMA view reads (and, for the reference layout, as float4 runs of 4 frames).
+// 4l..4l+3, so a frame's bf16 values leave as one coalesced row of the time-major layout the conv stem's TMA view reads
+// (256 bytes from 32 lanes at 128 bins, 160 bytes from lanes 0-19 at 80 bins; for the reference layout, as float4 runs
+// of 4 frames).  The FFT phases, the staging and the floor do not depend on the bin count.
 // The per-clip floor needs the maximum over the WHOLE clip.  (x + 4) / 4 and the bf16 rounding are monotone, so
 //   (max(l, m - 8) + 4) / 4 == max((l + 4) / 4, ((m - 8) + 4) / 4)      bit for bit,
 // i.e. the kernel can store the un-floored value right away, publish its tile's max / min (ordered-int atomicMax, a
@@ -32,7 +34,6 @@ namespace logmel {
 constexpr int N_FFT = 400;
 constexpr int HOP = 160;
 constexpr int N_BINS = 201;
-constexpr int N_MEL = 128;
 constexpr int N_FRAMES = 3000;
 constexpr int N_SAMPLES = 480000;
 constexpr int NC = 200;  // complex FFT length
@@ -42,27 +43,40 @@ constexpr int NWARP = NT / 32;
 constexpr int FPW = FR / NWARP;               // consecutive frames per warp
 constexpr int SX = FR * HOP + (N_FFT - HOP);  // 5360 staged samples
 constexpr int POW_LD = 203;                   // padded row length of the power buffer
-constexpr int MEL_MAX_TAPS = 12;
 constexpr int N_TILES = (N_FRAMES + FR - 1) / FR;   // 94 CTAs per clip
 constexpr int NCP = NC + NC / 16 + 1;               // padded FFT workspace length (213), see padi()
 
-struct Tables {
+// The two filterbanks the kernels are built for.  TAPS bounds the non-zero span of one slaney filter over the 201 FFT
+// bins (at most 9 at 128 bins, 14 at 80 bins).  Lane l of a warp owns bins 4l..4l+3: all 32 lanes at 128 bins, lanes
+// 0-19 at 80 bins (lanes 20-31 skip the mel phase).
+template <int NMEL>
+struct MelLayout {
+    static_assert(NMEL == 128 || NMEL == 80, "log-mel kernels are built for 128 or 80 mel bins");
+    static constexpr int TAPS = NMEL == 128 ? 12 : 14;
+    static constexpr int LANES = NMEL / 4;
+};
+
+template <int NMEL>
+struct MelTables {
+    static constexpr int TAPS = MelLayout<NMEL>::TAPS;
     float2 tw200[NC];       // exp(-2 pi i m / 200)
     float2 tw400[N_BINS];   // exp(-2 pi i k / 400)
     float window[N_FFT];    // periodic Hann
-    int mel_start[N_MEL];
-    int mel_cnt[N_MEL];
-    float mel_w[N_MEL][MEL_MAX_TAPS];
+    int mel_start[NMEL];
+    int mel_cnt[NMEL];
+    float mel_w[NMEL][TAPS];
 };
 
-struct Smem {
+template <int NMEL>
+struct MelSmem {
+    static constexpr int TAPS = MelLayout<NMEL>::TAPS;
     float x[SX];
     float2 a[NWARP][NCP];     // per-warp FFT ping (padded, see padi)
     float2 b[NWARP][NCP];     // per-warp FFT pong, then the power spectrum (N_BINS floats)
     float2 tw200[NC];
     float2 tw400[N_BINS];
     float window[N_FFT];
-    float4 mel_w4[MEL_MAX_TAPS][32];   // [tap][lane] = the tap's weight for mel bins 4*lane .. 4*lane+3 (one LDS.128, no conflicts)
+    float4 mel_w4[TAPS][32];           // [tap][lane] = the tap's weight for mel bins 4*lane .. 4*lane+3 (one LDS.128, no conflicts)
     int4 mel_start4[32];               // [lane] = first FFT bin of those four filters
     float red[2][NWARP];
 };
@@ -174,7 +188,8 @@ HD void phase_power(int tid, int nt, const float2* tw400, const float2* Z, float
     }
 }
 // phase 5: one mel bin of one frame: sparse projection + log10 clamp
-HD float mel_log10(int m, const int* mel_start, const int* mel_cnt, const float (*mel_w)[MEL_MAX_TAPS], const float* pw) {
+template <int TAPS>
+HD float mel_log10(int m, const int* mel_start, const int* mel_cnt, const float (*mel_w)[TAPS], const float* pw) {
     const int s = mel_start[m], c = mel_cnt[m];
     float acc = 0.0f;
     for (int i = 0; i < c; ++i) acc = fmaf(mel_w[m][i], pw[s + i], acc);
@@ -196,29 +211,58 @@ struct Scratch {            // per clip; zero-filled once by the owner, re-armed
     float tile_max[N_TILES];
 };
 
+// Fills the table part of the shared memory: twiddles, window, and the filterbank transposed to [tap][lane] float4s.
+template <int NMEL>
+TW_DEVINL void load_tables(int tid, const MelTables<NMEL>* __restrict__ tab, MelSmem<NMEL>& s) {
+    constexpr int TAPS = MelLayout<NMEL>::TAPS, LANES = MelLayout<NMEL>::LANES;
+    for (int i = tid; i < NC; i += NT) s.tw200[i] = tab->tw200[i];
+    for (int i = tid; i < N_BINS; i += NT) s.tw400[i] = tab->tw400[i];
+    for (int i = tid; i < N_FFT; i += NT) s.window[i] = tab->window[i];
+    for (int i = tid; i < TAPS * 32; i += NT) {
+        const int tap = i >> 5, l = i & 31;
+        if (l < LANES)
+            s.mel_w4[tap][l] = make_float4(tab->mel_w[4 * l][tap], tab->mel_w[4 * l + 1][tap], tab->mel_w[4 * l + 2][tap],
+                                           tab->mel_w[4 * l + 3][tap]);
+    }
+    if (tid < LANES) s.mel_start4[tid] = make_int4(tab->mel_start[4 * tid], tab->mel_start[4 * tid + 1], tab->mel_start[4 * tid + 2],
+                                                   tab->mel_start[4 * tid + 3]);
+}
+
+// Sparse mel projection of the four bins 4*lane .. 4*lane+3 of the frame whose power spectrum is pw: taps beyond a
+// filter's length carry weight 0 (same fmaf order as mel_log10, so the sums are identical to the host emulation's).
+template <int NMEL>
+TW_DEVINL void mel_project(int lane, const MelSmem<NMEL>& s, const float* pw, float (&acc)[4]) {
+    const int4 st4 = s.mel_start4[lane];
+#pragma unroll
+    for (int q = 0; q < 4; ++q) acc[q] = 0.f;
+#pragma unroll
+    for (int tp = 0; tp < MelLayout<NMEL>::TAPS; ++tp) {
+        const float4 w = s.mel_w4[tp][lane];
+        acc[0] = fmaf(w.x, pw[min(st4.x + tp, N_BINS - 1)], acc[0]);
+        acc[1] = fmaf(w.y, pw[min(st4.y + tp, N_BINS - 1)], acc[1]);
+        acc[2] = fmaf(w.z, pw[min(st4.z + tp, N_BINS - 1)], acc[2]);
+        acc[3] = fmaf(w.w, pw[min(st4.w + tp, N_BINS - 1)], acc[3]);
+    }
+}
+// log10 through the hardware log2 (abs. error < 2e-7 here, the stated tolerance is 1e-4)
+TW_DEVINL float fast_log10(float acc) { return __log2f(fmaxf(acc, 1e-10f)) * 0.30102999566398120f; }
+
+template <int NMEL>
 __global__ void __launch_bounds__(NT) logmel_kernel(const float* __restrict__ pcm, long long pcm_stride,
-                                                   const int* __restrict__ n_valid, const Tables* __restrict__ tab,
+                                                   const int* __restrict__ n_valid, const MelTables<NMEL>* __restrict__ tab,
                                                    Scratch* __restrict__ scratch, float* __restrict__ out_f32,
                                                    __nv_bfloat16* __restrict__ out_t, long long out_t_bstride,
                                                    int row_off) {
+    constexpr int LANES = MelLayout<NMEL>::LANES;
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    Smem& s = *reinterpret_cast<Smem*>(smem_raw);
+    MelSmem<NMEL>& s = *reinterpret_cast<MelSmem<NMEL>*>(smem_raw);
     __shared__ int s_last;
     const int b = blockIdx.y, tile = blockIdx.x;
     const int f0 = tile * FR;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int nv = n_valid ? min(n_valid[b], N_SAMPLES) : N_SAMPLES;
 
-    for (int i = tid; i < NC; i += NT) s.tw200[i] = tab->tw200[i];
-    for (int i = tid; i < N_BINS; i += NT) s.tw400[i] = tab->tw400[i];
-    for (int i = tid; i < N_FFT; i += NT) s.window[i] = tab->window[i];
-    for (int i = tid; i < MEL_MAX_TAPS * 32; i += NT) {
-        const int tap = i >> 5, l = i & 31;
-        s.mel_w4[tap][l] = make_float4(tab->mel_w[4 * l][tap], tab->mel_w[4 * l + 1][tap], tab->mel_w[4 * l + 2][tap],
-                                       tab->mel_w[4 * l + 3][tap]);
-    }
-    if (tid < 32) s.mel_start4[tid] = make_int4(tab->mel_start[4 * tid], tab->mel_start[4 * tid + 1], tab->mel_start[4 * tid + 2],
-                                                tab->mel_start[4 * tid + 3]);
+    load_tables<NMEL>(tid, tab, s);
     phase_load(tid, NT, pcm + (size_t)b * pcm_stride, nv, f0, s.x);
     __syncthreads();
 
@@ -228,7 +272,7 @@ __global__ void __launch_bounds__(NT) logmel_kernel(const float* __restrict__ pc
     float* pw = reinterpret_cast<float*>(wb);
     float vmax = -INFINITY, vmin = INFINITY;
     float keep[FPW][4];                       // reference-layout output: 4 mel rows x FPW consecutive frames per lane
-    float* of = out_f32 ? out_f32 + ((size_t)b * N_MEL + 4 * lane) * N_FRAMES : nullptr;
+    float* of = (out_f32 && lane < LANES) ? out_f32 + ((size_t)b * NMEL + 4 * lane) * N_FRAMES : nullptr;
     __nv_bfloat16* ot = out_t ? out_t + (size_t)b * out_t_bstride : nullptr;
 #pragma unroll
     for (int i = 0; i < FPW; ++i) {
@@ -243,33 +287,23 @@ __global__ void __launch_bounds__(NT) logmel_kernel(const float* __restrict__ pc
             __syncwarp();
             phase_power(lane, 32, s.tw400, wa, pw);
             __syncwarp();
-            // sparse mel projection of this lane's four bins: taps beyond a filter's length carry weight 0 (same fmaf order
-            // as mel_log10, so the sums are identical to the host emulation's)
-            const int4 st4 = s.mel_start4[lane];
-            float acc[4] = {0.f, 0.f, 0.f, 0.f};
+            if (lane < LANES) {               // all lanes at 128 bins
+                float acc[4], y[4];
+                mel_project<NMEL>(lane, s, pw, acc);
 #pragma unroll
-            for (int tp = 0; tp < MEL_MAX_TAPS; ++tp) {
-                const float4 w = s.mel_w4[tp][lane];
-                acc[0] = fmaf(w.x, pw[min(st4.x + tp, N_BINS - 1)], acc[0]);
-                acc[1] = fmaf(w.y, pw[min(st4.y + tp, N_BINS - 1)], acc[1]);
-                acc[2] = fmaf(w.z, pw[min(st4.z + tp, N_BINS - 1)], acc[2]);
-                acc[3] = fmaf(w.w, pw[min(st4.w + tp, N_BINS - 1)], acc[3]);
-            }
-            float y[4];
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-                // log10 through the hardware log2 (abs. error < 2e-7 here, the stated tolerance is 1e-4)
-                const float l = __log2f(fmaxf(acc[q], 1e-10f)) * 0.30102999566398120f;
-                vmax = fmaxf(vmax, l);
-                vmin = fminf(vmin, l);
-                y[q] = scaled(l);
-                keep[i][q] = y[q];
-            }
-            if (ot) {
-                uint2 pk;
-                pk.x = pack_bf16x2(y[0], y[1]);
-                pk.y = pack_bf16x2(y[2], y[3]);
-                reinterpret_cast<uint2*>(ot + (size_t)(row_off + f) * N_MEL)[lane] = pk;
+                for (int q = 0; q < 4; ++q) {
+                    const float l = fast_log10(acc[q]);
+                    vmax = fmaxf(vmax, l);
+                    vmin = fminf(vmin, l);
+                    y[q] = scaled(l);
+                    keep[i][q] = y[q];
+                }
+                if (ot) {
+                    uint2 pk;
+                    pk.x = pack_bf16x2(y[0], y[1]);
+                    pk.y = pack_bf16x2(y[2], y[3]);
+                    reinterpret_cast<uint2*>(ot + (size_t)(row_off + f) * NMEL)[lane] = pk;
+                }
             }
             __syncwarp();                     // pw (= wb) and wa are reused by the next frame
         } else {
@@ -318,9 +352,9 @@ __global__ void __launch_bounds__(NT) logmel_kernel(const float* __restrict__ pc
     for (int t = 0; t < (int)gridDim.x; ++t) {
         if (!(__ldcg(&sc.tile_min[t]) < floor_l)) continue;      // block-uniform
         const int tf0 = t * FR, nfr = min(FR, N_FRAMES - tf0);
-        if (ot) {   // nfr rows of 128 bf16, contiguous: 16 uint4 per row
-            uint4* base = reinterpret_cast<uint4*>(ot + (size_t)(row_off + tf0) * N_MEL);
-            for (int i = tid; i < nfr * 16; i += NT) {
+        if (ot) {   // nfr rows of NMEL bf16, contiguous: NMEL / 8 uint4 per row
+            uint4* base = reinterpret_cast<uint4*>(ot + (size_t)(row_off + tf0) * NMEL);
+            for (int i = tid; i < nfr * (NMEL / 8); i += NT) {
                 uint4 v = __ldcg(base + i);
                 uint32_t* w = reinterpret_cast<uint32_t*>(&v);
                 bool changed = false;
@@ -335,8 +369,8 @@ __global__ void __launch_bounds__(NT) logmel_kernel(const float* __restrict__ pc
             }
         }
         if (out_f32) {
-            float* fb = out_f32 + (size_t)b * N_MEL * N_FRAMES + tf0;
-            for (int i = tid; i < N_MEL * nfr; i += NT) {
+            float* fb = out_f32 + (size_t)b * NMEL * N_FRAMES + tf0;
+            for (int i = tid; i < NMEL * nfr; i += NT) {
                 const int m = i / nfr, fr = i - m * nfr;
                 float* p = fb + (size_t)m * N_FRAMES + fr;
                 if (__ldcg(p) < floor_y) *p = floor_y;
@@ -354,29 +388,22 @@ __global__ void __launch_bounds__(NT) logmel_kernel(const float* __restrict__ pc
 // window that does not touch the window's own reflect padding equals the clip's frame; window b contributes its frames
 // [frame_lo[b], frame_hi[b]) to rows out_row0[b].. of the clip's time-major output.  The clamp uses the maximum of the
 // WHOLE clip: this kernel stores un-floored values and raises ONE maximum, logmel_floor_kernel applies the floor.
+template <int NMEL>
 __global__ void __launch_bounds__(NT) logmel_long_kernel(const float* __restrict__ pcm, long long hop_samples,
-                                                        const Tables* __restrict__ tab, const int* __restrict__ frame_lo,
+                                                        const MelTables<NMEL>* __restrict__ tab, const int* __restrict__ frame_lo,
                                                         const int* __restrict__ frame_hi, const int* __restrict__ out_row0,
                                                         unsigned int* __restrict__ long_max,
                                                         __nv_bfloat16* __restrict__ out_t, int row_off) {
+    constexpr int LANES = MelLayout<NMEL>::LANES;
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    Smem& s = *reinterpret_cast<Smem*>(smem_raw);
+    MelSmem<NMEL>& s = *reinterpret_cast<MelSmem<NMEL>*>(smem_raw);
     const int b = blockIdx.y, tile = blockIdx.x;
     const int f0 = tile * FR;
     const int lo = frame_lo[b], hi = frame_hi[b];
     if (f0 + FR <= lo || f0 >= hi) return;       // block-uniform: no frame of this tile belongs to the window's share
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
 
-    for (int i = tid; i < NC; i += NT) s.tw200[i] = tab->tw200[i];
-    for (int i = tid; i < N_BINS; i += NT) s.tw400[i] = tab->tw400[i];
-    for (int i = tid; i < N_FFT; i += NT) s.window[i] = tab->window[i];
-    for (int i = tid; i < MEL_MAX_TAPS * 32; i += NT) {
-        const int tap = i >> 5, l = i & 31;
-        s.mel_w4[tap][l] = make_float4(tab->mel_w[4 * l][tap], tab->mel_w[4 * l + 1][tap], tab->mel_w[4 * l + 2][tap],
-                                       tab->mel_w[4 * l + 3][tap]);
-    }
-    if (tid < 32) s.mel_start4[tid] = make_int4(tab->mel_start[4 * tid], tab->mel_start[4 * tid + 1], tab->mel_start[4 * tid + 2],
-                                                tab->mel_start[4 * tid + 3]);
+    load_tables<NMEL>(tid, tab, s);
     phase_load(tid, NT, pcm + (size_t)b * hop_samples, N_SAMPLES, f0, s.x);
     __syncthreads();
 
@@ -384,7 +411,7 @@ __global__ void __launch_bounds__(NT) logmel_long_kernel(const float* __restrict
     float2* wb = s.b[warp];
     float* pw = reinterpret_cast<float*>(wb);
     float vmax = -INFINITY;
-    __nv_bfloat16* ot = out_t + (size_t)(row_off + out_row0[b] - lo) * N_MEL;    // row of window frame 0 (may lie before row 0)
+    __nv_bfloat16* ot = out_t + (size_t)(row_off + out_row0[b] - lo) * NMEL;     // row of window frame 0 (may lie before row 0)
 #pragma unroll
     for (int i = 0; i < FPW; ++i) {
         const int fl = warp * FPW + i;
@@ -398,27 +425,20 @@ __global__ void __launch_bounds__(NT) logmel_long_kernel(const float* __restrict
             __syncwarp();
             phase_power(lane, 32, s.tw400, wa, pw);
             __syncwarp();
-            const int4 st4 = s.mel_start4[lane];
-            float acc[4] = {0.f, 0.f, 0.f, 0.f};
+            if (lane < LANES) {               // all lanes at 128 bins
+                float acc[4], y[4];
+                mel_project<NMEL>(lane, s, pw, acc);
 #pragma unroll
-            for (int tp = 0; tp < MEL_MAX_TAPS; ++tp) {
-                const float4 w = s.mel_w4[tp][lane];
-                acc[0] = fmaf(w.x, pw[min(st4.x + tp, N_BINS - 1)], acc[0]);
-                acc[1] = fmaf(w.y, pw[min(st4.y + tp, N_BINS - 1)], acc[1]);
-                acc[2] = fmaf(w.z, pw[min(st4.z + tp, N_BINS - 1)], acc[2]);
-                acc[3] = fmaf(w.w, pw[min(st4.w + tp, N_BINS - 1)], acc[3]);
+                for (int q = 0; q < 4; ++q) {
+                    const float l = fast_log10(acc[q]);
+                    vmax = fmaxf(vmax, l);
+                    y[q] = scaled(l);
+                }
+                uint2 pk;
+                pk.x = pack_bf16x2(y[0], y[1]);
+                pk.y = pack_bf16x2(y[2], y[3]);
+                reinterpret_cast<uint2*>(ot + (size_t)f * NMEL)[lane] = pk;
             }
-            float y[4];
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-                const float l = __log2f(fmaxf(acc[q], 1e-10f)) * 0.30102999566398120f;
-                vmax = fmaxf(vmax, l);
-                y[q] = scaled(l);
-            }
-            uint2 pk;
-            pk.x = pack_bf16x2(y[0], y[1]);
-            pk.y = pack_bf16x2(y[2], y[3]);
-            reinterpret_cast<uint2*>(ot + (size_t)f * N_MEL)[lane] = pk;
             __syncwarp();
         }
     }
@@ -434,7 +454,7 @@ __global__ void __launch_bounds__(NT) logmel_long_kernel(const float* __restrict
 }
 
 // raise every value below the clip's floor (max - 8 in log10 units, compared after the bf16 rounding of the output, like
-// the floor pass of logmel_kernel)
+// the floor pass of logmel_kernel).  It sees the output as a flat run of uint4, so one kernel serves both bin counts.
 __global__ void __launch_bounds__(256) logmel_floor_kernel(uint4* __restrict__ mel, long long n_vec,
                                                           const unsigned int* __restrict__ long_max) {
     const float floor_y = scaled_floor(umono_to_float(*long_max));
@@ -456,34 +476,44 @@ __global__ void __launch_bounds__(256) logmel_floor_kernel(uint4* __restrict__ m
 }
 #endif  // TW_HOST_TEST
 
-// Host: build the constant tables from the dense [201,128] fp32 filterbank (HF mel_filters).
-int build_tables(const float* mel_filters_201x128, Tables* t) {
+// Host: build the constant tables from the dense [201, NMEL] fp32 filterbank (HF mel_filters).
+template <int NMEL>
+int build_tables(const float* mel_filters, MelTables<NMEL>* t) {
+    constexpr int TAPS = MelLayout<NMEL>::TAPS;
     const double PI = 3.14159265358979323846;
     for (int m = 0; m < NC; ++m)
         t->tw200[m] = make_float2((float)cos(2.0 * PI * m / NC), (float)-sin(2.0 * PI * m / NC));
     for (int k = 0; k < N_BINS; ++k)
         t->tw400[k] = make_float2((float)cos(2.0 * PI * k / N_FFT), (float)-sin(2.0 * PI * k / N_FFT));
     for (int n = 0; n < N_FFT; ++n) t->window[n] = (float)(0.5 - 0.5 * cos(2.0 * PI * n / N_FFT));
-    for (int m = 0; m < N_MEL; ++m) {
+    for (int m = 0; m < NMEL; ++m) {
         int first = -1, last = -1;
         for (int k = 0; k < N_BINS; ++k)
-            if (mel_filters_201x128[k * N_MEL + m] != 0.0f) {
+            if (mel_filters[k * NMEL + m] != 0.0f) {
                 if (first < 0) first = k;
                 last = k;
             }
         if (first < 0) { first = 0; last = -1; }
         const int cnt = last - first + 1;
-        if (cnt > MEL_MAX_TAPS) {
-            set_error("mel filter %d has %d taps (max %d)", m, cnt, MEL_MAX_TAPS);
+        if (cnt > TAPS) {
+            set_error("mel filter %d has %d taps (max %d)", m, cnt, TAPS);
             return 2;
         }
         t->mel_start[m] = first;
         t->mel_cnt[m] = cnt;
-        for (int i = 0; i < MEL_MAX_TAPS; ++i)
-            t->mel_w[m][i] = (i < cnt) ? mel_filters_201x128[(first + i) * N_MEL + m] : 0.0f;
+        for (int i = 0; i < TAPS; ++i)
+            t->mel_w[m][i] = (i < cnt) ? mel_filters[(first + i) * NMEL + m] : 0.0f;
     }
     return 0;
 }
+
+#ifdef TW_HOST_TEST
+// The names tests/csrc/logmel_host_test.cu is written against: the 128-bin layout.
+constexpr int N_MEL = 128;
+constexpr int MEL_MAX_TAPS = MelLayout<N_MEL>::TAPS;
+using Tables = MelTables<N_MEL>;
+using Smem = MelSmem<N_MEL>;
+#endif
 
 }  // namespace logmel
 }  // namespace tw
@@ -492,15 +522,19 @@ int build_tables(const float* mel_filters_201x128, Tables* t) {
 using namespace tw;
 using namespace tw::logmel;
 
-extern "C" size_t tw_logmel_tables_bytes(void) { return sizeof(Tables); }
+extern "C" size_t tw_logmel_tables_bytes(void) { return std::max(sizeof(MelTables<128>), sizeof(MelTables<80>)); }
 extern "C" size_t tw_logmel_scratch_bytes(int batch) { return (size_t)batch * sizeof(Scratch); }
 
-extern "C" int tw_logmel_init(void* tables_dev, const float* mel_filters_host_201x128) {
-    TW_REQUIRE(tables_dev && mel_filters_host_201x128, "tw_logmel_init: null argument");
-    Tables* h = new Tables;
-    int rc = build_tables(mel_filters_host_201x128, h);
+#define TW_REQUIRE_N_MELS(fn, n)                                                                        \
+    TW_REQUIRE((n) == 128 || (n) == 80, fn ": n_mels %d is not supported (the kernels are built for 80 and 128)", (int)(n))
+
+namespace {
+template <int NMEL>
+int logmel_init(void* tables_dev, const float* mel_filters) {
+    MelTables<NMEL>* h = new MelTables<NMEL>;
+    int rc = build_tables<NMEL>(mel_filters, h);
     if (rc == 0) {
-        cudaError_t e = cudaMemcpy(tables_dev, h, sizeof(Tables), cudaMemcpyHostToDevice);
+        cudaError_t e = cudaMemcpy(tables_dev, h, sizeof(MelTables<NMEL>), cudaMemcpyHostToDevice);
         if (e != cudaSuccess) {
             set_error("tw_logmel_init: cudaMemcpy failed: %s", cudaGetErrorString(e));
             rc = 1;
@@ -510,11 +544,63 @@ extern "C" int tw_logmel_init(void* tables_dev, const float* mel_filters_host_20
     return rc;
 }
 
-extern "C" int tw_logmel(const void* tables_dev, const float* pcm, int64_t pcm_stride,
-                         const int32_t* n_valid, int batch, void* scratch, float* out_f32,
-                         void* out_bf16_t, int64_t out_t_bstride, int32_t out_t_row_off,
-                         void* stream) {
+template <int NMEL>
+int logmel_launch(const void* tables_dev, const float* pcm, int64_t pcm_stride, const int32_t* n_valid, int batch,
+                  void* scratch, float* out_f32, void* out_bf16_t, int64_t out_t_bstride, int32_t out_t_row_off,
+                  cudaStream_t stream) {
+    static std::atomic<unsigned long long> attr_done{0};
+    if (device_needs_setup(attr_done)) {
+        TW_CUDA_CHECK(cudaFuncSetAttribute(logmel_kernel<NMEL>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                           (int)sizeof(MelSmem<NMEL>)));
+        mark_device_done(attr_done);
+    }
+    logmel_kernel<NMEL><<<dim3(N_TILES, batch), NT, sizeof(MelSmem<NMEL>), stream>>>(
+        pcm, (long long)pcm_stride, n_valid, (const MelTables<NMEL>*)tables_dev, (Scratch*)scratch, out_f32,
+        (__nv_bfloat16*)out_bf16_t, (long long)out_t_bstride, out_t_row_off);
+    TW_CUDA_CHECK(cudaGetLastError());
+    return 0;
+}
+
+template <int NMEL>
+int logmel_long_launch(const void* tables_dev, const float* pcm_long, int64_t hop_samples, int32_t n_windows,
+                       const int32_t* frame_lo, const int32_t* frame_hi, const int32_t* out_row0, uint32_t* max_scratch,
+                       void* out_bf16_t, int64_t total_frames, int32_t out_t_row_off, cudaStream_t st) {
+    static std::atomic<unsigned long long> attr_done{0};
+    if (device_needs_setup(attr_done)) {
+        TW_CUDA_CHECK(cudaFuncSetAttribute(logmel_long_kernel<NMEL>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                           (int)sizeof(MelSmem<NMEL>)));
+        mark_device_done(attr_done);
+    }
+    TW_CUDA_CHECK(cudaMemsetAsync(max_scratch, 0, sizeof(uint32_t), st));     // below every real value in the ordered map
+    logmel_long_kernel<NMEL><<<dim3(N_TILES, n_windows), NT, sizeof(MelSmem<NMEL>), st>>>(
+        pcm_long, (long long)hop_samples, (const MelTables<NMEL>*)tables_dev, frame_lo, frame_hi, out_row0, max_scratch,
+        (__nv_bfloat16*)out_bf16_t, out_t_row_off);
+    TW_CUDA_CHECK(cudaGetLastError());
+    const long long n_vec = (long long)total_frames * NMEL / 8;
+    uint4* first = reinterpret_cast<uint4*>((__nv_bfloat16*)out_bf16_t + (size_t)out_t_row_off * NMEL);
+    const int blocks = (int)std::min<long long>((n_vec + 255) / 256, 148 * 8);
+    logmel_floor_kernel<<<blocks, 256, 0, st>>>(first, n_vec, max_scratch);
+    TW_CUDA_CHECK(cudaGetLastError());
+    return 0;
+}
+}  // namespace
+
+extern "C" int tw_logmel_init_n(void* tables_dev, const float* mel_filters_host, int32_t n_mels) {
+    TW_REQUIRE(tables_dev && mel_filters_host, "tw_logmel_init: null argument");
+    TW_REQUIRE_N_MELS("tw_logmel_init", n_mels);
+    return n_mels == 128 ? logmel_init<128>(tables_dev, mel_filters_host) : logmel_init<80>(tables_dev, mel_filters_host);
+}
+
+extern "C" int tw_logmel_init(void* tables_dev, const float* mel_filters_host_201x128) {
+    return tw_logmel_init_n(tables_dev, mel_filters_host_201x128, 128);
+}
+
+extern "C" int tw_logmel_n(const void* tables_dev, const float* pcm, int64_t pcm_stride,
+                           const int32_t* n_valid, int batch, void* scratch, float* out_f32,
+                           void* out_bf16_t, int64_t out_t_bstride, int32_t out_t_row_off,
+                           int32_t n_mels, void* stream) {
     TW_REQUIRE(tables_dev && pcm && scratch, "tw_logmel: null argument");
+    TW_REQUIRE_N_MELS("tw_logmel", n_mels);
     if (tw::ensure_device(pcm)) return 1;
     TW_REQUIRE(batch >= 0 && batch <= 65535, "tw_logmel: batch %d out of range", batch);
     TW_REQUIRE(pcm_stride >= N_SAMPLES, "tw_logmel: pcm_stride %lld < %d", (long long)pcm_stride,
@@ -523,45 +609,47 @@ extern "C" int tw_logmel(const void* tables_dev, const float* pcm, int64_t pcm_s
                "tw_logmel: the time-major output must be 16-byte aligned");
     TW_REQUIRE(!out_f32 || ((uintptr_t)out_f32 & 15) == 0, "tw_logmel: out_f32 must be 16-byte aligned");
     if (batch == 0) return 0;
-    static std::atomic<unsigned long long> attr_done{0};
-    if (device_needs_setup(attr_done)) {
-        TW_CUDA_CHECK(cudaFuncSetAttribute(logmel_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem)));
-        mark_device_done(attr_done);
-    }
-    logmel_kernel<<<dim3(N_TILES, batch), NT, sizeof(Smem), (cudaStream_t)stream>>>(
-        pcm, (long long)pcm_stride, n_valid, (const Tables*)tables_dev, (Scratch*)scratch, out_f32,
-        (__nv_bfloat16*)out_bf16_t, (long long)out_t_bstride, out_t_row_off);
-    TW_CUDA_CHECK(cudaGetLastError());
-    return 0;
+    cudaStream_t st = (cudaStream_t)stream;
+    return n_mels == 128
+        ? logmel_launch<128>(tables_dev, pcm, pcm_stride, n_valid, batch, scratch, out_f32, out_bf16_t, out_t_bstride,
+                             out_t_row_off, st)
+        : logmel_launch<80>(tables_dev, pcm, pcm_stride, n_valid, batch, scratch, out_f32, out_bf16_t, out_t_bstride,
+                            out_t_row_off, st);
+}
+
+extern "C" int tw_logmel(const void* tables_dev, const float* pcm, int64_t pcm_stride,
+                         const int32_t* n_valid, int batch, void* scratch, float* out_f32,
+                         void* out_bf16_t, int64_t out_t_bstride, int32_t out_t_row_off,
+                         void* stream) {
+    return tw_logmel_n(tables_dev, pcm, pcm_stride, n_valid, batch, scratch, out_f32, out_bf16_t, out_t_bstride,
+                       out_t_row_off, 128, stream);
+}
+
+extern "C" int tw_logmel_long_n(const void* tables_dev, const float* pcm_long, int64_t hop_samples, int32_t n_windows,
+                                const int32_t* frame_lo, const int32_t* frame_hi, const int32_t* out_row0,
+                                uint32_t* max_scratch, void* out_bf16_t, int64_t total_frames, int32_t out_t_row_off,
+                                int32_t n_mels, void* stream) {
+    TW_REQUIRE(tables_dev && pcm_long && frame_lo && frame_hi && out_row0 && max_scratch && out_bf16_t,
+               "tw_logmel_long: null argument");
+    TW_REQUIRE_N_MELS("tw_logmel_long", n_mels);
+    if (tw::ensure_device(pcm_long)) return 1;
+    TW_REQUIRE(n_windows >= 0 && n_windows <= 65535, "tw_logmel_long: %d windows out of range", n_windows);
+    TW_REQUIRE(hop_samples > 0 && hop_samples % HOP == 0, "tw_logmel_long: hop_samples must be a positive multiple of %d", HOP);
+    TW_REQUIRE(((uintptr_t)out_bf16_t & 15) == 0 && total_frames >= 0, "tw_logmel_long: the output must be 16-byte aligned");
+    if (n_windows == 0 || total_frames == 0) return 0;
+    cudaStream_t st = (cudaStream_t)stream;
+    return n_mels == 128
+        ? logmel_long_launch<128>(tables_dev, pcm_long, hop_samples, n_windows, frame_lo, frame_hi, out_row0, max_scratch,
+                                  out_bf16_t, total_frames, out_t_row_off, st)
+        : logmel_long_launch<80>(tables_dev, pcm_long, hop_samples, n_windows, frame_lo, frame_hi, out_row0, max_scratch,
+                                 out_bf16_t, total_frames, out_t_row_off, st);
 }
 
 extern "C" int tw_logmel_long(const void* tables_dev, const float* pcm_long, int64_t hop_samples, int32_t n_windows,
                               const int32_t* frame_lo, const int32_t* frame_hi, const int32_t* out_row0,
                               uint32_t* max_scratch, void* out_bf16_t, int64_t total_frames, int32_t out_t_row_off,
                               void* stream) {
-    TW_REQUIRE(tables_dev && pcm_long && frame_lo && frame_hi && out_row0 && max_scratch && out_bf16_t,
-               "tw_logmel_long: null argument");
-    if (tw::ensure_device(pcm_long)) return 1;
-    TW_REQUIRE(n_windows >= 0 && n_windows <= 65535, "tw_logmel_long: %d windows out of range", n_windows);
-    TW_REQUIRE(hop_samples > 0 && hop_samples % HOP == 0, "tw_logmel_long: hop_samples must be a positive multiple of %d", HOP);
-    TW_REQUIRE(((uintptr_t)out_bf16_t & 15) == 0 && total_frames >= 0, "tw_logmel_long: the output must be 16-byte aligned");
-    if (n_windows == 0 || total_frames == 0) return 0;
-    static std::atomic<unsigned long long> attr_done{0};
-    if (device_needs_setup(attr_done)) {
-        TW_CUDA_CHECK(cudaFuncSetAttribute(logmel_long_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem)));
-        mark_device_done(attr_done);
-    }
-    cudaStream_t st = (cudaStream_t)stream;
-    TW_CUDA_CHECK(cudaMemsetAsync(max_scratch, 0, sizeof(uint32_t), st));     // below every real value in the ordered map
-    logmel_long_kernel<<<dim3(N_TILES, n_windows), NT, sizeof(Smem), st>>>(
-        pcm_long, (long long)hop_samples, (const Tables*)tables_dev, frame_lo, frame_hi, out_row0, max_scratch,
-        (__nv_bfloat16*)out_bf16_t, out_t_row_off);
-    TW_CUDA_CHECK(cudaGetLastError());
-    const long long n_vec = (long long)total_frames * N_MEL / 8;
-    uint4* first = reinterpret_cast<uint4*>((__nv_bfloat16*)out_bf16_t + (size_t)out_t_row_off * N_MEL);
-    const int blocks = (int)std::min<long long>((n_vec + 255) / 256, 148 * 8);
-    logmel_floor_kernel<<<blocks, 256, 0, st>>>(first, n_vec, max_scratch);
-    TW_CUDA_CHECK(cudaGetLastError());
-    return 0;
+    return tw_logmel_long_n(tables_dev, pcm_long, hop_samples, n_windows, frame_lo, frame_hi, out_row0, max_scratch,
+                            out_bf16_t, total_frames, out_t_row_off, 128, stream);
 }
 #endif

@@ -236,7 +236,7 @@ class WhisperEngine:
             self._capture_stream = torch.cuda.Stream(device=dev)
             bf, f32, i32 = torch.bfloat16, torch.float32, torch.int32
             z = lambda *shape, dtype: torch.zeros(*shape, dtype=dtype, device=dev)
-            self.logmel = ops.LogMel(dev, Be)
+            self.logmel = ops.LogMel(dev, Be, dims.n_mels)
             # ---- encoder workspaces
             self.pcm = z(Be, N_SAMPLES, dtype=f32)
             self.n_valid = z(Be, dtype=i32)
@@ -417,7 +417,7 @@ class WhisperEngine:
         return B
 
     def features(self, B: int, out_f32: Optional[torch.Tensor] = None):
-        """K1: PCM (self.pcm[:B]) -> time-major bf16 features in self.mel_t (and optionally fp32 [B,128,3000])."""
+        """K1: PCM (self.pcm[:B]) -> time-major bf16 features in self.mel_t (and optionally fp32 [B, n_mels, 3000])."""
         self.logmel(self.pcm[:B], self.n_valid[:B], out_f32=out_f32, out_t=self.mel_t, out_t_row_off=1)
         self.stats["launches"] += 1
 
@@ -432,7 +432,8 @@ class WhisperEngine:
         mel = self.mel_t if mel is None else mel
         C1 = d.n_mels
         with torch.cuda.device(self.device):
-            # conv1 (k=3, pad 1) + GELU: A row t = [x[t-1], x[t], x[t+1]] = 3*128 contiguous elements of the padded buffer
+            # conv1 (k=3, pad 1) + GELU: A row t = [x[t-1], x[t], x[t+1]] = 3*n_mels contiguous elements of the padded buffer
+            # (K = 240 at 80 mels: the TMA box reads zeros past K in the last 64-wide k-block)
             ops.gemm(mel, w["conv1_w"], rows=T, batches=B, a_row_stride=C1, a_batch_stride=(T + 2) * C1, a_rows=T,
                      bias=w["conv1_b"], act=1, out=self.h1, out_ld=D, out_batch_rows=T + 2, out_row_off=1)
             # conv2 (k=3, stride 2, pad 1) + GELU + positional embedding -> fp32 residual stream
@@ -915,7 +916,7 @@ class WhisperEngine:
         fp32 time per returned id (seek offset added, as `segments[...]["token_timestamps"]` of HF's generate;
         ``self.last_token_ts_raw[b]`` = the padded `token_timestamps` output, no offset).
 
-        ``long_mel`` (bf16 [T, 128], T > 3000, B == 1): HF's long-form mode — the loop runs over T frames and every
+        ``long_mel`` (bf16 [T, n_mels], T > 3000, B == 1): HF's long-form mode — the loop runs over T frames and every
         iteration's window is gathered from ``long_mel`` (zero-padded to 3000 frames, _get_input_segment :1831-1850)."""
         gen = self.gen
         if long_mel is not None:

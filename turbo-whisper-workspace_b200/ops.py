@@ -13,7 +13,7 @@ import torch
 from . import _lib
 from ._lib import GemmArgs, check
 
-N_SAMPLES, N_MELS, N_FRAMES = 480000, 128, 3000
+N_SAMPLES, N_FRAMES = 480000, 3000
 
 
 def _ptr(t):
@@ -30,10 +30,10 @@ def _need_cuda(*ts):
             raise _lib.TwError("turbo-whisper-workspace_b200 operators need CUDA tensors (no CPU path)")
 
 
-def slaney_mel_filters() -> np.ndarray:
-    """[201,128] fp32 — the filterbank WhisperFeatureExtractor(feature_size=128) builds
+def slaney_mel_filters(n_mels: int = 128) -> np.ndarray:
+    """[201, n_mels] fp32 — the filterbank WhisperFeatureExtractor(feature_size=n_mels) builds
     ($TF/models/whisper/feature_extraction_whisper.py:95-103; $TF/audio_utils.py:453-544):
-    128 triangular filters on the slaney mel scale over 0-8 kHz, slaney area normalisation."""
+    n_mels triangular filters on the slaney mel scale over 0-8 kHz, slaney area normalisation."""
     def hz_to_mel(f):
         f = np.asarray(f, dtype=np.float64)
         return np.where(f >= 1000.0, 15.0 + np.log(np.maximum(f, 1e-300) / 1000.0) * (27.0 / np.log(6.4)),
@@ -42,7 +42,7 @@ def slaney_mel_filters() -> np.ndarray:
     def mel_to_hz(m):
         return np.where(m >= 15.0, 1000.0 * np.exp((np.log(6.4) / 27.0) * (m - 15.0)), 200.0 * m / 3.0)
 
-    pts = mel_to_hz(np.linspace(hz_to_mel(0.0), hz_to_mel(8000.0), N_MELS + 2))
+    pts = mel_to_hz(np.linspace(hz_to_mel(0.0), hz_to_mel(8000.0), n_mels + 2))
     bins = np.linspace(0, 8000, 201)
     d = np.diff(pts)
     slopes = pts[None, :] - bins[:, None]
@@ -52,43 +52,45 @@ def slaney_mel_filters() -> np.ndarray:
 
 
 class LogMel:
-    """K1 front end bound to one device: owns the constant tables and the scratch buffer."""
+    """K1 front end bound to one device and one filterbank size (``n_mels``: 128 or 80, the model's
+    ``WhisperDims.n_mels``): owns the constant tables and the scratch buffer."""
 
-    def __init__(self, device, max_batch: int):
+    def __init__(self, device, max_batch: int, n_mels: int = 128):
         lib = _lib.load()
         self.device = torch.device(device)
         self.max_batch = max_batch
+        self.n_mels = n_mels
         self.tables = torch.empty(lib.tw_logmel_tables_bytes(), dtype=torch.uint8, device=self.device)
         # zero-filled ONCE: the kernel keeps its per-clip maximum / arrival counters here and re-arms them itself
         self.scratch = torch.zeros(lib.tw_logmel_scratch_bytes(max_batch), dtype=torch.uint8, device=self.device)
-        fb = slaney_mel_filters()
+        fb = slaney_mel_filters(n_mels)
         with torch.cuda.device(self.device):
-            check(lib.tw_logmel_init(_ptr(self.tables), fb.ctypes.data_as(C.c_void_p)), "tw_logmel_init")
+            check(lib.tw_logmel_init_n(_ptr(self.tables), fb.ctypes.data_as(C.c_void_p), n_mels), "tw_logmel_init_n")
 
     def __call__(self, pcm, n_valid=None, out_f32=None, out_t=None, out_t_row_off: int = 0):
         """pcm: cuda fp32 [B, >=480000]; n_valid: cuda int32 [B] or None.
-        out_f32: cuda fp32 [B,128,3000] or None; out_t: cuda bf16 [B, rows, 128] or None."""
+        out_f32: cuda fp32 [B, n_mels, 3000] or None; out_t: cuda bf16 [B, rows, n_mels] or None."""
         lib = _lib.load()
         _need_cuda(pcm, n_valid, out_f32, out_t)
-        B = pcm.shape[0]
+        B, M = pcm.shape[0], self.n_mels
         if B > self.max_batch:
             raise _lib.TwError(f"batch {B} exceeds LogMel max_batch {self.max_batch}")
         assert pcm.dtype == torch.float32 and pcm.stride(1) == 1
         if out_f32 is not None:
-            assert out_f32.dtype == torch.float32 and out_f32.is_contiguous() and tuple(out_f32.shape) == (B, N_MELS, N_FRAMES)
+            assert out_f32.dtype == torch.float32 and out_f32.is_contiguous() and tuple(out_f32.shape) == (B, M, N_FRAMES)
         tb = 0
         if out_t is not None:
-            assert out_t.dtype == torch.bfloat16 and out_t.shape[0] >= B and out_t.shape[2] == N_MELS and out_t.stride(2) == 1
-            assert out_t.stride(1) == N_MELS and out_t.shape[1] >= out_t_row_off + N_FRAMES
+            assert out_t.dtype == torch.bfloat16 and out_t.shape[0] >= B and out_t.shape[2] == M and out_t.stride(2) == 1
+            assert out_t.stride(1) == M and out_t.shape[1] >= out_t_row_off + N_FRAMES
             tb = out_t.stride(0)
         with torch.cuda.device(self.device):
-            check(lib.tw_logmel(_ptr(self.tables), _ptr(pcm), pcm.stride(0), _ptr(n_valid), B, _ptr(self.scratch),
-                                _ptr(out_f32), _ptr(out_t), tb, out_t_row_off, _stream()), "tw_logmel")
+            check(lib.tw_logmel_n(_ptr(self.tables), _ptr(pcm), pcm.stride(0), _ptr(n_valid), B, _ptr(self.scratch),
+                                  _ptr(out_f32), _ptr(out_t), tb, out_t_row_off, M, _stream()), "tw_logmel_n")
 
 
     def long(self, audio: np.ndarray) -> torch.Tensor:
         """Whole-clip features of one clip longer than 30 s (un-chunked long-form input): host fp32 PCM -> cuda bf16
-        [n // 160, 128], time-major (tw_logmel_long; window plan: :func:`longform_plan`)."""
+        [n // 160, n_mels], time-major (tw_logmel_long_n; window plan: :func:`longform_plan`)."""
         lib = _lib.load()
         audio = np.asarray(audio, dtype=np.float32).reshape(-1)
         plan = longform_plan(audio.shape[0])
@@ -97,10 +99,11 @@ class LogMel:
             pcm = host.to(self.device, non_blocking=False)
             ints = torch.tensor([plan["lo"], plan["hi"], plan["row0"]], dtype=torch.int32).to(self.device)
             mx = torch.zeros(1, dtype=torch.int32, device=self.device)
-            out = torch.empty(plan["frames"], N_MELS, dtype=torch.bfloat16, device=self.device)
-            check(lib.tw_logmel_long(_ptr(self.tables), _ptr(pcm), plan["hop_samples"], len(plan["lo"]), _ptr(ints[0]),
-                                     _ptr(ints[1]), _ptr(ints[2]), _ptr(mx), _ptr(out), plan["frames"], 0, _stream()),
-                  "tw_logmel_long")
+            out = torch.empty(plan["frames"], self.n_mels, dtype=torch.bfloat16, device=self.device)
+            check(lib.tw_logmel_long_n(_ptr(self.tables), _ptr(pcm), plan["hop_samples"], len(plan["lo"]), _ptr(ints[0]),
+                                       _ptr(ints[1]), _ptr(ints[2]), _ptr(mx), _ptr(out), plan["frames"], 0, self.n_mels,
+                                       _stream()),
+                  "tw_logmel_long_n")
             torch.cuda.current_stream(self.device).synchronize()      # `pcm` / `ints` are freed when this returns
         return out
 

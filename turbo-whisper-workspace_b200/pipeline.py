@@ -280,7 +280,12 @@ class B200WhisperPipeline:
     def from_hf_model(cls, model, tokenizer, devices=("cuda:0",), max_batch: int = 24,
                       contexts_per_device: int = 4, scheduler=None) -> "B200WhisperPipeline":
         """Build from a ``transformers.WhisperForConditionalGeneration`` (weights, config, generation_config).
-        ``scheduler``: inject an engine stand-in instead of building GPU engines (tests)."""
+        ``scheduler``: inject an engine stand-in instead of building GPU engines (tests).
+        English-only checkpoints (``*.en``) are rejected: their prompt has no language or task token."""
+        if getattr(model.generation_config, "is_multilingual", None) is False:
+            raise ValueError("English-only Whisper checkpoints (*.en, generation_config.is_multilingual=False) are not "
+                             "supported: their decoder prompt has no language or task token, and only the multilingual "
+                             "prompt is implemented")
         dims = WhisperDims.from_hf_config(model.config)
         gen = GenerationSettings.from_hf(model.generation_config)
         gen.median_filter_width = int(getattr(model.config, "median_filter_width", 7))
