@@ -244,6 +244,31 @@ int tw_dec_finalize(const float* part_val, const int32_t* part_idx, int32_t n_pa
                     int32_t tokens_ld, const int32_t* forced, int32_t* choices, void* row_state,
                     const tw_grammar* g, int32_t batch, void* stream);
 
+/* ---- decoder prefill (generate(prompt_ids=...)) ----------------------------------------------------------------
+ * Runs positions 0 .. n_pos - 1 of `rows` decode rows through the decoder in one pass, so that the step loop continues
+ * at position n_pos as if it had fed those tokens itself.  Prompt row r, position t is activation row r * n_pos + t of
+ * every buffer below.  The projections are tw_gemm_bf16 launches over rows * n_pos rows (the engine's
+ * WhisperEngine.prefill); these functions are the rest of WhisperDecoderLayer for those rows
+ * ($TF/models/whisper/modeling_whisper.py:449-506, :736-759).
+ * x[r * n_pos + t, :] = tok_emb[tokens[r, t], :] + pos_emb[t, :]   (fp32 [rows * n_pos, d_model]) */
+int tw_prefill_embed(const int32_t* tokens, int32_t tokens_ld, int32_t rows, int32_t n_pos, const void* tok_emb_bf16,
+                     const float* pos_emb, float* x, int32_t d_model, void* stream);
+/* K and V columns of the fused q|k|v projection (bf16 [rows * n_pos, 3 * d_model]) -> the paged self-attention cache
+ * at positions 0 .. n_pos - 1, in the layout tw_dec_qkv writes (pool layer base [2][n_pages][64][d_model]). */
+int tw_prefill_kv_store(const void* qkv_bf16, int32_t rows, int32_t n_pos, int32_t d_model, void* kv_pool_layer,
+                        const int32_t* block_table, int32_t pages_per_row, int32_t n_pages, void* stream);
+/* causal self-attention of the prompt positions (head_dim 64, q pre-scaled) read from the fused q|k|v projection;
+ * out: bf16 [rows * n_pos, heads * 64].  n_pos <= 448. */
+int tw_prefill_self_attn(const void* qkv_bf16, void* out_bf16, int32_t rows, int32_t n_pos, int32_t heads,
+                         void* stream);
+/* cross-attention of the prompt queries (q: bf16 row r * n_pos + t at q + (r * n_pos + t) * q_ld) over src_len encoder
+ * positions; K / V addressing as tw_dec_cross_attn (row r reads window enc_row[r], NULL = r).
+ * out: bf16 [rows * n_pos, heads * 64]. */
+int tw_prefill_cross_attn(const void* q_bf16, int64_t q_ld, void* out_bf16, const void* k_bf16, const void* v_bf16,
+                          int64_t kv_row_stride, int64_t kv_batch_stride, int64_t kv_head_stride,
+                          const int32_t* enc_row, int32_t src_len, int32_t rows, int32_t n_pos, int32_t heads,
+                          void* stream);
+
 /* ---- word-level timestamps (return_timestamps="word") --------------------------------------------------------
  * Replaces the `output_attentions` plumbing + WhisperGenerationMixin._extract_token_timestamps
  * ($TF/models/whisper/generation_whisper.py:241-381; _median_filter :43-61, _dynamic_time_warping :64-112).

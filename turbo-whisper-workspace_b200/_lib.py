@@ -95,6 +95,11 @@ SIGNATURES = {
                                   c_int32, c_void_p]),
     "tw_resample": (C.c_int, [c_void_p, c_int32, c_int32, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_int32, c_int32,
                               c_int32, c_void_p]),
+    "tw_prefill_embed": (C.c_int, [c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_int32, c_void_p]),
+    "tw_prefill_kv_store": (C.c_int, [c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_int32, c_int32, c_void_p]),
+    "tw_prefill_self_attn": (C.c_int, [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_void_p]),
+    "tw_prefill_cross_attn": (C.c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p,
+                                        c_int32, c_int32, c_int32, c_int32, c_void_p]),
     "tw_dec_align_tap": (C.c_int, [c_void_p, c_int32, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_void_p, c_void_p,
                                    c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p]),
     "tw_align_matrix": (C.c_int, [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32,

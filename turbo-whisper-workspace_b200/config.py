@@ -137,3 +137,36 @@ class GenerationSettings:
         if getattr(gc, "alignment_heads", None) is not None:
             s.alignment_heads = [[int(l), int(h)] for l, h in gc.alignment_heads]
         return s
+
+
+def validate_prompt_ids(prompt_ids, vocab: int) -> List[int]:
+    """``prompt_ids`` of generate (list / numpy / torch, normally ``[<|startofprev|>, text ids...]``) -> list of ints.
+    Raises ValueError unless it is a non-empty 1-D sequence of integer ids in [0, vocab)."""
+    import numpy as np
+    if hasattr(prompt_ids, "detach"):
+        prompt_ids = prompt_ids.detach().cpu().numpy()
+    arr = np.asarray(prompt_ids)
+    if arr.ndim != 1:
+        raise ValueError(f"`prompt_ids` must be a 1-D sequence of token ids, got shape {tuple(arr.shape)}")
+    if arr.size == 0:
+        raise ValueError("`prompt_ids` is empty")
+    if not (np.issubdtype(arr.dtype, np.integer) or arr.dtype == object and all(isinstance(v, (int, np.integer)) for v in arr)):
+        raise ValueError(f"`prompt_ids` must hold integer token ids, got dtype {arr.dtype}")
+    ids = [int(v) for v in arr]
+    bad = [v for v in ids if not 0 <= v < vocab]
+    if bad:
+        raise ValueError(f"`prompt_ids` holds ids outside the vocabulary [0, {vocab}): {bad[:8]}")
+    return ids
+
+
+def decoder_prompt_len(prompt_ids, timestamps: bool, max_len: int) -> int:
+    """Positions of the decoder input prompt_ids + [<|startoftranscript|>, language, task] (+ <|notimestamps|>)
+    ($TF/models/whisper/generation_whisper.py:1909-1913).  ``max_len`` = min(max_length, max_target_positions): the
+    prompt counts against it, so a long prompt leaves fewer positions to generate.  ValueError unless the input is
+    shorter than ``max_len`` (HF indexes past its positional embedding there)."""
+    n = (3 if timestamps else 4) + (0 if prompt_ids is None else len(prompt_ids))
+    if n >= max_len:
+        raise ValueError(f"The decoder input (prompt_ids and the {3 if timestamps else 4} special start tokens) has "
+                         f"{n} positions; it must be shorter than {max_len} (min(max_length, max_target_positions)). "
+                         "Shorten the prompt.")
+    return n

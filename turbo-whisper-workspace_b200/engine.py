@@ -22,11 +22,12 @@ import torch
 
 from . import _lib, ops
 from ._lib import Grammar, SkinnyArgs, check
-from .config import N_FRAMES, N_SAMPLES, GenerationSettings, WhisperDims
+from .config import N_FRAMES, N_SAMPLES, GenerationSettings, WhisperDims, decoder_prompt_len, validate_prompt_ids
 
 MAX_DECODE_BATCH = 96   # decode rows per engine context (projections: up to tw_dec_max_rows(); the LM head runs per 48-row chunk)
 LMHEAD_ROWS = 48
 _CAPTURE_LOCK = threading.Lock()   # CUDA-graph capture is serialised across the engine contexts of a process
+_PREFILL_WEIGHTS_LOCK = threading.Lock()   # the contexts of a device share (and lazily extend) one weight dict
 PAGE = 64
 ROWSTATE_INTS = 8
 
@@ -51,6 +52,14 @@ def pack_skinny_weight(w: torch.Tensor) -> torch.Tensor:
     if n_pad != n:
         w = torch.cat([w, torch.zeros(n_pad - n, k, dtype=w.dtype, device=w.device)], 0)
     return (w.view(n_pad // 16, 2, 8, k // 32, 4, 8).permute(0, 3, 1, 2, 4, 5).contiguous().view(n_pad, k))
+
+
+def unpack_skinny_weight(w: torch.Tensor, n: int) -> torch.Tensor:
+    """Inverse of :func:`pack_skinny_weight`: fragment-major [N_padded, K] -> row-major [n, K] (nn.Linear layout, the
+    tcgen05 GEMM's B operand).  A permutation of the same bf16 values, so the result is exact; runs wherever ``w``
+    lives (the engine derives the prefill's row-major weights on the device)."""
+    n_pad, k = w.shape
+    return w.view(n_pad // 16, k // 32, 2, 8, 4, 8).permute(0, 2, 3, 1, 4, 5).contiguous().view(n_pad, k)[:n].contiguous()
 
 
 def ln_fold_enabled() -> bool:
@@ -425,7 +434,8 @@ class WhisperEngine:
     def encode(self, B: int, mel: Optional[torch.Tensor] = None, taps: Optional[dict] = None) -> torch.Tensor:
         """WhisperEncoder.forward for B windows whose time-major features are in ``mel`` (default
         self.mel_t).  Leaves the final-LayerNorm output in self.xn[:B*1500] and the cross-attention
-        K/V of all decoder layers in self.ckv."""
+        K/V of all decoder layers in self.ckv.  The activation buffers (x, xn, qkv, att, hid) are the prompt prefill's
+        scratch as well: the returned xn is only valid until the next :meth:`prefill`."""
         d, w = self.dims, self.w
         D, S, T, F = d.d_model, d.max_source_positions, N_FRAMES, d.ffn
         M = B * S
@@ -575,6 +585,139 @@ class WhisperEngine:
                                       p(self.forced), None if self.choices is None else p(self.choices), p(self.state),
                                       C.byref(self.grammar), B, st), "tw_dec_finalize")
 
+    # ------------------------------------------------------------------------------------ prompt prefill
+    def _prefill_table(self) -> List[Dict[str, tuple]]:
+        """Per decoder layer and projection: (row-major weight [N, K], bias, LayerNorm gamma, beta) of the prefill GEMMs.
+        Where the decode step folds a LayerNorm into the projection (``ln_fold``), the prefill feeds the GEMM
+        x_hat = (x - mean) rstd (gamma = 1, beta = 0) and uses the folded W' = W diag(gamma) with bias d = W beta + b —
+        the algebra of the step's folded epilogue; elsewhere (layer 0's q|k|v, the TWB200_NO_LN_FOLD build) it is
+        LayerNorm(gamma, beta) with W and b.  gamma / beta None = no LayerNorm in front (the residual projections).
+        The row-major copies are derived on the device from the fragment-major decode weights (unpack_skinny_weight)
+        at the first prompted call on a device and shared by every engine context of that device through ``self.w``."""
+        w, d = self.w, self.dims
+        D, F = d.d_model, d.ffn
+        if "prefill.ones" not in w:
+            with _PREFILL_WEIGHTS_LOCK:
+                if "prefill.ones" not in w:
+                    with torch.cuda.device(self.device):
+                        rm = {}
+                        for i in range(d.dec_layers):
+                            q = f"dec{i}."
+                            names = {"out_w": D, "cout_w": D, "fc2_w": D}
+                            names.update({"qkv_wf": 3 * D, "cq_wf": D, "fc1_wf": F} if self.ln_fold else {})
+                            names.update({"qkv_w": 3 * D, "cq_w": D, "fc1_w": F})
+                            for nm, n in names.items():
+                                if q + nm in w:
+                                    rm[f"prefill.{q}{nm}"] = unpack_skinny_weight(w[q + nm], n)
+                        rm["prefill.zeros"] = torch.zeros(D, dtype=torch.float32, device=self.device)
+                        # the copies are made on this context's stream; other contexts use them on theirs
+                        torch.cuda.current_stream(self.device).synchronize()
+                    w.update(rm)
+                    w["prefill.ones"] = torch.ones(D, dtype=torch.float32, device=self.device)
+        table = []
+        for i in range(d.dec_layers):
+            q = f"dec{i}."
+            ident = ("prefill.ones", "prefill.zeros")
+
+            def proj(base, ln):
+                if self.ln_fold and f"prefill.{q}{base}_wf" in w:
+                    return (f"prefill.{q}{base}_wf", q + base + "_d") + ident
+                return (f"prefill.{q}{base}_w", q + base + "_b") + ((q + ln + "_w", q + ln + "_b") if ln else (None, None))
+            table.append({"qkv": proj("qkv", "ln1"), "out": proj("out", None), "cq": proj("cq", "ln2"),
+                          "cout": proj("cout", None), "fc1": proj("fc1", "ln3"), "fc2": proj("fc2", None)})
+        return table
+
+    def prefill(self, R: int, P: int, timing: Optional[dict] = None) -> None:
+        """Decoder prefill of a text prompt: positions 0 .. P-2 of the rows self.tokens[:R] (P = prompt length with
+        the special tokens) through every decoder layer as one batch of M = R (P-1) activation rows — embeddings
+        (tw_prefill_embed), LayerNorms (tw_layernorm), the projections on the tcgen05 GEMM (tw_gemm_bf16 with its bias /
+        GELU / residual epilogues), K / V into the paged cache (tw_prefill_kv_store), causal self-attention and
+        cross-attention against the windows of self.enc_row (tw_prefill_self_attn / _cross_attn).  Position P-1 is fed
+        by the first decode step, which also produces the first generated token.  The last layer stops after its K / V.
+        Scratch: the encoder's activation buffers (free once encode() has written self.ckv; R (P-1) <= max_enc_batch
+        x 1500 always holds).  ``timing``: receives CUDA-event milliseconds per phase ("gemm", "attn", "other")."""
+        T = P - 1
+        if T <= 0:
+            return
+        d, w, lib = self.dims, self.w, _lib.load()
+        D, F, H, L, S = d.d_model, d.ffn, d.heads, d.dec_layers, d.max_source_positions
+        if R > self.max_batch or P > self.max_len:
+            raise ValueError(f"prefill of {R} rows x {P} positions exceeds the engine ({self.max_batch} rows, {self.max_len} positions)")
+        table = self._prefill_table()
+        M = R * T
+        p = lambda t: C.c_void_p(t.data_ptr())
+        st = self._stream()
+        x, xn, qkv, att, hid = self.x[:M], self.xn[:M], self.qkv[:M], self.att[:M], self.hid[:M]
+        cq = self.qkv.view(-1)[:M * D].view(M, D)
+        blk = self._ckv_batch * S * 64
+        events: List[tuple] = []
+
+        def mark(kind):
+            if timing is not None:
+                ev = torch.cuda.Event(enable_timing=True)
+                ev.record()
+                events.append((kind, ev))
+
+        launches = 0
+
+        def gemm(name, a, out, act=0, resid=False):
+            nonlocal launches
+            wt, bias, _, _ = table[i][name]
+            mark("gemm")
+            ops.gemm(a, w[wt], rows=M, bias=w[bias], act=act, resid=x if resid else None, resid_ld=D if resid else 0,
+                     out=out)
+            launches += 1
+
+        def norm(name):
+            nonlocal launches
+            _, _, g, b = table[i][name]
+            mark("other")
+            ops.layernorm(x, w[g], w[b], out=xn)
+            launches += 1
+
+        with torch.cuda.device(self.device):
+            mark("other")
+            check(lib.tw_prefill_embed(p(self.tokens), self.max_len, R, T, p(w["tok_emb"]), p(w["dec_pos"]), p(x), D, st),
+                  "tw_prefill_embed")
+            launches += 1
+            for i in range(L):
+                pool = self.kv_pool[i]
+                norm("qkv")
+                gemm("qkv", xn, qkv)
+                mark("other")
+                check(lib.tw_prefill_kv_store(p(qkv), R, T, D, p(pool), p(self.block_table), self.pages_per_row,
+                                              self.n_pages, st), "tw_prefill_kv_store")
+                launches += 1
+                if i + 1 == L:      # nothing reads the last layer's outputs at the prompt positions
+                    break
+                mark("attn")
+                check(lib.tw_prefill_self_attn(p(qkv), p(att), R, T, H, st), "tw_prefill_self_attn")
+                gemm("out", att, x, resid=True)
+                norm("cq")
+                gemm("cq", xn, cq)
+                mark("attn")
+                kptr = C.c_void_p(self.ckv.data_ptr() + ((i * 2 + 0) * H) * blk * 2)
+                vptr = C.c_void_p(self.ckv.data_ptr() + ((i * 2 + 1) * H) * blk * 2)
+                check(lib.tw_prefill_cross_attn(p(cq), D, p(att), kptr, vptr, 64, S * 64, blk, p(self.enc_row), S, R, T,
+                                                H, st), "tw_prefill_cross_attn")
+                launches += 2
+                gemm("cout", att, x, resid=True)
+                norm("fc1")
+                gemm("fc1", xn, hid, act=1)
+                gemm("fc2", hid, x, resid=True)
+            mark("end")
+        self.stats["launches"] += launches
+        self.stats["prefill_rows"] = self.stats.get("prefill_rows", 0) + M
+        if timing is not None:
+            torch.cuda.current_stream(self.device).synchronize()
+            for (kind, a), (_, b) in zip(events[:-1], events[1:]):
+                timing[kind] = timing.get(kind, 0.0) + a.elapsed_time(b)
+
+    def prompt_row_len(self, prompt_ids: Optional[Sequence[int]], timestamps: bool) -> int:
+        """Length of the decoder prompt: prompt_ids + [<|startoftranscript|>, language, task] (+ <|notimestamps|>).
+        ValueError (before any device work) unless it is shorter than min(max_length, max_target_positions)."""
+        return decoder_prompt_len(prompt_ids, timestamps, self.max_len)
+
     @property
     def launches_per_step(self) -> int:
         taps = sum(len(r) for r in self.align["layers"].values()) if self._align_on else 0
@@ -604,7 +747,8 @@ class WhisperEngine:
         return g
 
     def decode(self, B: int, prompts: Optional[torch.Tensor], n_steps: Optional[int] = None,
-               forced: Optional[torch.Tensor] = None, on_step=None, timestamps: bool = True) -> torch.Tensor:
+               forced: Optional[torch.Tensor] = None, on_step=None, timestamps: bool = True,
+               prompt_ids: Optional[Sequence[int]] = None, prefill_timing: Optional[dict] = None) -> torch.Tensor:
         """Greedy decode of B rows against the encoder state left by encode().
 
         prompts: int32 [B, 3] = [<|startoftranscript|>, language, task]; a language of -1 asks for
@@ -612,6 +756,9 @@ class WhisperEngine:
         forced:  optional int32 [B, max_len] teacher-forcing table (-1 = free running).
         timestamps: False = generate(return_timestamps=False): <|notimestamps|> is appended to the prompt and only
                  the two suppress lists are applied (no WhisperTimeStampLogitsProcessor).
+        prompt_ids: text prompt of generate(prompt_ids=...): the rows start with prompt_ids + [SOT, language, task]
+                 (+ <|notimestamps|>) = P positions, of which 0 .. P-2 run as one batched prefill (:meth:`prefill`) and
+                 the step loop starts at position P-1; the timestamp grammar begins at P.  The language must be known.
         Returns the int32 token matrix [B, max_len] on the device (prompt included)."""
         dev = self.device
         max_len = self.max_len
@@ -621,22 +768,42 @@ class WhisperEngine:
             st0 = torch.zeros(B, ROWSTATE_INTS, dtype=torch.int32)
             st0[:, 2] = -1
             pr = prompts.cpu()
-            for b in range(B):
-                tok0[b, 0] = int(pr[b, 0])
-                if int(pr[b, 1]) < 0:
-                    st0[b, 7] = 1          # language detection at position 0
-                else:
-                    frc[b, 1] = int(pr[b, 1])
-                frc[b, 2] = int(pr[b, 2])
-                if not timestamps:
-                    st0[b, 7] |= 2
-                    frc[b, 3] = self.gen.no_timestamps_token_id
-            self.grammar.begin_index = 3 if timestamps else 4
+            P = 0
+            if prompt_ids is None:
+                for b in range(B):
+                    tok0[b, 0] = int(pr[b, 0])
+                    if int(pr[b, 1]) < 0:
+                        st0[b, 7] = 1          # language detection at position 0
+                    else:
+                        frc[b, 1] = int(pr[b, 1])
+                    frc[b, 2] = int(pr[b, 2])
+                    if not timestamps:
+                        st0[b, 7] |= 2
+                        frc[b, 3] = self.gen.no_timestamps_token_id
+                self.grammar.begin_index = 3 if timestamps else 4
+            else:
+                if bool((pr[:, 1] < 0).any()):
+                    raise ValueError("decode with prompt_ids needs the language of every row (detect it first)")
+                tail = [] if timestamps else [self.gen.no_timestamps_token_id]
+                P = self.prompt_row_len(prompt_ids, timestamps)
+                tok0[:, :P] = torch.tensor([list(prompt_ids) + [int(v) for v in pr[b, :3]] + tail for b in range(B)],
+                                           dtype=torch.int32)
+                # the row state the forced steps would leave at position P-1: the next token is the first generated one
+                g = self.grammar
+                st0[:, 0] = P - 1
+                st0[:, 3] = st0[:, 4] = g.ts_begin
+                st0[:, 5] = g.ts_begin + g.max_initial_ts
+                st0[:, 6] = 1
+                st0[:, 7] = 0 if timestamps else 2
+                g.begin_index = P
             self.tokens[:B].copy_(tok0.to(dev, non_blocking=False))
             self.forced[:B].copy_(frc.to(dev))
             self.state[:B].copy_(st0.to(dev))
             self.stats["h2d_bytes"] += 2 * B * max_len * 4 + B * ROWSTATE_INTS * 4
             steps = (max_len - 1) if n_steps is None else min(n_steps, max_len - 1)
+            if P:
+                self.prefill(B, P, timing=prefill_timing)
+                steps = min(steps, max_len - P)
             _lib.load().tw_set_pdl(0 if (self.use_graphs or os.environ.get("TWB200_NO_PDL")) else 1)   # PDL only pays off for eager stepping
             graph = self._graph_for(B) if self.use_graphs else None
             for s in range(steps):
@@ -711,7 +878,7 @@ class WhisperEngine:
                                        p(ws["copy_len"]), p(ws["origin"]), n, self._stream()), "tw_beam_step")
 
     def decode_beams(self, n: int, prompts: torch.Tensor, num_beams: int, timestamps: bool = True,
-                     frames_keep: Optional[Sequence[int]] = None) -> torch.Tensor:
+                     frames_keep: Optional[Sequence[int]] = None, prompt_ids: Optional[Sequence[int]] = None) -> torch.Tensor:
         """Beam search ($TF/generation/utils.py:3076 `_beam_search`, early_stopping=False) for n windows against the
         encoder state left by encode(): n * num_beams decode rows share the windows' cross K/V through `enc_row`; per
         position ONE CUDA-graph replay runs the decode kernels (raw fp32 logits of every row) and `tw_beam_step`
@@ -723,7 +890,9 @@ class WhisperEngine:
         ``frames_keep``: per window the encoder frames kept for the token-timestamp DTW; the alignment tap runs in
         every step, the search keeps HF's `beam_indices`, the tapped rows of every position are gathered from the beam
         that produced it ($TF/models/whisper/generation_whisper.py:265-303) and ``self.last_beam_frames`` receives
-        the frames."""
+        the frames.
+        ``prompt_ids``: text prompt (see :meth:`decode`): the rows start with prompt_ids + prompts (+ <|notimestamps|>),
+        whose positions but the last run as one prefill over the n * num_beams rows instead of forced steps."""
         K, R = int(num_beams), n * int(num_beams)
         if R > self.max_batch:
             raise ValueError(f"{n} windows x {K} beams exceed max_batch {self.max_batch}")
@@ -736,7 +905,11 @@ class WhisperEngine:
         want_frames = frames_keep is not None
         with torch.cuda.device(dev):
             tail = [] if timestamps else [gen.no_timestamps_token_id]
-            prompt = torch.cat([prompts.to(torch.long).cpu(), torch.tensor([tail] * n, dtype=torch.long).view(n, len(tail))], dim=1)
+            head = [] if prompt_ids is None else [int(v) for v in prompt_ids]
+            if prompt_ids is not None:
+                self.prompt_row_len(head, timestamps)
+            prompt = torch.cat([torch.tensor([head] * n, dtype=torch.long).view(n, len(head)), prompts.to(torch.long).cpu(),
+                                torch.tensor([tail] * n, dtype=torch.long).view(n, len(tail))], dim=1)
             P = prompt.shape[1]
             rows_prompt = prompt.repeat_interleave(K, dim=0)                      # [R, P]
             tok0 = torch.full((R, self.max_len), gen.pad_token_id, dtype=torch.int32)
@@ -746,6 +919,12 @@ class WhisperEngine:
             st0 = torch.zeros(R, ROWSTATE_INTS, dtype=torch.int32)
             st0[:, 2] = -1
             st0[:, 7] = 2      # "flat" mode: the grammar is applied by tw_beam_step on the tapped logits, not by the LM head
+            if prompt_ids is not None:
+                # prefilled prompt: the row state the forced steps would leave at position P-1
+                st0[:, 0] = P - 1
+                st0[:, 3] = st0[:, 4] = self.grammar.ts_begin
+                st0[:, 5] = self.grammar.ts_begin + self.grammar.max_initial_ts
+                st0[:, 6] = 1
             self.tokens[:R].copy_(tok0.to(dev))
             self.forced[:R].copy_(frc.to(dev))
             self.state[:R].copy_(st0.to(dev))
@@ -774,13 +953,19 @@ class WhisperEngine:
                 self.enable_alignment()
             self._align_on = want_frames
             try:
-                # the prompt but its last token: plain forced steps (their logits are not needed)
-                plain = self._graph_for(R) if (self.use_graphs and P > 1) else None
-                for _ in range(P - 1):
-                    if plain is not None:
-                        plain.replay()
-                    else:
-                        self._decode_step(R)
+                if prompt_ids is not None:
+                    # the prompt but its last token: one prefill over the R rows (no alignment tap: the DTW drops the
+                    # prompt positions)
+                    self.prefill(R, P)
+                else:
+                    # the prompt but its last token: plain forced steps (their logits are not needed)
+                    plain = self._graph_for(R) if (self.use_graphs and P > 1) else None
+                    for _ in range(P - 1):
+                        if plain is not None:
+                            plain.replay()
+                        else:
+                            self._decode_step(R)
+                forced_steps = 0 if prompt_ids is not None else P - 1
                 key = ("beam", R, K, self._ckv_batch, P, bool(timestamps), want_frames)
                 graph = self._graphs.get(key) if self.use_graphs else None
                 if self.use_graphs and graph is None:
@@ -819,8 +1004,8 @@ class WhisperEngine:
                 if not int(ctrl[1]):
                     raise RuntimeError("beam search did not terminate within max_length")
                 taken, par = int(ctrl[4]), int(ctrl[0])
-                self.stats["dec_steps"] += P - 1 + steps
-                self.stats["launches"] += (P - 1) * self.launches_per_step + steps * (self.launches_per_step - 1 + 3)
+                self.stats["dec_steps"] += forced_steps + steps
+                self.stats["launches"] += forced_steps * self.launches_per_step + steps * (self.launches_per_step - 1 + 3)
                 fin_len = ws["fin_len"][:, 0].cpu()
                 fin_score = ws["fin_score"][:, 0].cpu()
                 # the search's own accounting of the returned hypotheses (sum of processed log-probabilities, length)
@@ -850,22 +1035,27 @@ class WhisperEngine:
     # ------------------------------------------------------------------------------------ generate
     def generate_from_pcm(self, clips: Sequence[np.ndarray], task: str = "transcribe",
                           language: Optional[str] = None, return_timestamps: bool = True, num_beams: int = 1,
-                          token_timestamps: bool = False):
+                          token_timestamps: bool = False, prompt_ids: Optional[Sequence[int]] = None):
         """PCM windows (<= 30 s each) -> generated token ids per window (segments concatenated), the
         output contract of ``WhisperGenerationMixin.generate(..., return_timestamps=True)`` minus padding.
         ``token_timestamps``: every window becomes ``(ids, times)`` with one fp32 time per id — the per-segment
         `token_timestamps` of generate(return_token_timestamps=True, return_segments=True), which the ASR pipeline
-        reads for return_timestamps="word"."""
+        reads for return_timestamps="word".
+        ``prompt_ids``: generate(prompt_ids=...) (see :meth:`generate`); validated before any device work."""
+        if prompt_ids is not None:
+            prompt_ids = validate_prompt_ids(prompt_ids, self.dims.vocab)
+            self.prompt_row_len(prompt_ids, bool(return_timestamps))
+
         def run():
             B = self.load_pcm(clips)
             self.features(B)
             if not token_timestamps:
                 return self.generate(B, task=task, language=language, return_timestamps=return_timestamps,
-                                     num_beams=num_beams)
+                                     num_beams=num_beams, prompt_ids=prompt_ids)
             # attention_mask.sum(-1) of the feature extractor: the sample mask taken every hop (160) samples
             nf = [min(N_FRAMES, -(-min(len(np.asarray(c).reshape(-1)), N_SAMPLES) // 160)) for c in clips]
             rows = self.generate(B, task=task, language=language, return_timestamps=return_timestamps,
-                                 num_beams=num_beams, token_timestamps=True, num_frames=nf)
+                                 num_beams=num_beams, token_timestamps=True, num_frames=nf, prompt_ids=prompt_ids)
             return list(zip(rows, self.last_token_ts))
         if self.stream is not None:
             with torch.cuda.stream(self.stream):
@@ -873,18 +1063,25 @@ class WhisperEngine:
         return run()
 
     def generate_long_from_pcm(self, audio: np.ndarray, task: str = "transcribe", language: Optional[str] = None,
-                               num_beams: int = 1, trace: Optional[dict] = None) -> List[int]:
+                               num_beams: int = 1, trace: Optional[dict] = None,
+                               prompt_ids: Optional[Sequence[int]] = None) -> List[int]:
         """ONE clip longer than 30 s, un-chunked (the ASR pipeline without chunk_length_s,
         $TF/pipelines/automatic_speech_recognition.py:446-454): features of the whole clip (tw_logmel_long) and HF's
         long-form generate — the same seek loop as :meth:`generate`, over all n // 160 frames
         ($TF/models/whisper/generation_whisper.py:654-658, :785-870); timestamps are mandatory (:1388-1394).  Sequential
         by construction: one window is encoded and decoded per iteration.  Returns the generated ids (segments
-        concatenated; timestamp tokens restart in every 30 s segment, which `_decode_asr` undoes)."""
+        concatenated; timestamp tokens restart in every 30 s segment, which `_decode_asr` undoes).
+        ``prompt_ids``: prepended in every seek iteration (HF with condition_on_prev_tokens off)."""
+        if prompt_ids is not None:
+            prompt_ids = validate_prompt_ids(prompt_ids, self.dims.vocab)
+            self.prompt_row_len(prompt_ids, True)
+
         def run():
             mel = self.logmel.long(audio)
             self.stats["launches"] += 2
             self.stats["h2d_bytes"] += int(np.asarray(audio).size) * 4
-            return self.generate(1, task=task, language=language, num_beams=num_beams, long_mel=mel, trace=trace)[0]
+            return self.generate(1, task=task, language=language, num_beams=num_beams, long_mel=mel, trace=trace,
+                                 prompt_ids=prompt_ids)[0]
         if self.stream is not None:
             with torch.cuda.stream(self.stream):
                 return run()
@@ -907,7 +1104,8 @@ class WhisperEngine:
     def generate(self, B: int, task: str = "transcribe", language: Optional[str] = None,
                  trace: Optional[dict] = None, return_timestamps: bool = True, num_beams: int = 1,
                  token_timestamps: bool = False, num_frames: Optional[Sequence[int]] = None,
-                 long_mel: Optional[torch.Tensor] = None) -> List[List[int]]:
+                 long_mel: Optional[torch.Tensor] = None, prompt_ids: Optional[Sequence[int]] = None,
+                 prefill_timing: Optional[dict] = None) -> List[List[int]]:
         """Short-form seek loop over the features in self.mel_t[:B] (greedy; timestamp grammar on unless
         ``return_timestamps`` is False, in which case <|notimestamps|> joins the prompt).
 
@@ -917,8 +1115,15 @@ class WhisperEngine:
         ``self.last_token_ts_raw[b]`` = the padded `token_timestamps` output, no offset).
 
         ``long_mel`` (bf16 [T, n_mels], T > 3000, B == 1): HF's long-form mode — the loop runs over T frames and every
-        iteration's window is gathered from ``long_mel`` (zero-padded to 3000 frames, _get_input_segment :1831-1850)."""
+        iteration's window is gathered from ``long_mel`` (zero-padded to 3000 frames, _get_input_segment :1831-1850).
+
+        ``prompt_ids`` (generate(prompt_ids=...), $TF/models/whisper/generation_whisper.py:1909-1913): every seek
+        iteration's decoder input is prompt_ids + [SOT, language, task] (+ <|notimestamps|>), run as one batched prefill
+        after encode(); the returned ids exclude it.  An unknown language is detected first on [SOT] alone (one decode
+        position), as detect_language does before the prompt is built.  ``prefill_timing``: per-phase prefill times."""
         gen = self.gen
+        if prompt_ids is not None:
+            prompt_ids = validate_prompt_ids(prompt_ids, self.dims.vocab)
         if long_mel is not None:
             if B != 1 or token_timestamps or not return_timestamps:
                 raise ValueError("long-form generate takes one clip, needs timestamps and has no token timestamps")
@@ -937,7 +1142,7 @@ class WhisperEngine:
                 raise ValueError(f"Unsupported language: {language}")
             lang_id = gen.lang_to_id[key]
         ts_begin = gen.timestamp_begin
-        P = 3 if return_timestamps else 4
+        P = self.prompt_row_len(prompt_ids, bool(return_timestamps))
         seek = [0] * B
         max_frames = [N_FRAMES] * B if long_mel is None else [int(long_mel.shape[0])]
         langs = [lang_id] * B
@@ -970,15 +1175,15 @@ class WhisperEngine:
                 self.encode(n, mel)
                 prompts = torch.tensor([[gen.decoder_start_token_id, langs[b], gen.task_to_id[task]] for b in rows],
                                        dtype=torch.int32)
+                if (num_beams > 1 or prompt_ids is not None) and any(langs[b] < 0 for b in rows):
+                    # language detection first (one decoder position), as detect_language does before generate
+                    first = self.decode(n, prompts, n_steps=1, timestamps=bool(return_timestamps))[:, 1].cpu().tolist()
+                    for i, b in enumerate(rows):
+                        if langs[b] < 0:
+                            langs[b] = int(first[i])
+                    prompts = torch.tensor([[gen.decoder_start_token_id, langs[b], gen.task_to_id[task]] for b in rows],
+                                           dtype=torch.int32)
                 if num_beams > 1:
-                    if any(l < 0 for l in (langs[b] for b in rows)):
-                        # language detection first (one decoder position), as detect_language does before generate
-                        first = self.decode(n, prompts, n_steps=1, timestamps=bool(return_timestamps))[:, 1].cpu().tolist()
-                        for i, b in enumerate(rows):
-                            if langs[b] < 0:
-                                langs[b] = int(first[i])
-                        prompts = torch.tensor([[gen.decoder_start_token_id, langs[b], gen.task_to_id[task]] for b in rows],
-                                               dtype=torch.int32)
                     keep_b = None
                     if token_timestamps:
                         S_ = self.dims.max_source_positions
@@ -986,13 +1191,15 @@ class WhisperEngine:
                         twice_ = len(set(left_)) == 1
                         keep_b = [len((range(S_)[: v // 2] if twice_ else range(S_))[: v // 2]) for v in left_]
                     best = self.decode_beams(n, prompts, num_beams, timestamps=bool(return_timestamps),
-                                             frames_keep=keep_b).cpu().tolist()
+                                             frames_keep=keep_b, prompt_ids=prompt_ids).cpu().tolist()
+                    pre = list(prompt_ids or [])
                     head = [gen.decoder_start_token_id, 0, gen.task_to_id[task]] + ([] if return_timestamps else [gen.no_timestamps_token_id])
-                    toks = [[head[0], langs[b]] + head[2:] + best[i] for i, b in enumerate(rows)]
+                    toks = [pre + [head[0], langs[b]] + head[2:] + best[i] for i, b in enumerate(rows)]
                 else:
                     self._align_on = bool(token_timestamps)
                     try:
-                        toks = self.decode(n, prompts, timestamps=bool(return_timestamps)).cpu().tolist()
+                        toks = self.decode(n, prompts, timestamps=bool(return_timestamps), prompt_ids=prompt_ids,
+                                           prefill_timing=prefill_timing).cpu().tolist()
                     finally:
                         self._align_on = False
                 self.stats["d2h_bytes"] += n * self.max_len * 4

@@ -26,7 +26,7 @@ from typing import Any, Dict, List, Optional, Sequence, Tuple, Union
 
 import numpy as np
 
-from .config import N_SAMPLES, SAMPLING_RATE, GenerationSettings, WhisperDims
+from .config import N_SAMPLES, SAMPLING_RATE, GenerationSettings, WhisperDims, decoder_prompt_len, validate_prompt_ids
 
 
 # ------------------------------------------------------------------------------------------------
@@ -307,6 +307,7 @@ class B200WhisperPipeline:
         task = generate_kwargs.pop("task", None) or "transcribe"
         language = generate_kwargs.pop("language", None)
         num_beams = int(generate_kwargs.pop("num_beams", None) or self.num_beams or 1)
+        prompt_ids = self._prompt(generate_kwargs, return_timestamps)
         if return_timestamps == "char":
             raise ValueError("Whisper cannot return `char` timestamps, only word level or segment level timestamps. "
                              "Use `return_timestamps='word'` or `return_timestamps=True` respectively.")
@@ -323,6 +324,9 @@ class B200WhisperPipeline:
             run_kw["return_timestamps"] = False
         if num_beams > 1:
             run_kw["num_beams"] = num_beams      # beam search: every window occupies num_beams decode rows
+        long_kw: Dict[str, Any] = {}
+        if prompt_ids is not None:
+            run_kw["prompt_ids"] = long_kw["prompt_ids"] = prompt_ids
         bs = max(1, int(batch_size or 1))
         token_times = None
         if return_timestamps == "word":
@@ -343,7 +347,7 @@ class B200WhisperPipeline:
         if return_timestamps == "word":
             token_times = [np.asarray(t, dtype=np.float32) for _, t in token_rows]
             token_rows = [r for r, _ in token_rows]
-        long_rows = {i: self.scheduler.run_long(p["longform"], task=task, language=language, num_beams=num_beams)
+        long_rows = {i: self.scheduler.run_long(p["longform"], task=task, language=language, num_beams=num_beams, **long_kw)
                      for i, p in enumerate(prepared) if "longform" in p}
         t2 = time.perf_counter()
         self.last_token_rows = token_rows      # the engines' rows of this call, window order (bench.py's output check)
@@ -361,6 +365,31 @@ class B200WhisperPipeline:
                                audio_seconds=sum(p["n_samples"] for p in prepared) / sr,
                                host_seconds={"prepare": t1 - t0, "engines": t2 - t1, "finish": time.perf_counter() - t2})
         return results if many else results[0]
+
+    def _prompt(self, generate_kwargs: dict, return_timestamps) -> Optional[List[int]]:
+        """Pops ``prompt_ids`` (list, numpy or torch; normally ``processor.get_prompt_ids(text)``) and
+        ``prompt_condition_type`` from generate_kwargs and validates them as WhisperGenerationMixin.generate does
+        ($TF/models/whisper/generation_whisper.py:1731-1748).  Every window's decoder input then starts with
+        prompt_ids; the returned ids, and so the text, exclude it.  ``"all-segments"`` needs condition_on_prev_tokens,
+        which is not implemented."""
+        prompt_ids = generate_kwargs.pop("prompt_ids", None)
+        cond = generate_kwargs.pop("prompt_condition_type", None) or "first-segment"
+        allowed = ["first-segment", "all-segments"]
+        if cond not in allowed:
+            raise ValueError(f"`prompt_condition_type={cond} does not exist. Make sure to set `prompt_condition_type` "
+                             f"to one of {', '.join(allowed)}")
+        if cond == "all-segments":
+            if generate_kwargs.get("condition_on_prev_tokens") is not True:
+                raise ValueError("Make sure to set `condition_on_prev_tokens=True` when setting "
+                                 "`prompt_condition_type='all-segments'`.")
+            raise NotImplementedError("prompt_condition_type='all-segments' needs condition_on_prev_tokens, which the "
+                                      "engine does not implement")
+        if prompt_ids is None:
+            return None
+        ids = validate_prompt_ids(prompt_ids, self.dims.vocab)
+        max_len = min(self.generation.max_length, self.dims.max_target_positions)
+        decoder_prompt_len(ids, bool(return_timestamps), max_len)
+        return ids
 
     def _prepare(self, inputs, chunk_length_s, stride_length_s) -> Dict[str, Any]:
         """preprocess ($TF/pipelines/automatic_speech_recognition.py:341-477) of one input: PCM, windows, clips."""

@@ -34,10 +34,13 @@ def partition(n_items: int, n_workers: int) -> List[Tuple[int, int]]:
     return out
 
 
-def _extra(return_timestamps: bool, num_beams: int, token_timestamps: bool = False) -> Dict[str, Any]:
+def _extra(return_timestamps: bool, num_beams: int, token_timestamps: bool = False,
+           prompt_ids: Optional[Sequence[int]] = None) -> Dict[str, Any]:
     """Keyword arguments beyond (task, language), passed only when they differ from the defaults so that simple
     engine stand-ins keep working."""
     kw: Dict[str, Any] = {}
+    if prompt_ids is not None:
+        kw["prompt_ids"] = list(prompt_ids)
     if not return_timestamps:
         kw["return_timestamps"] = False
     if num_beams > 1:
@@ -63,12 +66,12 @@ def group_ranges(n_items: int, n_workers: int, mb: int) -> List[Tuple[int, int]]
 
 def run_in_microbatches(engine, clips: Sequence[np.ndarray], task: str, language: Optional[str],
                         return_timestamps: bool = True, num_beams: int = 1, token_timestamps: bool = False,
-                        group: Optional[int] = None) -> List[Any]:
+                        group: Optional[int] = None, prompt_ids: Optional[Sequence[int]] = None) -> List[Any]:
     rows: List[Any] = []
     mb = microbatch_size(engine.max_batch, num_beams, group)
     for i in range(0, len(clips), mb):
         rows.extend(engine.generate_from_pcm(clips[i:i + mb], task=task, language=language,
-                                             **_extra(return_timestamps, num_beams, token_timestamps)))
+                                             **_extra(return_timestamps, num_beams, token_timestamps, prompt_ids)))
     return rows
 
 
@@ -147,8 +150,8 @@ class WindowScheduler:
 
     def run(self, clips: Sequence[np.ndarray], task: str = "transcribe", language: Optional[str] = None,
             return_timestamps: bool = True, num_beams: int = 1, token_timestamps: bool = False,
-            group: Optional[int] = None) -> List[Any]:
-        """Token rows per window, in order.  ``token_timestamps``: every row is ``(ids, times)`` (word timestamps);
+            group: Optional[int] = None, prompt_ids: Optional[Sequence[int]] = None) -> List[Any]:
+        """Token rows per window, in order.  ``prompt_ids``: the text prompt of every window (generate(prompt_ids=...)).  ``token_timestamps``: every row is ``(ids, times)`` (word timestamps);
         ``group`` = the HF pipeline's batch_size: micro-batches then are HF's generate batches (the per-token times of
         a row depend on the longest row of its batch, $TF/models/whisper/generation_whisper.py:241-381)."""
         t0 = time.perf_counter()
@@ -166,7 +169,7 @@ class WindowScheduler:
         queue = WorkQueue(n, mb)
         results: List[Optional[List[int]]] = [None] * n
         errors: List[BaseException] = []
-        extra = _extra(return_timestamps, num_beams, token_timestamps)
+        extra = _extra(return_timestamps, num_beams, token_timestamps, prompt_ids)
 
         def work(engine):
             try:
@@ -198,10 +201,11 @@ class WindowScheduler:
         return [r for r in results]
 
     def run_long(self, audio: np.ndarray, task: str = "transcribe", language: Optional[str] = None,
-                 num_beams: int = 1) -> List[int]:
+                 num_beams: int = 1, prompt_ids: Optional[Sequence[int]] = None) -> List[int]:
         """Token row of ONE un-chunked long-form clip (> 30 s): HF's long-form generate is a sequential seek loop over the
         clip's frames, so it runs on one engine context."""
-        return self.engines[0][0].generate_long_from_pcm(audio, task=task, language=language, num_beams=num_beams)
+        kw = {} if prompt_ids is None else {"prompt_ids": list(prompt_ids)}
+        return self.engines[0][0].generate_long_from_pcm(audio, task=task, language=language, num_beams=num_beams, **kw)
 
     def close(self):
         self.engines = []
@@ -230,16 +234,17 @@ class DistributedWindowScheduler:
 
     def run_local(self, clips: Sequence[np.ndarray], task: str = "transcribe", language: Optional[str] = None,
                   return_timestamps: bool = True, num_beams: int = 1, token_timestamps: bool = False,
-                  group: Optional[int] = None) -> List[Any]:
+                  group: Optional[int] = None, prompt_ids: Optional[Sequence[int]] = None) -> List[Any]:
         mb = microbatch_size(self.engine.max_batch, num_beams, group) if group else None
         s, e = self.local_range(len(clips), mb)
         if e <= s:
             return []
         if hasattr(self.engine, "run"):          # a local WindowScheduler (engine contexts of this rank's GPU)
+            kw = {} if prompt_ids is None else {"prompt_ids": prompt_ids}
             return self.engine.run(clips[s:e], task=task, language=language, return_timestamps=return_timestamps,
-                                   num_beams=num_beams, token_timestamps=token_timestamps, group=group)
+                                   num_beams=num_beams, token_timestamps=token_timestamps, group=group, **kw)
         return run_in_microbatches(self.engine, clips[s:e], task, language, return_timestamps, num_beams,
-                                   token_timestamps, group)
+                                   token_timestamps, group, prompt_ids)
 
     def gather(self, local_rows: List[List[int]]) -> List[List[int]]:
         if self.world_size == 1:
@@ -254,20 +259,22 @@ class DistributedWindowScheduler:
 
     def run(self, clips: Sequence[np.ndarray], task: str = "transcribe", language: Optional[str] = None,
             return_timestamps: bool = True, num_beams: int = 1, token_timestamps: bool = False,
-            group: Optional[int] = None) -> List[Any]:
+            group: Optional[int] = None, prompt_ids: Optional[Sequence[int]] = None) -> List[Any]:
         t0 = time.perf_counter()
         s, e = self.local_range(len(clips), microbatch_size(self.engine.max_batch, num_beams, group) if group else None)
-        rows = self.gather(self.run_local(clips, task, language, return_timestamps, num_beams, token_timestamps, group))
+        rows = self.gather(self.run_local(clips, task, language, return_timestamps, num_beams, token_timestamps, group,
+                                          prompt_ids))
         self.last_stats = {"workers": self.world_size, "rank": self.rank, "local_range": (s, e),
                            "seconds": time.perf_counter() - t0}
         return rows
 
     def run_long(self, audio: np.ndarray, task: str = "transcribe", language: Optional[str] = None,
-                 num_beams: int = 1) -> List[int]:
+                 num_beams: int = 1, prompt_ids: Optional[Sequence[int]] = None) -> List[int]:
         """Un-chunked long-form input does not shard (one sequential seek loop): every rank computes the same row."""
+        kw = {} if prompt_ids is None else {"prompt_ids": list(prompt_ids)}
         if hasattr(self.engine, "run_long"):
-            return self.engine.run_long(audio, task=task, language=language, num_beams=num_beams)
-        return self.engine.generate_long_from_pcm(audio, task=task, language=language, num_beams=num_beams)
+            return self.engine.run_long(audio, task=task, language=language, num_beams=num_beams, **kw)
+        return self.engine.generate_long_from_pcm(audio, task=task, language=language, num_beams=num_beams, **kw)
 
     def close(self):
         if hasattr(self.engine, "close"):
