@@ -143,10 +143,7 @@ int tw_shift_frames(const void* src_bf16, void* dst_bf16, const int32_t* src_row
 /* ------------------------------------------------------------------------------------------------
  * K7 / K8  batched greedy decode step (<= 32 rows per call).  All per-row state lives on the
  * device so a step is a fixed launch sequence (CUDA-graph capturable):
- *   row_state: int32 [batch][8] = {pos, finished, last_ts, text_lo, ts_lo, ts_hi, begin, mode}
- *     pos   index in tokens[] of the token fed this step;  mode 1 = language detection
- *     text_lo / ts_lo / ts_hi / begin encode what WhisperTimeStampLogitsProcessor and the two
- *     Suppress* processors allow for the NEXT token ($TF/generation/logits_process.py:1812-2043).
+ *   row_state: tw_row_state [batch] (below; passed as void*)
  *   self-attention KV cache is paged: pool layer base bf16 [2][n_pages][64][D],
  *   block_table int32 [batch][pages_per_row].
  * Replaces WhisperDecoder.forward / WhisperDecoderLayer with cache
@@ -154,6 +151,21 @@ int tw_shift_frames(const void* src_bf16, void* dst_bf16, const int32_t* src_row
  * ($TF/cache_utils.py:102-119), the logits processors and GenerationMixin._sample's
  * fp32-logits -> processors -> argmax -> pad-if-finished step ($TF/generation/utils.py:2762-2797).
  * ---------------------------------------------------------------------------------------------- */
+/* Decoding state of one decode row (8 x int32, 32 bytes).  text_lo / ts_lo / ts_hi / begin encode what
+ * WhisperTimeStampLogitsProcessor and the two Suppress* processors allow for the NEXT token
+ * ($TF/generation/logits_process.py:1812-2043). */
+typedef struct tw_row_state {
+    int32_t pos;        /* index in tokens[] of the token fed this step */
+    int32_t finished;   /* row has emitted eos */
+    int32_t last_ts;    /* last timestamp token generated so far, or -1 */
+    int32_t text_lo;    /* non-timestamp ids < text_lo are forbidden next step */
+    int32_t ts_lo;      /* timestamp ids < ts_lo forbidden */
+    int32_t ts_hi;      /* timestamp ids > ts_hi forbidden (ts_hi < ts_lo: none allowed) */
+    int32_t begin;      /* 1 if the next token is the first generated one (begin-suppress applies) */
+    int32_t mode;       /* bit 0: language detection at this step (only language ids allowed, cleared afterwards);
+                         * bit 1: row generates without timestamps (suppress lists only, plain arg-max) */
+} tw_row_state;
+
 typedef struct tw_skinny_args {
     const void* w;      /* bf16, n rounded up to 16 rows x k, FRAGMENT-MAJOR: [n/16][k/32][2][8][4][8] with element
                          * W[16*slab + 8*half + g][32*kstep + 8*tg + e] (zero rows beyond n) — each warp load of the
@@ -275,7 +287,7 @@ int tw_prefill_cross_attn(const void* q_bf16, int64_t q_ld, void* out_bf16, cons
  * tw_dec_align_tap runs inside the decode step of an alignment layer, right after the cross-attention query
  * projection: for the layer's alignment heads it writes softmax(q_h K_h^T) (fp32, all src_len encoder positions) of
  * every decode row to probs[row][slot0 + i][pos_row][:]  (probs: fp32 [batch][n_slots][max_len][src_len]; pos_row =
- * row_state[row][0]).  K addressing as in tw_dec_cross_attn.  heads_dev: device int32 [n_heads]. */
+ * row_state[row].pos).  K addressing as in tw_dec_cross_attn.  heads_dev: device int32 [n_heads]. */
 int tw_dec_align_tap(const void* q_bf16, int32_t q_ld, const void* k_bf16, int64_t kv_row_stride,
                      int64_t kv_batch_stride, int64_t kv_head_stride, const int32_t* enc_row, const void* row_state,
                      const int32_t* heads_dev, int32_t n_heads, int32_t slot0, int32_t n_slots, int32_t max_len,

@@ -38,20 +38,28 @@ def test_ctypes_table_mirrors_header():
 
 
 def test_struct_layouts_match_header(tmp_path):
-    """sizeof of every struct of the public header, as gcc lays it out in plain C99, equals the ctypes mirror's."""
+    """sizeof and the offsetof of every field of every struct of the public header, as gcc lays it out in plain C99,
+    equal the ctypes mirror's."""
     import subprocess
     from turbo_whisper_workspace_b200 import _lib
     structs = {"tw_gemm_args": _lib.GemmArgs, "tw_skinny_args": _lib.SkinnyArgs, "tw_grammar": _lib.Grammar,
-               "tw_beam_config": _lib.BeamConfig, "tw_beam_state": _lib.BeamState, "tw_flac_info": _lib.FlacInfo}
+               "tw_row_state": _lib.RowState, "tw_beam_config": _lib.BeamConfig, "tw_beam_state": _lib.BeamState,
+               "tw_flac_info": _lib.FlacInfo}
     src = tmp_path / "sizes.c"
-    src.write_text('#include <stdio.h>\n#include "twb200.h"\nint main(void) {\n' +
-                   "".join(f'  printf("{n} %zu\\n", sizeof({n}));\n' for n in structs) + "  return 0;\n}\n")
+    src.write_text('#include <stddef.h>\n#include <stdio.h>\n#include "twb200.h"\nint main(void) {\n' +
+                   "".join(f'  printf("{n} %zu\\n", sizeof({n}));\n' for n in structs) +
+                   "".join(f'  printf("{n}.{f} %zu\\n", offsetof({n}, {f}));\n'
+                           for n, cls in structs.items() for f, _ in cls._fields_) + "  return 0;\n}\n")
     exe = tmp_path / "sizes"
     subprocess.run(["gcc", "-std=c99", "-I", os.path.join(ROOT, "include"), "-o", str(exe), str(src)], check=True)
     out = dict(line.split() for line in subprocess.run([str(exe)], capture_output=True, text=True, check=True).stdout.splitlines())
     for name, cls in structs.items():
         assert int(out[name]) == C.sizeof(cls), f"{name}: header {out[name]} bytes, ctypes {C.sizeof(cls)}"
+        for f, _ in cls._fields_:
+            off = getattr(cls, f).offset
+            assert int(out[f"{name}.{f}"]) == off, f"{name}.{f}: header offset {out[f'{name}.{f}']}, ctypes {off}"
     assert C.sizeof(_lib.GemmArgs) == 144 and C.sizeof(_lib.SkinnyArgs) == 120 and C.sizeof(_lib.Grammar) == 36
+    assert C.sizeof(_lib.RowState) == 32
 
 
 def test_error_convention_without_gpu(lib):

@@ -252,3 +252,59 @@ def test_generate_matches_oracle_varied_prefix(setup):
             n_ok += 1
         agreed += n_ok
     assert agreed >= 3 * B, "free-running prefix agreement is implausibly short"
+
+
+def test_unfolded_layernorm_matches_default(cuda_device, monkeypatch):
+    """TWB200_NO_LN_FOLD (every residual projection's last CTA writes the next LayerNorm) against the default engine
+    (that LayerNorm folded into the projection that consumes it) on the same weights: the same launches per decode step
+    and, teacher-forced on the same tokens, the same logits within the stated bf16 tolerance."""
+    from oracle import whisper_ref as R
+    from turbo_whisper_workspace_b200 import _lib
+    from turbo_whisper_workspace_b200.config import WhisperDims
+    from turbo_whisper_workspace_b200.engine import WhisperEngine
+    clips = [helpers.synth_clip(0), helpers.synth_clip(1, kind="mod"), helpers.synth_clip(2, seconds=11.3, kind="mod")]
+    sd = helpers.variant_state_dict(R.WhisperDims(**helpers.TINY), "varied")
+    B, n_steps = len(clips), 64
+    prompts = torch.tensor([[R.SOT, -1, R.TRANSCRIBE]] * B, dtype=torch.int32)
+    lib = _lib.load()
+    names = [n for n in _lib.SIGNATURES if n.startswith("tw_dec_")]
+    forced, runs = None, []
+    for no_fold in (False, True):
+        if no_fold:
+            monkeypatch.setenv("TWB200_NO_LN_FOLD", "1")
+        else:
+            monkeypatch.delenv("TWB200_NO_LN_FOLD", raising=False)
+        eng = WhisperEngine(WhisperDims(**helpers.TINY), sd, device=cuda_device, max_batch=B)
+        assert eng.ln_fold is not no_fold
+        eng.enable_taps()
+        eng.load_pcm(clips)
+        eng.features(B)
+        eng.encode(B)
+        if forced is None:      # the default engine's greedy tokens, teacher-forced on both
+            forced = eng.decode(B, prompts, n_steps=n_steps).cpu().clone()
+        logits = []
+        launches = eng.stats["launches"]
+        eng.decode(B, prompts, n_steps=n_steps, forced=forced, on_step=lambda s: logits.append(eng.logits[:B].cpu().clone()))
+        launches = eng.stats["launches"] - launches
+        # one eager step with every decode-kernel call recorded
+        seq, saved = [], {n: getattr(lib, n) for n in names}
+        for n in names:
+            setattr(lib, n, lambda *a, _n=n: seq.append(_n) or saved[_n](*a))
+        try:
+            eng._decode_step(B)
+        finally:
+            for n in names:
+                setattr(lib, n, saved[n])
+        torch.cuda.synchronize()
+        assert len(seq) == eng.launches_per_step
+        runs.append((logits, launches, seq))
+    (want, launches, seq), (got, launches_nf, seq_nf) = runs
+    assert launches == launches_nf and seq == seq_nf
+    assert len(got) == len(want) > 0
+    worst = 0.0
+    for s, (g, w) in enumerate(zip(got, want)):
+        err, bound = float((g - w).abs().max()), LOGIT_REL_TOL * float(w.abs().max()) + LOGIT_ABS_FLOOR
+        worst = max(worst, err / bound)
+        assert err < bound, f"step {s}: max |logit unfolded - folded| = {err} > {bound}"
+    print(f"\n[TWB200_NO_LN_FOLD] {len(got)} teacher-forced steps: max |logit diff| / bound = {worst:.3f}; "
+          f"{launches} launches, {len(seq)} per step")

@@ -34,17 +34,10 @@ def _lang_gen(**kw):
 
 def _forced_route(eng, R, row, timestamps):
     """The prompt through the existing step loop: row[0] fed at position 0, row[1:] teacher-forced, the grammar's
-    begin index set by hand to the prompt length.  Returns the row state after the steps that feed positions 0 .. P-2
-    (the state the prefill path sets up by hand); returns after the step that feeds position P-1."""
-    P = len(row)
-    pad = eng.gen.pad_token_id
-    tok0 = torch.full((R, eng.max_len), pad, dtype=torch.int32)
-    tok0[:, 0] = row[0]
-    frc = torch.full((R, eng.max_len), -1, dtype=torch.int32)
-    frc[:, 1:P] = torch.tensor(row[1:], dtype=torch.int32)
-    st0 = torch.zeros(R, 8, dtype=torch.int32)
-    st0[:, 2] = -1
-    st0[:, 7] = 0 if timestamps else 2
+    begin index at the prompt length.  Returns the row state after the steps that feed positions 0 .. P-2 (the state
+    the prefill path starts from); returns after the step that feeds position P-1."""
+    from turbo_whisper_workspace_b200.engine import init_rows
+    tok0, frc, st0, P = init_rows(torch.tensor([row] * R), eng.max_len, eng.grammar, timestamps)
     eng.grammar.begin_index = P
     eng.tokens[:R].copy_(tok0.to(eng.device))
     eng.forced[:R].copy_(frc.to(eng.device))

@@ -54,6 +54,10 @@ class Grammar(C.Structure):
                                        "max_initial_ts", "begin_index")]
 
 
+class RowState(C.Structure):
+    _fields_ = [(n, c_int32) for n in ("pos", "finished", "last_ts", "text_lo", "ts_lo", "ts_hi", "begin", "mode")]
+
+
 # name -> (restype, argtypes); mirrors include/twb200.h one to one (tests/test_abi.py checks it)
 SIGNATURES = {
     "tw_last_error": (C.c_char_p, []),

@@ -222,13 +222,11 @@ HD void apply_plan_rows(const Cfg& c, const State& s, const Plan& p, int n, int 
 // ---------------------------------------------------------------------------------------------------------------
 // device kernels
 // ---------------------------------------------------------------------------------------------------------------
-struct RowState8 { int pos, finished, last_ts, text_lo, ts_lo, ts_hi, begin, mode; };
-
 constexpr int TOPK_THREADS = 1024;
 
 struct TopkParams {
     const float* logits;      // [R][V] raw fp32 logits of this step
-    const RowState8* st;      // [R]
+    const tw_row_state* st;   // [R]
     const float* run_score;   // [R]
     const Gram* gram;         // [R]
     const uint32_t* sup;
@@ -341,7 +339,7 @@ struct AdvanceParams {
     State s;
     const float* cand_val;
     const int* cand_tok;
-    RowState8* st;         // [R]
+    tw_row_state* st;      // [R]
     int* tokens;           // [R][tokens_ld]: the token every decode row feeds next is written at index cur
     int tokens_ld;
     int* block_table;      // [R][ppr]
@@ -385,7 +383,7 @@ __global__ void __launch_bounds__(128) beam_advance_kernel(const AdvanceParams p
         p.origin_out[r] = w * K + o;
         // the decode row: next token, position, grammar state
         if (cur < p.tokens_ld) p.tokens[(size_t)r * p.tokens_ld + cur] = plan.tok[cs];
-        RowState8 st = p.st[r];
+        tw_row_state st = p.st[r];
         st.pos = cur;
         st.finished = 0;
         p.st[r] = st;
@@ -503,12 +501,12 @@ extern "C" int tw_beam_step(const tw_beam_config* b, const tw_beam_state* state,
     cudaStream_t st = (cudaStream_t)stream;
     const int R = n_windows * c.K;
     TopkParams tp;
-    tp.logits = logits; tp.st = (const RowState8*)row_state; tp.run_score = state->run_score; tp.gram = (const Gram*)state->gram;
+    tp.logits = logits; tp.st = (const tw_row_state*)row_state; tp.run_score = state->run_score; tp.gram = (const Gram*)state->gram;
     tp.sup = suppress_bits; tp.bsup = begin_suppress_bits; tp.ctrl = state->ctrl; tp.cand_val = cand_val; tp.cand_tok = cand_tok;
     tp.c = c;
     beam_row_topk_kernel<<<R, TOPK_THREADS, smem, st>>>(tp);
     AdvanceParams ap;
-    ap.s = to_state(state); ap.cand_val = cand_val; ap.cand_tok = cand_tok; ap.st = (RowState8*)row_state; ap.tokens = tokens;
+    ap.s = to_state(state); ap.cand_val = cand_val; ap.cand_tok = cand_tok; ap.st = (tw_row_state*)row_state; ap.tokens = tokens;
     ap.tokens_ld = tokens_ld; ap.block_table = block_table; ap.ppr = pages_per_row; ap.bank_pages = bank_pages;
     ap.copy_src = copy_src; ap.copy_dst = copy_dst; ap.copy_len = copy_len; ap.origin_out = origin_out; ap.n = n_windows;
     ap.c = c;

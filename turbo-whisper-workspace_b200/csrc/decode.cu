@@ -28,21 +28,6 @@ namespace dec {
 constexpr int MAXB = 128;  // decode rows per launch (ln_part / ln_stats strides; engine.MAX_DECODE_BATCH <= this)
 constexpr int PAGE = 64;  // positions per KV page
 
-// ------------------------------------------------------------------------------------------------
-// per-row decoding state (device resident)
-// ------------------------------------------------------------------------------------------------
-struct RowState {
-    int pos;        // index of the token being fed this step (0-based position in tokens[])
-    int finished;   // row has emitted eos
-    int last_ts;    // last timestamp token generated so far, or -1
-    int text_lo;    // non-timestamp ids < text_lo are forbidden next step
-    int ts_lo;      // timestamp ids < ts_lo forbidden
-    int ts_hi;      // timestamp ids > ts_hi forbidden (ts_hi < ts_lo: none allowed)
-    int begin;      // 1 if the next token is the first generated one (begin-suppress applies)
-    int mode;       // bit 0: language detection at this step (only language ids allowed, cleared afterwards);
-                    // bit 1: row generates without timestamps (suppress lists only, plain arg-max)
-};
-
 struct GrammarConst {
     int eos, pad, no_timestamps, ts_begin, vocab, lang_first, lang_last, max_initial_ts, begin_index;
 };
@@ -52,7 +37,7 @@ struct GrammarConst {
 // ------------------------------------------------------------------------------------------------
 // also emits LayerNorm(x) (first decoder layer's self_attn_layer_norm) as bf16 when ln_out is given
 __global__ void __launch_bounds__(256) decode_embed_kernel(const int* __restrict__ tokens, int tokens_ld,
-                                                          const RowState* __restrict__ st,
+                                                          const tw_row_state* __restrict__ st,
                                                           const __nv_bfloat16* __restrict__ tok_emb,
                                                           const float* __restrict__ pos_emb,
                                                           float* __restrict__ x, int D,
@@ -147,7 +132,7 @@ struct SkinnyParams {
     __nv_bfloat16* kv_pool;  // layer base: [2][n_pages][PAGE][D]
     const int* block_table;  // [B, pages_per_row]
     int pages_per_row, n_pages, D;
-    const RowState* st;
+    const tw_row_state* st;
     // EPI_LOGITS
     float* logits_out;       // optional raw logits [B, N]
     const uint32_t* suppress_bits;        // vocab bitmap
@@ -186,7 +171,7 @@ TW_DEVINL void mma_bf16_16816(float (&c)[4], uint32_t a0, uint32_t a1, uint32_t 
         : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
 }
 
-TW_DEVINL bool token_allowed(int v, const RowState& s, const GrammarConst& gc, const uint32_t* sup,
+TW_DEVINL bool token_allowed(int v, const tw_row_state& s, const GrammarConst& gc, const uint32_t* sup,
                              const uint32_t* bsup) {
     if (s.mode & 1) return v >= gc.lang_first && v <= gc.lang_last;
     if (s.mode & 2) return !((sup[v >> 5] >> (v & 31)) & 1u) && !(s.begin && ((bsup[v >> 5] >> (v & 31)) & 1u));
@@ -441,7 +426,7 @@ constexpr int LMH_WARPS = LMH_WARPS_DEF;   // warps per CTA of the persistent LM
 template <int NB>
 __global__ void __launch_bounds__(LMH_WARPS * 32, 1) lmhead_kernel(const SkinnyParams p) {
     // grammar state of the batch rows: shared memory, not 6 register copies per thread (the registers go to fragments)
-    __shared__ RowState s_st[MAXB];
+    __shared__ tw_row_state s_st[MAXB];
     constexpr int UN = 4;  // k-steps (of 32) per round
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int g = lane >> 2, tg = lane & 3;
@@ -539,7 +524,7 @@ __global__ void __launch_bounds__(LMH_WARPS * 32, 1) lmhead_kernel(const SkinnyP
         for (int c = 0; c < NB * 2; ++c) {
             const int j = c >> 1, e = c & 1;
             const int bb = j * 8 + 2 * tg + e;
-            const RowState& rs = s_st[min(bb, p.B - 1)];
+            const tw_row_state& rs = s_st[min(bb, p.B - 1)];
             float vt = -INFINITY, vs = -INFINITY;
             int jt = 0x7fffffff, js = 0x7fffffff;
             bool ts_ok[2];
@@ -628,7 +613,7 @@ struct FinalizeParams {
     int tokens_ld;
     const int* forced;  // [B, tokens_ld]: forced[b][i] >= 0 overrides the token written at index i
     int* choices;       // optional [B, tokens_ld]: the engine's own pick before the forced override
-    RowState* st;
+    tw_row_state* st;
     GrammarConst gc;
     int max_len;        // generation stops writing at tokens_ld / max_length
 };
@@ -685,7 +670,7 @@ __global__ void __launch_bounds__(128) decode_finalize_kernel(const FinalizePara
     __syncthreads();
     if (tid == 0) {
         for (int w = 1; w < 4; ++w) merge(s_text[w], s_itext[w], s_ts[w], s_its[w], s_sum[w]);
-        RowState s = p.st[b];
+        tw_row_state s = p.st[b];
         const GrammarConst& gc = p.gc;
         int tok;
         if (s.mode != 0) {
@@ -751,7 +736,7 @@ struct AttnParams {
     const __nv_bfloat16* kv_pool;
     const int* block_table;
     int pages_per_row, n_pages;
-    const RowState* st;
+    const tw_row_state* st;
     // cross: K row j of (row b, head h) at ck + b*batch_stride + h*head_stride + j*row_stride (elements)
     const __nv_bfloat16* ck;
     const __nv_bfloat16* cv;
@@ -939,7 +924,7 @@ static cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
     return cudaLaunchKernelEx(&cfg, kernel, args...);
 }
 
-static_assert(sizeof(RowState) == 32, "RowState layout is part of the ABI (8 x int32)");
+static_assert(sizeof(tw_row_state) == 32, "tw_row_state layout is part of the ABI (8 x int32)");
 
 template <int EPI, int WARPS, bool LNF = false>
 static int launch_nb(const SkinnyParams& p, int grid, cudaStream_t st) {
@@ -980,7 +965,7 @@ extern "C" int tw_dec_embed(const int32_t* tokens, int32_t tokens_ld, const void
     TW_REQUIRE(!ln_out_bf16 || (ln_gamma && ln_beta), "tw_dec_embed: LayerNorm output needs gamma and beta");
     if (batch <= 0) return 0;
     TW_CUDA_CHECK(launch_pdl(decode_embed_kernel, dim3(batch), dim3(256), 0, (cudaStream_t)stream, tokens, (int)tokens_ld,
-                             (const RowState*)row_state, (const __nv_bfloat16*)tok_emb_bf16, pos_emb, x, (int)d_model,
+                             (const tw_row_state*)row_state, (const __nv_bfloat16*)tok_emb_bf16, pos_emb, x, (int)d_model,
                              ln_gamma, ln_beta, (__nv_bfloat16*)ln_out_bf16));
     TW_CUDA_CHECK(cudaGetLastError());
     return 0;
@@ -1054,7 +1039,7 @@ extern "C" int tw_dec_qkv(const tw_skinny_args* a, void* q_out_bf16, void* kv_po
     p.pages_per_row = pages_per_row;
     p.n_pages = n_pages;
     p.D = a->n / 3;
-    p.st = (const RowState*)row_state;
+    p.st = (const tw_row_state*)row_state;
     return launch_skinny<EPI_QKV>(p, (cudaStream_t)stream);
 }
 
@@ -1082,7 +1067,7 @@ extern "C" int tw_dec_lmhead(const tw_skinny_args* a, const tw_grammar* g, const
     TW_REQUIRE(a->n == g->vocab, "tw_dec_lmhead: N (%d) != vocab (%d)", a->n, g->vocab);
     SkinnyParams p;
     fill_common(p, a);
-    p.st = (const RowState*)row_state;
+    p.st = (const tw_row_state*)row_state;
     p.suppress_bits = suppress_bits;
     p.begin_suppress_bits = begin_suppress_bits;
     p.gc = to_gc(g);
@@ -1112,7 +1097,7 @@ extern "C" int tw_dec_finalize(const float* part_val, const int32_t* part_idx, i
     if (batch <= 0) return 0;
     FinalizeParams p;
     p.part_val = part_val; p.part_idx = part_idx; p.n_parts = n_parts; p.tokens = tokens; p.tokens_ld = tokens_ld;
-    p.forced = forced; p.choices = choices; p.st = (RowState*)row_state; p.gc = to_gc(g); p.max_len = tokens_ld;
+    p.forced = forced; p.choices = choices; p.st = (tw_row_state*)row_state; p.gc = to_gc(g); p.max_len = tokens_ld;
     TW_CUDA_CHECK(launch_pdl(decode_finalize_kernel, dim3(batch), dim3(128), 0, (cudaStream_t)stream, p));
     TW_CUDA_CHECK(cudaGetLastError());
     return 0;
@@ -1128,7 +1113,7 @@ extern "C" int tw_dec_self_attn(const void* q_bf16, void* out_bf16, const void* 
     AttnParams p{};
     p.q = (const __nv_bfloat16*)q_bf16; p.out = (__nv_bfloat16*)out_bf16; p.D = heads * 64; p.H = heads;
     p.is_cross = 0; p.kv_pool = (const __nv_bfloat16*)kv_pool_layer; p.block_table = block_table;
-    p.pages_per_row = pages_per_row; p.n_pages = n_pages; p.st = (const RowState*)row_state; p.splits = 1;
+    p.pages_per_row = pages_per_row; p.n_pages = n_pages; p.st = (const tw_row_state*)row_state; p.splits = 1;
     TW_CUDA_CHECK(launch_pdl(decode_attn_kernel, dim3(1, heads, batch), dim3(ATT_THREADS), 0, (cudaStream_t)stream, p));
     TW_CUDA_CHECK(cudaGetLastError());
     return 0;

@@ -25,7 +25,7 @@ struct TapParams {
     const __nv_bfloat16* k;      // this layer's K, element (row, head, j, e) at k + row*bs + head*hs + j*rs + e
     long long rs, bs, hs;
     const int* enc_row;          // decode row -> encoder-batch row
-    const int* row_state;        // int32 [batch][8]; [0] = position of the token fed this step
+    const tw_row_state* row_state;  // [batch]
     const int* heads;            // device int32 [n_heads]: head index of every alignment slot of this layer
     int slot0, n_slots, max_len, src_len, q_ld;
     float* probs;                // [batch][n_slots][max_len][src_len]
@@ -60,7 +60,7 @@ __global__ void __launch_bounds__(TAP_THREADS) align_tap_kernel(const TapParams 
     __shared__ float red[TAP_THREADS / 32];
     const int b = blockIdx.y, slot = blockIdx.x;
     const int h = p.heads[slot];
-    const int pos = p.row_state[b * 8 + 0];
+    const int pos = p.row_state[b].pos;
     if (pos < 0 || pos >= p.max_len) return;    // uniform per CTA
     if (threadIdx.x < 64) qs[threadIdx.x] = __bfloat162float(p.q[(long long)b * p.q_ld + h * 64 + threadIdx.x]);
     __syncthreads();
@@ -192,7 +192,7 @@ extern "C" int tw_dec_align_tap(const void* q_bf16, int32_t q_ld, const void* k_
     p.q = (const __nv_bfloat16*)q_bf16;
     p.k = (const __nv_bfloat16*)k_bf16;
     p.rs = kv_row_stride; p.bs = kv_batch_stride; p.hs = kv_head_stride;
-    p.enc_row = enc_row; p.row_state = (const int*)row_state; p.heads = heads_dev;
+    p.enc_row = enc_row; p.row_state = (const tw_row_state*)row_state; p.heads = heads_dev;
     p.slot0 = slot0; p.n_slots = n_slots; p.max_len = max_len; p.src_len = src_len; p.q_ld = q_ld;
     p.probs = probs;
     align_tap_kernel<<<dim3(n_heads, batch), TAP_THREADS, 0, (cudaStream_t)stream>>>(p);

@@ -29,7 +29,7 @@ LMHEAD_ROWS = 48
 _CAPTURE_LOCK = threading.Lock()   # CUDA-graph capture is serialised across the engine contexts of a process
 _PREFILL_WEIGHTS_LOCK = threading.Lock()   # the contexts of a device share (and lazily extend) one weight dict
 PAGE = 64
-ROWSTATE_INTS = 8
+ROW_STATE = np.dtype(_lib.RowState)   # tw_row_state of include/twb200.h as a numpy record
 
 
 def _bf16(t: torch.Tensor) -> torch.Tensor:
@@ -212,6 +212,35 @@ def retrieve_segment(seq: List[int], seek_num_frames: int, ts_begin: int):
     return segs, (seq[last - 2] - ts_begin) * 2  # input_stride = 2 mel frames per encoder position
 
 
+def init_rows(rows: torch.Tensor, max_len: int, g: Grammar, timestamps: bool, prefilled: bool = False,
+              flat: bool = False):
+    """Host-side start of R decode rows whose decoder prompts are ``rows`` (int [R, P], :meth:`WhisperEngine.prompt_row`;
+    a language of -1 asks for language detection at position 0).  Returns (tokens int32 [R, max_len], forced int32
+    [R, max_len], state int32 [R, 8] = tw_row_state [R], the grammar's begin_index = P).
+    ``prefilled``: positions 0 .. P-2 run as one prefill (:meth:`WhisperEngine.prefill`) and the state is the one the
+    forced steps would leave at position P-1; otherwise the steps feed row[0] and teacher-force the rest of the row.
+    ``flat`` (beam search): the grammar is applied by tw_beam_step on the tapped logits, not by the LM head."""
+    R, P = rows.shape
+    rows = rows.to(torch.int32)
+    tokens = torch.full((R, max_len), g.pad, dtype=torch.int32)
+    forced = torch.full((R, max_len), -1, dtype=torch.int32)
+    st = np.zeros(R, dtype=ROW_STATE)
+    st["last_ts"] = -1
+    st["mode"] = (rows < 0).any(dim=1).numpy() | (2 if flat or not timestamps else 0)
+    if prefilled or flat:
+        tokens[:, :P] = rows
+    else:
+        tokens[:, 0] = rows[:, 0]
+    if flat or not prefilled:
+        forced[:, 1:P] = rows[:, 1:]      # an unknown language (-1) stays free
+    if prefilled:
+        st["pos"] = P - 1
+        st["text_lo"] = st["ts_lo"] = g.ts_begin
+        st["ts_hi"] = g.ts_begin + g.max_initial_ts
+        st["begin"] = 1
+    return tokens, forced, torch.from_numpy(st.view(np.int32).reshape(R, -1)), P
+
+
 class WhisperEngine:
     """One engine per GPU.  ``max_batch`` bounds the number of 30 s windows processed together."""
 
@@ -263,10 +292,10 @@ class WhisperEngine:
             self.pages_per_row = (self.max_len + PAGE - 1) // PAGE
             self.n_pages = Bm * self.pages_per_row
             self.kv_pool = z(L, 2, self.n_pages, PAGE, D, dtype=bf)
-            self.block_table = torch.arange(self.n_pages, dtype=i32, device=dev).view(Bm, self.pages_per_row).contiguous()
+            self.block_table = z(Bm, self.pages_per_row, dtype=i32)
             self.tokens = z(Bm, self.max_len, dtype=i32)
             self.forced = torch.full((Bm, self.max_len), -1, dtype=i32, device=dev)
-            self.state = z(Bm, ROWSTATE_INTS, dtype=i32)
+            self.state = z(Bm, ROW_STATE.itemsize // 4, dtype=i32)
             self.dx = z(Bm, D, dtype=f32)
             self.dxn = z(Bm, D, dtype=bf)
             self.dxb = z(Bm, D, dtype=bf)                        # bf16 copy of the residual rows (operand of the folded-LayerNorm projections)
@@ -282,8 +311,8 @@ class WhisperEngine:
             self.cross_part = z(Bm, dims.heads, cross_splits, 66, dtype=f32)
             self.cross_cnt = z(Bm, dims.heads, dtype=i32)
             self.ln_cnt = z(1, dtype=i32)
-            # decode row -> window of the encoder batch whose cross K/V it reads (identity; beams of one window share a row)
-            self.enc_row = torch.arange(Bm, dtype=i32, device=dev)
+            self.enc_row = z(Bm, dtype=i32)
+            self._identity_rows()
             self.align = None    # word-timestamp workspaces (enable_alignment)
             self._align_on = False
             self.logits = None   # optional [Bm, vocab] fp32 raw-logit tap for parity tests
@@ -313,6 +342,13 @@ class WhisperEngine:
     # ------------------------------------------------------------------------------------ helpers
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+
+    def _identity_rows(self):
+        """Decode row r reads the cross K/V of encoder window r (enc_row) and owns the KV pages r * pages_per_row ..
+        (block_table).  Beam search permutes both and restores them with this."""
+        dev, Bm, ppr = self.device, self.max_batch, self.pages_per_row
+        self.enc_row.copy_(torch.arange(Bm, dtype=torch.int32, device=dev))
+        self.block_table.copy_(torch.arange(Bm * ppr, dtype=torch.int32, device=dev).view(Bm, ppr))
 
     def enable_taps(self):
         """Parity-test taps: raw fp32 logits of the last step and the un-forced picks of every step."""
@@ -499,6 +535,14 @@ class WhisperEngine:
             a.ln_stats_in, a.ln_c = self.ln_stats.data_ptr(), self.w[fold + "_c"].data_ptr()
         return a
 
+    def _cross_kv(self, i: int):
+        """K and V pointers of decoder layer i in the head-major cross K/V ([(layer, k|v, head)][window][position][64] of
+        the encoder batch that produced self.ckv) and the elements per (layer, k|v, head) block."""
+        H, S = self.dims.heads, self.dims.max_source_positions
+        blk = self._ckv_batch * S * 64
+        base = self.ckv.data_ptr()
+        return C.c_void_p(base + ((i * 2 + 0) * H) * blk * 2), C.c_void_p(base + ((i * 2 + 1) * H) * blk * 2), blk
+
     def _decode_step(self, B: int, finalize: bool = True) -> None:
         """One greedy step for rows 0..B-1: fixed launch sequence, positions read from self.state.
         ``finalize=False`` (beam search): the LM head only taps the raw logits; tw_beam_step picks the tokens."""
@@ -508,72 +552,46 @@ class WhisperEngine:
         S = d.max_source_positions
         check(lib.tw_dec_embed(p(self.tokens), self.max_len, p(self.state), p(w["tok_emb"]), p(w["dec_pos"]), p(self.dx),
                                B, D, p(w["dec0.ln1_w"]), p(w["dec0.ln1_b"]), p(self.dxn), st), "tw_dec_embed")
-        Bc = self._ckv_batch                 # windows in the encoder batch that produced self.ckv
-        blk = Bc * S * 64                    # elements per (layer, k|v, head) block of the head-major K/V
-        if not self.ln_fold:
-            # round-1 form: a last-CTA LayerNorm fused into every residual projection (TWB200_NO_LN_FOLD, A/B only)
-            for i in range(L):
-                q = f"dec{i}."
-                nxt = f"dec{i + 1}.ln1" if i + 1 < L else "dec_ln"
-                pool = C.c_void_p(self.kv_pool[i].data_ptr())
-                check(lib.tw_dec_qkv(C.byref(self._skinny(q + "qkv_w", self.dxn, q + "qkv_b", B, D)), p(self.dq), pool,
-                                     p(self.block_table), self.pages_per_row, self.n_pages, p(self.state), st), "tw_dec_qkv")
-                check(lib.tw_dec_self_attn(p(self.dq), p(self.datt), pool, p(self.block_table), self.pages_per_row,
-                                           self.n_pages, p(self.state), B, H, st), "tw_dec_self_attn")
-                check(lib.tw_dec_linear(C.byref(self._skinny(q + "out_w", self.datt, q + "out_b", B, D, ln=q + "ln2")), 2,
-                                        p(self.dx), D, st), "self out_proj")
-                check(lib.tw_dec_linear(C.byref(self._skinny(q + "cq_w", self.dxn, q + "cq_b", B, D)), 0, p(self.dq), D, st),
-                      "cross q_proj")
-                kptr = C.c_void_p(self.ckv.data_ptr() + ((i * 2 + 0) * H) * blk * 2)
-                vptr = C.c_void_p(self.ckv.data_ptr() + ((i * 2 + 1) * H) * blk * 2)
-                if self._align_on and i in self.align["layers"]:
-                    al = self.align
-                    for slot0, heads_dev in al["layers"][i]:
-                        check(lib.tw_dec_align_tap(p(self.dq), D, kptr, 64, S * 64, blk, p(self.enc_row), p(self.state),
-                                                   p(heads_dev), int(heads_dev.numel()), slot0, al["n_slots"], self.max_len,
-                                                   S, B, p(al["probs"]), st), "tw_dec_align_tap")
-                check(lib.tw_dec_cross_attn(p(self.dq), p(self.datt), kptr, vptr, 64, S * 64, blk, p(self.enc_row), S, B, H,
-                                            self.cross_splits, p(self.cross_part), p(self.cross_cnt), st), "tw_dec_cross_attn")
-                check(lib.tw_dec_linear(C.byref(self._skinny(q + "cout_w", self.datt, q + "cout_b", B, D, ln=q + "ln3")), 2,
-                                        p(self.dx), D, st), "cross out_proj")
-                check(lib.tw_dec_linear(C.byref(self._skinny(q + "fc1_w", self.dxn, q + "fc1_b", B, D)), 3, p(self.dhid), F, st),
-                      "fc1")
-                check(lib.tw_dec_linear(C.byref(self._skinny(q + "fc2_w", self.dhid, q + "fc2_b", B, F, ln=nxt)), 2,
-                                        p(self.dx), D, st), "fc2")
-        else:
-            # Every LayerNorm but the first (embedding kernel) and the last (LM head operand) is folded into the projection
-            # that consumes it: the residual projections publish bf16(x) + per-CTA partials, no serial LayerNorm tail.
-            for i in range(L):
-                q = f"dec{i}."
-                last = i + 1 == L
-                pool = C.c_void_p(self.kv_pool[i].data_ptr())
-                qkv_args = self._skinny(q + "qkv_w", self.dxn, q + "qkv_b", B, D) if i == 0 else \
-                    self._skinny(None, self.dxb, None, B, D, fold=q + "qkv")
-                check(lib.tw_dec_qkv(C.byref(qkv_args), p(self.dq), pool,
-                                     p(self.block_table), self.pages_per_row, self.n_pages, p(self.state), st), "tw_dec_qkv")
-                check(lib.tw_dec_self_attn(p(self.dq), p(self.datt), pool, p(self.block_table), self.pages_per_row,
-                                           self.n_pages, p(self.state), B, H, st), "tw_dec_self_attn")
-                check(lib.tw_dec_linear(C.byref(self._skinny(q + "out_w", self.datt, q + "out_b", B, D, part_out=True)), 2,
-                                        p(self.dx), D, st), "self out_proj")
-                check(lib.tw_dec_linear(C.byref(self._skinny(None, self.dxb, None, B, D, fold=q + "cq")), 0, p(self.dq), D, st),
-                      "cross q_proj")
-                kptr = C.c_void_p(self.ckv.data_ptr() + ((i * 2 + 0) * H) * blk * 2)
-                vptr = C.c_void_p(self.ckv.data_ptr() + ((i * 2 + 1) * H) * blk * 2)
-                if self._align_on and i in self.align["layers"]:
-                    al = self.align
-                    for slot0, heads_dev in al["layers"][i]:
-                        check(lib.tw_dec_align_tap(p(self.dq), D, kptr, 64, S * 64, blk, p(self.enc_row), p(self.state),
-                                                   p(heads_dev), int(heads_dev.numel()), slot0, al["n_slots"], self.max_len,
-                                                   S, B, p(al["probs"]), st), "tw_dec_align_tap")
-                check(lib.tw_dec_cross_attn(p(self.dq), p(self.datt), kptr, vptr, 64, S * 64, blk, p(self.enc_row), S, B, H,
-                                            self.cross_splits, p(self.cross_part), p(self.cross_cnt), st), "tw_dec_cross_attn")
-                check(lib.tw_dec_linear(C.byref(self._skinny(q + "cout_w", self.datt, q + "cout_b", B, D, part_out=True)), 2,
-                                        p(self.dx), D, st), "cross out_proj")
-                check(lib.tw_dec_linear(C.byref(self._skinny(None, self.dxb, None, B, D, fold=q + "fc1")), 3, p(self.dhid), F, st),
-                      "fc1")
-                fc2 = self._skinny(q + "fc2_w", self.dhid, q + "fc2_b", B, F, ln="dec_ln") if last else \
-                    self._skinny(q + "fc2_w", self.dhid, q + "fc2_b", B, F, part_out=True)
-                check(lib.tw_dec_linear(C.byref(fc2), 2, p(self.dx), D, st), "fc2")
+        fold = self.ln_fold
+
+        def normed(q, base, folded):
+            """A projection that reads a LayerNorm output: folded into its weights (operand bf16(x)) or not (dxn)."""
+            if folded:
+                return self._skinny(None, self.dxb, None, B, D, fold=q + base)
+            return self._skinny(q + base + "_w", self.dxn, q + base + "_b", B, D)
+
+        def resid(q, base, x, k, ln):
+            """A residual projection followed by LayerNorm ``ln``.  With ln_fold it publishes bf16(x) + per-CTA partials
+            for the folded consumer (no serial LayerNorm tail), except before the LM head (dec_ln); without (the round-1
+            form, TWB200_NO_LN_FOLD, A/B only) its last CTA writes LayerNorm(x) into dxn."""
+            if fold and ln != "dec_ln":
+                return self._skinny(q + base + "_w", x, q + base + "_b", B, k, part_out=True)
+            return self._skinny(q + base + "_w", x, q + base + "_b", B, k, ln=ln)
+
+        for i in range(L):
+            q = f"dec{i}."
+            nxt = f"dec{i + 1}.ln1" if i + 1 < L else "dec_ln"
+            pool = C.c_void_p(self.kv_pool[i].data_ptr())
+            # layer 0's first LayerNorm is computed by the embedding kernel
+            check(lib.tw_dec_qkv(C.byref(normed(q, "qkv", fold and i > 0)), p(self.dq), pool,
+                                 p(self.block_table), self.pages_per_row, self.n_pages, p(self.state), st), "tw_dec_qkv")
+            check(lib.tw_dec_self_attn(p(self.dq), p(self.datt), pool, p(self.block_table), self.pages_per_row,
+                                       self.n_pages, p(self.state), B, H, st), "tw_dec_self_attn")
+            check(lib.tw_dec_linear(C.byref(resid(q, "out", self.datt, D, q + "ln2")), 2, p(self.dx), D, st), "self out_proj")
+            check(lib.tw_dec_linear(C.byref(normed(q, "cq", fold)), 0, p(self.dq), D, st), "cross q_proj")
+            kptr, vptr, blk = self._cross_kv(i)
+            if self._align_on and i in self.align["layers"]:
+                al = self.align
+                for slot0, heads_dev in al["layers"][i]:
+                    check(lib.tw_dec_align_tap(p(self.dq), D, kptr, 64, S * 64, blk, p(self.enc_row), p(self.state),
+                                               p(heads_dev), int(heads_dev.numel()), slot0, al["n_slots"], self.max_len,
+                                               S, B, p(al["probs"]), st), "tw_dec_align_tap")
+            check(lib.tw_dec_cross_attn(p(self.dq), p(self.datt), kptr, vptr, 64, S * 64, blk, p(self.enc_row), S, B, H,
+                                        self.cross_splits, p(self.cross_part), p(self.cross_cnt), st), "tw_dec_cross_attn")
+            check(lib.tw_dec_linear(C.byref(resid(q, "cout", self.datt, D, q + "ln3")), 2, p(self.dx), D, st),
+                  "cross out_proj")
+            check(lib.tw_dec_linear(C.byref(normed(q, "fc1", fold)), 3, p(self.dhid), F, st), "fc1")
+            check(lib.tw_dec_linear(C.byref(resid(q, "fc2", self.dhid, F, nxt)), 2, p(self.dx), D, st), "fc2")
         for r0 in range(0, B, LMHEAD_ROWS):      # the LM head kernel holds its per-row partials in registers: 48 rows per launch
             rows = min(LMHEAD_ROWS, B - r0)
             check(lib.tw_dec_lmhead(C.byref(self._skinny("tok_emb_frag", self.dxn[r0:], None, rows, D)), C.byref(self.grammar),
@@ -649,7 +667,6 @@ class WhisperEngine:
         st = self._stream()
         x, xn, qkv, att, hid = self.x[:M], self.xn[:M], self.qkv[:M], self.att[:M], self.hid[:M]
         cq = self.qkv.view(-1)[:M * D].view(M, D)
-        blk = self._ckv_batch * S * 64
         events: List[tuple] = []
 
         def mark(kind):
@@ -696,8 +713,7 @@ class WhisperEngine:
                 norm("cq")
                 gemm("cq", xn, cq)
                 mark("attn")
-                kptr = C.c_void_p(self.ckv.data_ptr() + ((i * 2 + 0) * H) * blk * 2)
-                vptr = C.c_void_p(self.ckv.data_ptr() + ((i * 2 + 1) * H) * blk * 2)
+                kptr, vptr, blk = self._cross_kv(i)
                 check(lib.tw_prefill_cross_attn(p(cq), D, p(att), kptr, vptr, 64, S * 64, blk, p(self.enc_row), S, R, T,
                                                 H, st), "tw_prefill_cross_attn")
                 launches += 2
@@ -718,33 +734,44 @@ class WhisperEngine:
         ValueError (before any device work) unless it is shorter than min(max_length, max_target_positions)."""
         return decoder_prompt_len(prompt_ids, timestamps, self.max_len)
 
+    def prompt_row(self, prompt_ids: Optional[Sequence[int]], prompt: Sequence[int], timestamps: bool) -> List[int]:
+        """The decoder prompt of one row: prompt_ids + ``prompt`` ([<|startoftranscript|>, language, task])
+        (+ <|notimestamps|> without timestamps)."""
+        return ([] if prompt_ids is None else [int(v) for v in prompt_ids]) + [int(v) for v in prompt] + \
+            ([] if timestamps else [self.gen.no_timestamps_token_id])
+
     @property
     def launches_per_step(self) -> int:
         taps = sum(len(r) for r in self.align["layers"].values()) if self._align_on else 0
         return 1 + 8 * self.dims.dec_layers + 2 + taps      # (+ one more LM-head launch per 48 rows beyond the first 48)
 
-    def _graph_for(self, B: int) -> torch.cuda.CUDAGraph:
-        # the K/V block stride depends on the encoder batch; begin_index (3 / 4 with <|notimestamps|>) is a kernel argument
-        key = (B, self._ckv_batch, int(self.grammar.begin_index), self._align_on)
+    def _graph(self, key: tuple, step, mutated: Sequence[torch.Tensor]) -> torch.cuda.CUDAGraph:
+        """The CUDA graph of ``step()`` cached under ``key``.  A new one is captured after a warm-up run outside capture
+        (sets kernel attributes); ``mutated``, everything the step writes, is restored after the warm-up and the capture."""
         g = self._graphs.get(key)
         if g is None:
-            # a warm-up step outside capture (sets kernel attributes); state is re-initialised afterwards
-            state_backup = self.state.clone()
-            tokens_backup = self.tokens.clone()
-            self._decode_step(B)
+            saved = [t.clone() for t in mutated]
+
+            def restore():
+                for t, v in zip(mutated, saved):
+                    t.copy_(v)
+            step()
             torch.cuda.current_stream(self.device).synchronize()
-            self.state.copy_(state_backup)
-            self.tokens.copy_(tokens_backup)
+            restore()
             g = torch.cuda.CUDAGraph()
             with _CAPTURE_LOCK:
                 # explicit per-device capture stream: torch's default capture stream is a process-wide singleton
                 # that lives on whichever device captured first
                 with torch.cuda.graph(g, stream=self._capture_stream, capture_error_mode="thread_local"):
-                    self._decode_step(B)
-            self.state.copy_(state_backup)
-            self.tokens.copy_(tokens_backup)
+                    step()
+            restore()
             self._graphs[key] = g
         return g
+
+    def _graph_for(self, B: int) -> torch.cuda.CUDAGraph:
+        # the K/V block stride depends on the encoder batch; begin_index (3 / 4 with <|notimestamps|>) is a kernel argument
+        key = (B, self._ckv_batch, int(self.grammar.begin_index), self._align_on)
+        return self._graph(key, lambda: self._decode_step(B), [self.state, self.tokens])
 
     def decode(self, B: int, prompts: Optional[torch.Tensor], n_steps: Optional[int] = None,
                forced: Optional[torch.Tensor] = None, on_step=None, timestamps: bool = True,
@@ -762,46 +789,24 @@ class WhisperEngine:
         Returns the int32 token matrix [B, max_len] on the device (prompt included)."""
         dev = self.device
         max_len = self.max_len
+        prefilled = prompt_ids is not None
         with torch.cuda.device(dev):
-            tok0 = torch.full((B, max_len), self.gen.pad_token_id, dtype=torch.int32)
-            frc = torch.full((B, max_len), -1, dtype=torch.int32) if forced is None else forced.clone().cpu().to(torch.int32)
-            st0 = torch.zeros(B, ROWSTATE_INTS, dtype=torch.int32)
-            st0[:, 2] = -1
             pr = prompts.cpu()
-            P = 0
-            if prompt_ids is None:
-                for b in range(B):
-                    tok0[b, 0] = int(pr[b, 0])
-                    if int(pr[b, 1]) < 0:
-                        st0[b, 7] = 1          # language detection at position 0
-                    else:
-                        frc[b, 1] = int(pr[b, 1])
-                    frc[b, 2] = int(pr[b, 2])
-                    if not timestamps:
-                        st0[b, 7] |= 2
-                        frc[b, 3] = self.gen.no_timestamps_token_id
-                self.grammar.begin_index = 3 if timestamps else 4
-            else:
+            if prefilled:
                 if bool((pr[:, 1] < 0).any()):
                     raise ValueError("decode with prompt_ids needs the language of every row (detect it first)")
-                tail = [] if timestamps else [self.gen.no_timestamps_token_id]
-                P = self.prompt_row_len(prompt_ids, timestamps)
-                tok0[:, :P] = torch.tensor([list(prompt_ids) + [int(v) for v in pr[b, :3]] + tail for b in range(B)],
-                                           dtype=torch.int32)
-                # the row state the forced steps would leave at position P-1: the next token is the first generated one
-                g = self.grammar
-                st0[:, 0] = P - 1
-                st0[:, 3] = st0[:, 4] = g.ts_begin
-                st0[:, 5] = g.ts_begin + g.max_initial_ts
-                st0[:, 6] = 1
-                st0[:, 7] = 0 if timestamps else 2
-                g.begin_index = P
+                self.prompt_row_len(prompt_ids, timestamps)
+            rows = torch.tensor([self.prompt_row(prompt_ids, pr[b, :3], timestamps) for b in range(B)], dtype=torch.int32)
+            tok0, frc, st0, self.grammar.begin_index = init_rows(rows, max_len, self.grammar, timestamps, prefilled)
+            if forced is not None:      # the caller's teacher forcing wherever the prompt leaves a position free
+                frc = torch.where(frc >= 0, frc, forced.cpu().to(torch.int32))
             self.tokens[:B].copy_(tok0.to(dev, non_blocking=False))
             self.forced[:B].copy_(frc.to(dev))
             self.state[:B].copy_(st0.to(dev))
-            self.stats["h2d_bytes"] += 2 * B * max_len * 4 + B * ROWSTATE_INTS * 4
+            self.stats["h2d_bytes"] += tok0.nbytes + frc.nbytes + st0.nbytes
             steps = (max_len - 1) if n_steps is None else min(n_steps, max_len - 1)
-            if P:
+            if prefilled:
+                P = rows.shape[1]
                 self.prefill(B, P, timing=prefill_timing)
                 steps = min(steps, max_len - P)
             _lib.load().tw_set_pdl(0 if (self.use_graphs or os.environ.get("TWB200_NO_PDL")) else 1)   # PDL only pays off for eager stepping
@@ -814,8 +819,8 @@ class WhisperEngine:
                 if on_step is not None:
                     on_step(s)
                 if self.finish_check_every and (s + 1) % self.finish_check_every == 0 and s + 1 < steps:
-                    self.stats["d2h_bytes"] += B * ROWSTATE_INTS * 4
-                    if bool(self.state[:B].cpu()[:, 1].all()):   # every row has emitted eos
+                    self.stats["d2h_bytes"] += B * ROW_STATE.itemsize
+                    if self.state[:B].cpu().numpy().view(ROW_STATE)["finished"].all():   # every row has emitted eos
                         steps = s + 1
                         break
             self.stats["dec_steps"] += steps
@@ -904,34 +909,17 @@ class WhisperEngine:
         self._enable_beam_pool()
         want_frames = frames_keep is not None
         with torch.cuda.device(dev):
-            tail = [] if timestamps else [gen.no_timestamps_token_id]
-            head = [] if prompt_ids is None else [int(v) for v in prompt_ids]
             if prompt_ids is not None:
-                self.prompt_row_len(head, timestamps)
-            prompt = torch.cat([torch.tensor([head] * n, dtype=torch.long).view(n, len(head)), prompts.to(torch.long).cpu(),
-                                torch.tensor([tail] * n, dtype=torch.long).view(n, len(tail))], dim=1)
-            P = prompt.shape[1]
-            rows_prompt = prompt.repeat_interleave(K, dim=0)                      # [R, P]
-            tok0 = torch.full((R, self.max_len), gen.pad_token_id, dtype=torch.int32)
-            tok0[:, :P] = rows_prompt.to(torch.int32)
-            frc = torch.full((R, self.max_len), -1, dtype=torch.int32)
-            frc[:, 1:P] = rows_prompt[:, 1:].to(torch.int32)
-            st0 = torch.zeros(R, ROWSTATE_INTS, dtype=torch.int32)
-            st0[:, 2] = -1
-            st0[:, 7] = 2      # "flat" mode: the grammar is applied by tw_beam_step on the tapped logits, not by the LM head
-            if prompt_ids is not None:
-                # prefilled prompt: the row state the forced steps would leave at position P-1
-                st0[:, 0] = P - 1
-                st0[:, 3] = st0[:, 4] = self.grammar.ts_begin
-                st0[:, 5] = self.grammar.ts_begin + self.grammar.max_initial_ts
-                st0[:, 6] = 1
+                self.prompt_row_len(prompt_ids, timestamps)
+            prompt = torch.tensor([self.prompt_row(prompt_ids, pr, timestamps) for pr in prompts.cpu()], dtype=torch.int32)
+            tok0, frc, st0, P = init_rows(prompt.repeat_interleave(K, dim=0), self.max_len, self.grammar, timestamps,
+                                          prefilled=prompt_ids is not None, flat=True)
+            self.grammar.begin_index = P
             self.tokens[:R].copy_(tok0.to(dev))
             self.forced[:R].copy_(frc.to(dev))
             self.state[:R].copy_(st0.to(dev))
+            self._identity_rows()
             self.enc_row[:R].copy_((torch.arange(R, dtype=torch.int32) // K).to(dev))
-            self.block_table.copy_(torch.arange(self.max_batch * self.pages_per_row, dtype=torch.int32,
-                                                device=dev).view(self.max_batch, self.pages_per_row))
-            self.grammar.begin_index = P
             _lib.load().tw_set_pdl(0)
             # ---- search state
             ws = self._beam_workspace(n, K, P, timestamps, want_frames)
@@ -941,7 +929,7 @@ class WhisperEngine:
             if want_frames:
                 ws["hist"][..., L:] = -1
                 ws["fin"][..., L:] = -1
-            ws["hist"][0, :, :, :P] = prompt.to(torch.int32).to(dev)[:, None, :]
+            ws["hist"][0, :, :, :P] = prompt.to(dev)[:, None, :]
             ws["run_score"].fill_(-1.0e9)
             ws["run_score"][:, 0] = 0
             ws["fin_score"].fill_(-1.0e9)
@@ -967,28 +955,9 @@ class WhisperEngine:
                             self._decode_step(R)
                 forced_steps = 0 if prompt_ids is not None else P - 1
                 key = ("beam", R, K, self._ckv_batch, P, bool(timestamps), want_frames)
-                graph = self._graphs.get(key) if self.use_graphs else None
-                if self.use_graphs and graph is None:
-                    # warm-up outside capture, then restore everything the step mutated
-                    keep = {k: ws[k].clone() for k in ("hist", "fin", "run_score", "fin_score", "fin_flag", "fin_len", "gram",
-                                                        "improvable", "hits_all", "ctrl")}
-                    sb, tb, bt = self.state.clone(), self.tokens.clone(), self.block_table.clone()
-                    self._beam_step(R, n, ws)
-                    torch.cuda.current_stream(dev).synchronize()
-
-                    def restore():
-                        for k, v in keep.items():
-                            ws[k].copy_(v)
-                        self.state.copy_(sb)
-                        self.tokens.copy_(tb)
-                        self.block_table.copy_(bt)
-                    restore()
-                    graph = torch.cuda.CUDAGraph()
-                    with _CAPTURE_LOCK:
-                        with torch.cuda.graph(graph, stream=self._capture_stream, capture_error_mode="thread_local"):
-                            self._beam_step(R, n, ws)
-                    restore()
-                    self._graphs[key] = graph
+                # restored after warm-up and capture: the search state (the tw_beam_state buffers) and the rows
+                mutated = [ws[name] for name, _ in _lib.BeamState._fields_] + [self.state, self.tokens, self.block_table]
+                graph = self._graph(key, lambda: self._beam_step(R, n, ws), mutated) if self.use_graphs else None
                 steps, max_steps, poll = 0, L - P, 8
                 while steps < max_steps:
                     if graph is not None:
@@ -1028,9 +997,7 @@ class WhisperEngine:
                 return best
             finally:
                 self._align_on = False
-                self.enc_row.copy_(torch.arange(self.max_batch, dtype=torch.int32, device=dev))
-                self.block_table.copy_(torch.arange(self.max_batch * self.pages_per_row, dtype=torch.int32,
-                                                    device=dev).view(self.max_batch, self.pages_per_row))
+                self._identity_rows()
 
     # ------------------------------------------------------------------------------------ generate
     def generate_from_pcm(self, clips: Sequence[np.ndarray], task: str = "transcribe",
@@ -1148,6 +1115,15 @@ class WhisperEngine:
         langs = [lang_id] * B
         out: List[List[int]] = [[] for _ in range(B)]
         it = 0
+
+        def frames_keep(rows):
+            # weights[..., : (num_frames - seek) // 2] (_postprocess_outputs :1146-1151, :354): python slice rules and,
+            # when every active row has the same value, cropped once more up front (:322-323) — a no-op for
+            # non-negative counts, a second crop from the end for negative ones
+            S = self.dims.max_source_positions
+            left = [int(num_frames[b]) - seek[b] for b in rows]
+            twice = len(set(left)) == 1
+            return [len((range(S)[: v // 2] if twice else range(S))[: v // 2]) for v in left]
         with torch.cuda.device(self.device):
             while any(s < m for s, m in zip(seek, max_frames)):
                 it += 1
@@ -1184,17 +1160,10 @@ class WhisperEngine:
                     prompts = torch.tensor([[gen.decoder_start_token_id, langs[b], gen.task_to_id[task]] for b in rows],
                                            dtype=torch.int32)
                 if num_beams > 1:
-                    keep_b = None
-                    if token_timestamps:
-                        S_ = self.dims.max_source_positions
-                        left_ = [int(num_frames[b]) - seek[b] for b in rows]
-                        twice_ = len(set(left_)) == 1
-                        keep_b = [len((range(S_)[: v // 2] if twice_ else range(S_))[: v // 2]) for v in left_]
                     best = self.decode_beams(n, prompts, num_beams, timestamps=bool(return_timestamps),
-                                             frames_keep=keep_b, prompt_ids=prompt_ids).cpu().tolist()
-                    pre = list(prompt_ids or [])
-                    head = [gen.decoder_start_token_id, 0, gen.task_to_id[task]] + ([] if return_timestamps else [gen.no_timestamps_token_id])
-                    toks = [pre + [head[0], langs[b]] + head[2:] + best[i] for i, b in enumerate(rows)]
+                                             frames_keep=frames_keep(rows) if token_timestamps else None,
+                                             prompt_ids=prompt_ids).cpu().tolist()
+                    toks = [self.prompt_row(prompt_ids, prompts[i], bool(return_timestamps)) + best[i] for i in range(n)]
                 else:
                     self._align_on = bool(token_timestamps)
                     try:
@@ -1207,14 +1176,7 @@ class WhisperEngine:
                 if token_timestamps and num_beams > 1:
                     tok_frames = self.last_beam_frames
                 elif token_timestamps:
-                    # weights[..., : (num_frames - seek) // 2] (_postprocess_outputs :1146-1151, :354): python slice rules
-                    # and, when every active row has the same value, cropped once more up front (:322-323) — a no-op for
-                    # non-negative counts, a second crop from the end for negative ones
-                    S = self.dims.max_source_positions
-                    left = [int(num_frames[b]) - seek[b] for b in rows]
-                    twice = len(set(left)) == 1
-                    keep = [len((range(S)[: v // 2] if twice else range(S))[: v // 2]) for v in left]
-                    tok_frames = self.token_frames(n, toks, P, keep)
+                    tok_frames = self.token_frames(n, toks, P, frames_keep(rows))
                 if trace is not None:
                     trace.setdefault("iterations", []).append({"rows": list(rows), "seek": [seek[b] for b in rows],
                                                                "tokens": [list(t) for t in toks]})
