@@ -92,7 +92,7 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("bench_prompt.py needs a CUDA device")
     import helpers
-    from turbo_whisper_workspace_b200.config import WhisperDims
+    from turbo_whisper_workspace_b200.config import WhisperDims, resolve_generate_options
     from turbo_whisper_workspace_b200.engine import WhisperEngine
     dev = torch.device("cuda:0")
     name, power = gpu_info()
@@ -114,7 +114,7 @@ def main():
             prompts = torch.tensor([[SOT, EN, TRANSCRIBE]] * R, dtype=torch.int32)
             for n in lengths:
                 ids = None if n == 0 else [PREV] + [1000 + (7 * i) % 40000 for i in range(n - 1)]
-                P = eng.prompt_row_len(ids, True)
+                P = resolve_generate_options(dims, eng.gen, prompt_ids=ids).prompt_len
                 # capture of a new prompt length: drop the cached step graphs of this shape first
                 eng._graphs = {k: v for k, v in eng._graphs.items() if not (k[0] == R and k[2] == P)}
                 eng.decode(R, prompts, n_steps=1, prompt_ids=ids)       # warm-up: tables, kernels, prefill weights

@@ -159,14 +159,53 @@ def validate_prompt_ids(prompt_ids, vocab: int) -> List[int]:
     return ids
 
 
-def decoder_prompt_len(prompt_ids, timestamps: bool, max_len: int) -> int:
+def decoder_prompt_len(n_prompt_ids: int, timestamps: bool, max_len: int) -> int:
     """Positions of the decoder input prompt_ids + [<|startoftranscript|>, language, task] (+ <|notimestamps|>)
-    ($TF/models/whisper/generation_whisper.py:1909-1913).  ``max_len`` = min(max_length, max_target_positions): the
-    prompt counts against it, so a long prompt leaves fewer positions to generate.  ValueError unless the input is
-    shorter than ``max_len`` (HF indexes past its positional embedding there)."""
-    n = (3 if timestamps else 4) + (0 if prompt_ids is None else len(prompt_ids))
+    ($TF/models/whisper/generation_whisper.py:1909-1913) for ``n_prompt_ids`` prompt ids.  ``max_len`` =
+    min(max_length, max_target_positions): the prompt counts against it, so a long prompt leaves fewer positions to
+    generate.  ValueError unless the input is shorter than ``max_len`` (HF indexes past its positional embedding there)."""
+    n = (3 if timestamps else 4) + n_prompt_ids
     if n >= max_len:
         raise ValueError(f"The decoder input (prompt_ids and the {3 if timestamps else 4} special start tokens) has "
                          f"{n} positions; it must be shorter than {max_len} (min(max_length, max_target_positions)). "
                          "Shorten the prompt.")
     return n
+
+
+@dataclass(frozen=True)
+class GenerateOptions:
+    """A call's decoding options as the engine uses them (:func:`resolve_generate_options`)."""
+    task_id: int
+    lang_id: int                        # -1: detect the language
+    timestamps: bool
+    num_beams: int
+    token_timestamps: bool
+    prompt_ids: Optional[List[int]]
+    prompt_len: int                     # P: positions of the decoder prompt, special tokens included
+
+
+def resolve_generate_options(dims: WhisperDims, gen: GenerationSettings, *, task: str = "transcribe",
+                             language: Optional[str] = None, return_timestamps: bool = True, num_beams: int = 1,
+                             token_timestamps: bool = False, prompt_ids=None, long_form: bool = False) -> GenerateOptions:
+    """The one check of a generate call's options, before any device work; ValueError for an invalid call.
+    ``task``: a key of ``gen.task_to_id``.  ``language``: ``"en"`` or ``"<|en|>"`` (a key of ``gen.lang_to_id``),
+    None = detect it.  ``return_timestamps``: False = <|notimestamps|> joins the prompt and the timestamp grammar is
+    off.  ``num_beams`` > 1: beam search.  ``token_timestamps``: per-token times from the alignment heads (word
+    timestamps).  ``prompt_ids``: generate(prompt_ids=...), see :func:`validate_prompt_ids`.  ``long_form``: one
+    un-chunked clip longer than 30 s, which needs timestamps and has no token timestamps."""
+    if prompt_ids is not None:
+        prompt_ids = validate_prompt_ids(prompt_ids, dims.vocab)
+    if long_form and (token_timestamps or not return_timestamps):
+        raise ValueError("long-form generate takes one clip, needs timestamps and has no token timestamps")
+    if task not in gen.task_to_id:
+        raise ValueError(f"The `{task}` task is not supported. The task should be one of {list(gen.task_to_id)}")
+    lang_id = -1
+    if language is not None:
+        key = language if language.startswith("<|") else f"<|{language}|>"
+        if key not in gen.lang_to_id:
+            raise ValueError(f"Unsupported language: {language}")
+        lang_id = gen.lang_to_id[key]
+    timestamps = bool(return_timestamps)
+    P = decoder_prompt_len(0 if prompt_ids is None else len(prompt_ids), timestamps,
+                           min(gen.max_length, dims.max_target_positions))
+    return GenerateOptions(gen.task_to_id[task], lang_id, timestamps, int(num_beams), bool(token_timestamps), prompt_ids, P)

@@ -22,7 +22,8 @@ import torch
 
 from . import _lib, ops
 from ._lib import Grammar, SkinnyArgs, check
-from .config import N_FRAMES, N_SAMPLES, GenerationSettings, WhisperDims, decoder_prompt_len, validate_prompt_ids
+from .config import (N_FRAMES, N_SAMPLES, GenerateOptions, GenerationSettings, WhisperDims, decoder_prompt_len,
+                     resolve_generate_options)
 
 MAX_DECODE_BATCH = 96   # decode rows per engine context (projections: up to tw_dec_max_rows(); the LM head runs per 48-row chunk)
 LMHEAD_ROWS = 48
@@ -219,8 +220,10 @@ def init_rows(rows: torch.Tensor, max_len: int, g: Grammar, timestamps: bool, pr
     [R, max_len], state int32 [R, 8] = tw_row_state [R], the grammar's begin_index = P).
     ``prefilled``: positions 0 .. P-2 run as one prefill (:meth:`WhisperEngine.prefill`) and the state is the one the
     forced steps would leave at position P-1; otherwise the steps feed row[0] and teacher-force the rest of the row.
-    ``flat`` (beam search): the grammar is applied by tw_beam_step on the tapped logits, not by the LM head."""
+    ``flat`` (beam search): the grammar is applied by tw_beam_step on the tapped logits, not by the LM head.
+    ValueError unless P < ``max_len`` (the rows must leave a position to generate)."""
     R, P = rows.shape
+    decoder_prompt_len(P - (3 if timestamps else 4), timestamps, max_len)
     rows = rows.to(torch.int32)
     tokens = torch.full((R, max_len), g.pad, dtype=torch.int32)
     forced = torch.full((R, max_len), -1, dtype=torch.int32)
@@ -729,11 +732,6 @@ class WhisperEngine:
             for (kind, a), (_, b) in zip(events[:-1], events[1:]):
                 timing[kind] = timing.get(kind, 0.0) + a.elapsed_time(b)
 
-    def prompt_row_len(self, prompt_ids: Optional[Sequence[int]], timestamps: bool) -> int:
-        """Length of the decoder prompt: prompt_ids + [<|startoftranscript|>, language, task] (+ <|notimestamps|>).
-        ValueError (before any device work) unless it is shorter than min(max_length, max_target_positions)."""
-        return decoder_prompt_len(prompt_ids, timestamps, self.max_len)
-
     def prompt_row(self, prompt_ids: Optional[Sequence[int]], prompt: Sequence[int], timestamps: bool) -> List[int]:
         """The decoder prompt of one row: prompt_ids + ``prompt`` ([<|startoftranscript|>, language, task])
         (+ <|notimestamps|> without timestamps)."""
@@ -775,7 +773,7 @@ class WhisperEngine:
 
     def decode(self, B: int, prompts: Optional[torch.Tensor], n_steps: Optional[int] = None,
                forced: Optional[torch.Tensor] = None, on_step=None, timestamps: bool = True,
-               prompt_ids: Optional[Sequence[int]] = None, prefill_timing: Optional[dict] = None) -> torch.Tensor:
+               prompt_ids: Optional[Sequence[int]] = None) -> torch.Tensor:
         """Greedy decode of B rows against the encoder state left by encode().
 
         prompts: int32 [B, 3] = [<|startoftranscript|>, language, task]; a language of -1 asks for
@@ -785,17 +783,16 @@ class WhisperEngine:
                  the two suppress lists are applied (no WhisperTimeStampLogitsProcessor).
         prompt_ids: text prompt of generate(prompt_ids=...): the rows start with prompt_ids + [SOT, language, task]
                  (+ <|notimestamps|>) = P positions, of which 0 .. P-2 run as one batched prefill (:meth:`prefill`) and
-                 the step loop starts at position P-1; the timestamp grammar begins at P.  The language must be known.
+                 the step loop starts at position P-1; the timestamp grammar begins at P.  The language must be known,
+                 and P must be shorter than max_len.
         Returns the int32 token matrix [B, max_len] on the device (prompt included)."""
         dev = self.device
         max_len = self.max_len
         prefilled = prompt_ids is not None
         with torch.cuda.device(dev):
             pr = prompts.cpu()
-            if prefilled:
-                if bool((pr[:, 1] < 0).any()):
-                    raise ValueError("decode with prompt_ids needs the language of every row (detect it first)")
-                self.prompt_row_len(prompt_ids, timestamps)
+            if prefilled and bool((pr[:, 1] < 0).any()):
+                raise ValueError("decode with prompt_ids needs the language of every row (detect it first)")
             rows = torch.tensor([self.prompt_row(prompt_ids, pr[b, :3], timestamps) for b in range(B)], dtype=torch.int32)
             tok0, frc, st0, self.grammar.begin_index = init_rows(rows, max_len, self.grammar, timestamps, prefilled)
             if forced is not None:      # the caller's teacher forcing wherever the prompt leaves a position free
@@ -807,7 +804,7 @@ class WhisperEngine:
             steps = (max_len - 1) if n_steps is None else min(n_steps, max_len - 1)
             if prefilled:
                 P = rows.shape[1]
-                self.prefill(B, P, timing=prefill_timing)
+                self.prefill(B, P)
                 steps = min(steps, max_len - P)
             _lib.load().tw_set_pdl(0 if (self.use_graphs or os.environ.get("TWB200_NO_PDL")) else 1)   # PDL only pays off for eager stepping
             graph = self._graph_for(B) if self.use_graphs else None
@@ -909,8 +906,6 @@ class WhisperEngine:
         self._enable_beam_pool()
         want_frames = frames_keep is not None
         with torch.cuda.device(dev):
-            if prompt_ids is not None:
-                self.prompt_row_len(prompt_ids, timestamps)
             prompt = torch.tensor([self.prompt_row(prompt_ids, pr, timestamps) for pr in prompts.cpu()], dtype=torch.int32)
             tok0, frc, st0, P = init_rows(prompt.repeat_interleave(K, dim=0), self.max_len, self.grammar, timestamps,
                                           prefilled=prompt_ids is not None, flat=True)
@@ -1000,55 +995,45 @@ class WhisperEngine:
                 self._identity_rows()
 
     # ------------------------------------------------------------------------------------ generate
-    def generate_from_pcm(self, clips: Sequence[np.ndarray], task: str = "transcribe",
-                          language: Optional[str] = None, return_timestamps: bool = True, num_beams: int = 1,
-                          token_timestamps: bool = False, prompt_ids: Optional[Sequence[int]] = None):
+    def generate_from_pcm(self, clips: Sequence[np.ndarray], **options):
         """PCM windows (<= 30 s each) -> generated token ids per window (segments concatenated), the
         output contract of ``WhisperGenerationMixin.generate(..., return_timestamps=True)`` minus padding.
-        ``token_timestamps``: every window becomes ``(ids, times)`` with one fp32 time per id — the per-segment
-        `token_timestamps` of generate(return_token_timestamps=True, return_segments=True), which the ASR pipeline
-        reads for return_timestamps="word".
-        ``prompt_ids``: generate(prompt_ids=...) (see :meth:`generate`); validated before any device work."""
-        if prompt_ids is not None:
-            prompt_ids = validate_prompt_ids(prompt_ids, self.dims.vocab)
-            self.prompt_row_len(prompt_ids, bool(return_timestamps))
+        ``options``: the generate options (task, language, return_timestamps, num_beams, token_timestamps, prompt_ids;
+        see :meth:`generate`), checked before any device work.  With ``token_timestamps`` every window becomes
+        ``(ids, times)`` with one fp32 time per id — the per-segment `token_timestamps` of
+        generate(return_token_timestamps=True, return_segments=True), which the ASR pipeline reads for
+        return_timestamps="word"."""
+        opts = resolve_generate_options(self.dims, self.gen, **options)
 
         def run():
             B = self.load_pcm(clips)
             self.features(B)
-            if not token_timestamps:
-                return self.generate(B, task=task, language=language, return_timestamps=return_timestamps,
-                                     num_beams=num_beams, prompt_ids=prompt_ids)
+            if not opts.token_timestamps:
+                return self._seek(B, opts)
             # attention_mask.sum(-1) of the feature extractor: the sample mask taken every hop (160) samples
             nf = [min(N_FRAMES, -(-min(len(np.asarray(c).reshape(-1)), N_SAMPLES) // 160)) for c in clips]
-            rows = self.generate(B, task=task, language=language, return_timestamps=return_timestamps,
-                                 num_beams=num_beams, token_timestamps=True, num_frames=nf, prompt_ids=prompt_ids)
-            return list(zip(rows, self.last_token_ts))
+            return list(zip(self._seek(B, opts, num_frames=nf), self.last_token_ts))
         if self.stream is not None:
             with torch.cuda.stream(self.stream):
                 return run()
         return run()
 
-    def generate_long_from_pcm(self, audio: np.ndarray, task: str = "transcribe", language: Optional[str] = None,
-                               num_beams: int = 1, trace: Optional[dict] = None,
-                               prompt_ids: Optional[Sequence[int]] = None) -> List[int]:
+    def generate_long_from_pcm(self, audio: np.ndarray, trace: Optional[dict] = None, **options) -> List[int]:
         """ONE clip longer than 30 s, un-chunked (the ASR pipeline without chunk_length_s,
         $TF/pipelines/automatic_speech_recognition.py:446-454): features of the whole clip (tw_logmel_long) and HF's
         long-form generate — the same seek loop as :meth:`generate`, over all n // 160 frames
         ($TF/models/whisper/generation_whisper.py:654-658, :785-870); timestamps are mandatory (:1388-1394).  Sequential
         by construction: one window is encoded and decoded per iteration.  Returns the generated ids (segments
         concatenated; timestamp tokens restart in every 30 s segment, which `_decode_asr` undoes).
-        ``prompt_ids``: prepended in every seek iteration (HF with condition_on_prev_tokens off)."""
-        if prompt_ids is not None:
-            prompt_ids = validate_prompt_ids(prompt_ids, self.dims.vocab)
-            self.prompt_row_len(prompt_ids, True)
+        ``options``: the generate options (see :meth:`generate`), checked before any device work; ``prompt_ids`` is
+        prepended in every seek iteration (HF with condition_on_prev_tokens off)."""
+        opts = resolve_generate_options(self.dims, self.gen, long_form=True, **options)
 
         def run():
             mel = self.logmel.long(audio)
             self.stats["launches"] += 2
             self.stats["h2d_bytes"] += int(np.asarray(audio).size) * 4
-            return self.generate(1, task=task, language=language, num_beams=num_beams, long_mel=mel, trace=trace,
-                                 prompt_ids=prompt_ids)[0]
+            return self._seek(1, opts, trace=trace, long_mel=mel)[0]
         if self.stream is not None:
             with torch.cuda.stream(self.stream):
                 return run()
@@ -1068,51 +1053,46 @@ class WhisperEngine:
             s = s[:-1]
         return s
 
-    def generate(self, B: int, task: str = "transcribe", language: Optional[str] = None,
-                 trace: Optional[dict] = None, return_timestamps: bool = True, num_beams: int = 1,
-                 token_timestamps: bool = False, num_frames: Optional[Sequence[int]] = None,
-                 long_mel: Optional[torch.Tensor] = None, prompt_ids: Optional[Sequence[int]] = None,
-                 prefill_timing: Optional[dict] = None) -> List[List[int]]:
-        """Short-form seek loop over the features in self.mel_t[:B] (greedy; timestamp grammar on unless
-        ``return_timestamps`` is False, in which case <|notimestamps|> joins the prompt).
+    def generate(self, B: int, trace: Optional[dict] = None, num_frames: Optional[Sequence[int]] = None,
+                 long_mel: Optional[torch.Tensor] = None, **options) -> List[List[int]]:
+        """Short-form seek loop over the features in self.mel_t[:B].  ``options`` are the generate options of
+        :func:`config.resolve_generate_options`, checked before any device work:
 
-        ``token_timestamps`` (greedy only; ``num_frames[b]`` = valid mel frames of row b, the attention-mask sum):
-        the decode steps also tap the alignment heads' cross-attention, and ``self.last_token_ts[b]`` receives one
-        fp32 time per returned id (seek offset added, as `segments[...]["token_timestamps"]` of HF's generate;
-        ``self.last_token_ts_raw[b]`` = the padded `token_timestamps` output, no offset).
+        ``task``, ``language`` (None: detected per row), ``num_beams`` (1: greedy, else beam search) and
+        ``return_timestamps`` (timestamp grammar on unless False, in which case <|notimestamps|> joins the prompt).
 
-        ``long_mel`` (bf16 [T, n_mels], T > 3000, B == 1): HF's long-form mode — the loop runs over T frames and every
-        iteration's window is gathered from ``long_mel`` (zero-padded to 3000 frames, _get_input_segment :1831-1850).
+        ``token_timestamps`` (``num_frames[b]`` = valid mel frames of row b, the attention-mask sum): the decode steps
+        also tap the alignment heads' cross-attention, and ``self.last_token_ts[b]`` receives one fp32 time per returned
+        id (seek offset added, as `segments[...]["token_timestamps"]` of HF's generate; ``self.last_token_ts_raw[b]`` =
+        the padded `token_timestamps` output, no offset).
 
         ``prompt_ids`` (generate(prompt_ids=...), $TF/models/whisper/generation_whisper.py:1909-1913): every seek
         iteration's decoder input is prompt_ids + [SOT, language, task] (+ <|notimestamps|>), run as one batched prefill
         after encode(); the returned ids exclude it.  An unknown language is detected first on [SOT] alone (one decode
-        position), as detect_language does before the prompt is built.  ``prefill_timing``: per-phase prefill times."""
+        position), as detect_language does before the prompt is built.
+
+        ``long_mel`` (bf16 [T, n_mels], T > 3000, B == 1): HF's long-form mode — the loop runs over T frames and every
+        iteration's window is gathered from ``long_mel`` (zero-padded to 3000 frames, _get_input_segment :1831-1850)."""
+        if long_mel is not None and B != 1:
+            raise ValueError("long-form generate takes one clip, needs timestamps and has no token timestamps")
+        opts = resolve_generate_options(self.dims, self.gen, long_form=long_mel is not None, **options)
+        return self._seek(B, opts, trace=trace, num_frames=num_frames, long_mel=long_mel)
+
+    def _seek(self, B: int, opts: GenerateOptions, trace: Optional[dict] = None,
+              num_frames: Optional[Sequence[int]] = None, long_mel: Optional[torch.Tensor] = None) -> List[List[int]]:
+        """The seek loop of :meth:`generate` with the options already resolved."""
         gen = self.gen
-        if prompt_ids is not None:
-            prompt_ids = validate_prompt_ids(prompt_ids, self.dims.vocab)
-        if long_mel is not None:
-            if B != 1 or token_timestamps or not return_timestamps:
-                raise ValueError("long-form generate takes one clip, needs timestamps and has no token timestamps")
-        if token_timestamps:
+        timestamps, num_beams, prompt_ids, P = opts.timestamps, opts.num_beams, opts.prompt_ids, opts.prompt_len
+        if opts.token_timestamps:
             if num_frames is None or len(num_frames) != B:
                 raise ValueError("token_timestamps needs num_frames for every row")
             self.enable_alignment()
         ts_out: List[List[float]] = [[] for _ in range(B)]
         ts_raw: List[List[float]] = [[] for _ in range(B)]
-        if task not in gen.task_to_id:
-            raise ValueError(f"The `{task}` task is not supported. The task should be one of {list(gen.task_to_id)}")
-        lang_id = -1
-        if language is not None:
-            key = language if language.startswith("<|") else f"<|{language}|>"
-            if key not in gen.lang_to_id:
-                raise ValueError(f"Unsupported language: {language}")
-            lang_id = gen.lang_to_id[key]
         ts_begin = gen.timestamp_begin
-        P = self.prompt_row_len(prompt_ids, bool(return_timestamps))
         seek = [0] * B
         max_frames = [N_FRAMES] * B if long_mel is None else [int(long_mel.shape[0])]
-        langs = [lang_id] * B
+        langs = [opts.lang_id] * B
         out: List[List[int]] = [[] for _ in range(B)]
         it = 0
 
@@ -1149,33 +1129,32 @@ class WhisperEngine:
                     self.stats["launches"] += 1
                     mel = self.mel_s
                 self.encode(n, mel)
-                prompts = torch.tensor([[gen.decoder_start_token_id, langs[b], gen.task_to_id[task]] for b in rows],
+                prompts = torch.tensor([[gen.decoder_start_token_id, langs[b], opts.task_id] for b in rows],
                                        dtype=torch.int32)
                 if (num_beams > 1 or prompt_ids is not None) and any(langs[b] < 0 for b in rows):
                     # language detection first (one decoder position), as detect_language does before generate
-                    first = self.decode(n, prompts, n_steps=1, timestamps=bool(return_timestamps))[:, 1].cpu().tolist()
+                    first = self.decode(n, prompts, n_steps=1, timestamps=timestamps)[:, 1].cpu().tolist()
                     for i, b in enumerate(rows):
                         if langs[b] < 0:
                             langs[b] = int(first[i])
-                    prompts = torch.tensor([[gen.decoder_start_token_id, langs[b], gen.task_to_id[task]] for b in rows],
+                    prompts = torch.tensor([[gen.decoder_start_token_id, langs[b], opts.task_id] for b in rows],
                                            dtype=torch.int32)
                 if num_beams > 1:
-                    best = self.decode_beams(n, prompts, num_beams, timestamps=bool(return_timestamps),
-                                             frames_keep=frames_keep(rows) if token_timestamps else None,
+                    best = self.decode_beams(n, prompts, num_beams, timestamps=timestamps,
+                                             frames_keep=frames_keep(rows) if opts.token_timestamps else None,
                                              prompt_ids=prompt_ids).cpu().tolist()
-                    toks = [self.prompt_row(prompt_ids, prompts[i], bool(return_timestamps)) + best[i] for i in range(n)]
+                    toks = [self.prompt_row(prompt_ids, prompts[i], timestamps) + best[i] for i in range(n)]
                 else:
-                    self._align_on = bool(token_timestamps)
+                    self._align_on = opts.token_timestamps
                     try:
-                        toks = self.decode(n, prompts, timestamps=bool(return_timestamps), prompt_ids=prompt_ids,
-                                           prefill_timing=prefill_timing).cpu().tolist()
+                        toks = self.decode(n, prompts, timestamps=timestamps, prompt_ids=prompt_ids).cpu().tolist()
                     finally:
                         self._align_on = False
                 self.stats["d2h_bytes"] += n * self.max_len * 4
                 tok_frames = None
-                if token_timestamps and num_beams > 1:
+                if opts.token_timestamps and num_beams > 1:
                     tok_frames = self.last_beam_frames
-                elif token_timestamps:
+                elif opts.token_timestamps:
                     tok_frames = self.token_frames(n, toks, P, frames_keep(rows))
                 if trace is not None:
                     trace.setdefault("iterations", []).append({"rows": list(rows), "seek": [seek[b] for b in rows],

@@ -26,7 +26,7 @@ from typing import Any, Dict, List, Optional, Sequence, Tuple, Union
 
 import numpy as np
 
-from .config import N_SAMPLES, SAMPLING_RATE, GenerationSettings, WhisperDims, decoder_prompt_len, validate_prompt_ids
+from .config import N_SAMPLES, SAMPLING_RATE, GenerationSettings, WhisperDims, resolve_generate_options
 
 
 # ------------------------------------------------------------------------------------------------
@@ -254,8 +254,10 @@ class B200WhisperPipeline:
     def __init__(self, state_dict, dims: WhisperDims, tokenizer, generation: Optional[GenerationSettings] = None,
                  devices: Sequence[Union[str, int]] = ("cuda:0",), max_batch: int = 24, time_precision: float = 0.02,
                  scheduler=None, contexts_per_device: int = 4):
-        """``scheduler``: any object with ``run(clips, task=, language=) -> token rows`` and ``last_stats``;
-        defaults to a :class:`WindowScheduler` with one GPU engine per entry of ``devices``."""
+        """``scheduler``: any object with ``run(clips, task=, language=) -> token rows`` and ``last_stats``; every other
+        generate option reaches ``run`` (and ``run_long``) as a keyword only when it differs from its default, which a
+        scheduler forwards to its engines untouched.  Defaults to a :class:`WindowScheduler` with one GPU engine per
+        entry of ``devices``."""
         self.dims = dims
         self.tokenizer = tokenizer
         self.generation = generation or GenerationSettings()
@@ -307,7 +309,25 @@ class B200WhisperPipeline:
         task = generate_kwargs.pop("task", None) or "transcribe"
         language = generate_kwargs.pop("language", None)
         num_beams = int(generate_kwargs.pop("num_beams", None) or self.num_beams or 1)
-        prompt_ids = self._prompt(generate_kwargs, return_timestamps)
+        prompt_ids = self._prompt(generate_kwargs)
+        # return_timestamps falsy (the HF default): <|notimestamps|> joins the prompt, no timestamp grammar, and the windows
+        # are merged on their overlapping text only.  "word": the engine also taps the alignment heads' cross-attention
+        opts = resolve_generate_options(self.dims, self.generation, task=task, language=language,
+                                        return_timestamps=bool(return_timestamps), num_beams=num_beams,
+                                        token_timestamps=return_timestamps == "word", prompt_ids=prompt_ids)
+        bs = max(1, int(batch_size or 1))
+        # the options reach the scheduler (and its engines) as keywords, each only when it differs from its default
+        run_kw: Dict[str, Any] = {"task": task, "language": language}
+        if not opts.timestamps:
+            run_kw["return_timestamps"] = False
+        if opts.num_beams > 1:
+            run_kw["num_beams"] = opts.num_beams      # beam search: every window occupies num_beams decode rows
+        if opts.token_timestamps:
+            # micro-batches follow HF's batches of `batch_size` consecutive windows (capped by the engine's max_batch)
+            # because a row's DTW spans the decode steps of its batch's longest row
+            run_kw.update(token_timestamps=True, group=bs)
+        if opts.prompt_ids is not None:
+            run_kw["prompt_ids"] = opts.prompt_ids
         if return_timestamps == "char":
             raise ValueError("Whisper cannot return `char` timestamps, only word level or segment level timestamps. "
                              "Use `return_timestamps='word'` or `return_timestamps=True` respectively.")
@@ -317,23 +337,7 @@ class B200WhisperPipeline:
         prepared = [self._prepare(x, chunk_length_s, stride_length_s) for x in items]
         t1 = time.perf_counter()
         clips = [c for p in prepared for c in p["clips"]]
-        # return_timestamps falsy (the HF default): generate runs with <|notimestamps|> in the prompt and without the
-        # timestamp grammar, and the windows are merged on their overlapping text only
-        run_kw: Dict[str, Any] = {}
-        if not return_timestamps:
-            run_kw["return_timestamps"] = False
-        if num_beams > 1:
-            run_kw["num_beams"] = num_beams      # beam search: every window occupies num_beams decode rows
-        long_kw: Dict[str, Any] = {}
-        if prompt_ids is not None:
-            run_kw["prompt_ids"] = long_kw["prompt_ids"] = prompt_ids
-        bs = max(1, int(batch_size or 1))
         token_times = None
-        if return_timestamps == "word":
-            # generate(return_token_timestamps=True, return_segments=True): the engine taps the alignment heads'
-            # cross-attention; micro-batches follow HF's batches of `batch_size` consecutive windows (capped by the
-            # engine's max_batch) because a row's DTW spans the decode steps of its batch's longest row
-            run_kw.update(token_timestamps=True, group=bs)
         if any("longform" in p for p in prepared):
             if not return_timestamps:
                 raise ValueError(
@@ -343,12 +347,13 @@ class B200WhisperPipeline:
             if return_timestamps == "word":
                 raise NotImplementedError("word timestamps for un-chunked long-form input are not implemented; pass "
                                           "chunk_length_s as the reference does")
-        token_rows = self.scheduler.run(clips, task=task, language=language, **run_kw) if clips else []
+        token_rows = self.scheduler.run(clips, **run_kw) if clips else []
         if return_timestamps == "word":
             token_times = [np.asarray(t, dtype=np.float32) for _, t in token_rows]
             token_rows = [r for r, _ in token_rows]
-        long_rows = {i: self.scheduler.run_long(p["longform"], task=task, language=language, num_beams=num_beams, **long_kw)
-                     for i, p in enumerate(prepared) if "longform" in p}
+        # long-form input is only reached with timestamps on and without word timestamps, so run_kw holds nothing that
+        # long-form generate refuses
+        long_rows = {i: self.scheduler.run_long(p["longform"], **run_kw) for i, p in enumerate(prepared) if "longform" in p}
         t2 = time.perf_counter()
         self.last_token_rows = token_rows      # the engines' rows of this call, window order (bench.py's output check)
         results, w0 = [], 0
@@ -366,12 +371,12 @@ class B200WhisperPipeline:
                                host_seconds={"prepare": t1 - t0, "engines": t2 - t1, "finish": time.perf_counter() - t2})
         return results if many else results[0]
 
-    def _prompt(self, generate_kwargs: dict, return_timestamps) -> Optional[List[int]]:
-        """Pops ``prompt_ids`` (list, numpy or torch; normally ``processor.get_prompt_ids(text)``) and
-        ``prompt_condition_type`` from generate_kwargs and validates them as WhisperGenerationMixin.generate does
-        ($TF/models/whisper/generation_whisper.py:1731-1748).  Every window's decoder input then starts with
-        prompt_ids; the returned ids, and so the text, exclude it.  ``"all-segments"`` needs condition_on_prev_tokens,
-        which is not implemented."""
+    def _prompt(self, generate_kwargs: dict):
+        """Pops ``prompt_ids`` (list, numpy or torch; normally ``processor.get_prompt_ids(text)``; validated by
+        resolve_generate_options) and ``prompt_condition_type`` from generate_kwargs and validates the latter as
+        WhisperGenerationMixin.generate does ($TF/models/whisper/generation_whisper.py:1731-1748).  Every window's
+        decoder input then starts with prompt_ids; the returned ids, and so the text, exclude it.  ``"all-segments"``
+        needs condition_on_prev_tokens, which is not implemented."""
         prompt_ids = generate_kwargs.pop("prompt_ids", None)
         cond = generate_kwargs.pop("prompt_condition_type", None) or "first-segment"
         allowed = ["first-segment", "all-segments"]
@@ -384,12 +389,7 @@ class B200WhisperPipeline:
                                  "`prompt_condition_type='all-segments'`.")
             raise NotImplementedError("prompt_condition_type='all-segments' needs condition_on_prev_tokens, which the "
                                       "engine does not implement")
-        if prompt_ids is None:
-            return None
-        ids = validate_prompt_ids(prompt_ids, self.dims.vocab)
-        max_len = min(self.generation.max_length, self.dims.max_target_positions)
-        decoder_prompt_len(ids, bool(return_timestamps), max_len)
-        return ids
+        return prompt_ids
 
     def _prepare(self, inputs, chunk_length_s, stride_length_s) -> Dict[str, Any]:
         """preprocess ($TF/pipelines/automatic_speech_recognition.py:341-477) of one input: PCM, windows, clips."""

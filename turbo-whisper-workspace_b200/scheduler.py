@@ -34,22 +34,6 @@ def partition(n_items: int, n_workers: int) -> List[Tuple[int, int]]:
     return out
 
 
-def _extra(return_timestamps: bool, num_beams: int, token_timestamps: bool = False,
-           prompt_ids: Optional[Sequence[int]] = None) -> Dict[str, Any]:
-    """Keyword arguments beyond (task, language), passed only when they differ from the defaults so that simple
-    engine stand-ins keep working."""
-    kw: Dict[str, Any] = {}
-    if prompt_ids is not None:
-        kw["prompt_ids"] = list(prompt_ids)
-    if not return_timestamps:
-        kw["return_timestamps"] = False
-    if num_beams > 1:
-        kw["num_beams"] = int(num_beams)
-    if token_timestamps:
-        kw["token_timestamps"] = True
-    return kw
-
-
 def microbatch_size(max_batch: int, num_beams: int = 1, group: Optional[int] = None) -> int:
     """Windows per engine call: every window occupies num_beams decode rows; ``group`` (word timestamps) caps it at
     the HF pipeline's batch_size so that a micro-batch is exactly one of HF's generate batches."""
@@ -64,14 +48,12 @@ def group_ranges(n_items: int, n_workers: int, mb: int) -> List[Tuple[int, int]]
     return [(min(n_items, a * mb), min(n_items, b * mb)) for a, b in partition(n_groups, n_workers)]
 
 
-def run_in_microbatches(engine, clips: Sequence[np.ndarray], task: str, language: Optional[str],
-                        return_timestamps: bool = True, num_beams: int = 1, token_timestamps: bool = False,
-                        group: Optional[int] = None, prompt_ids: Optional[Sequence[int]] = None) -> List[Any]:
+def run_in_microbatches(engine, clips: Sequence[np.ndarray], group: Optional[int] = None, **generate_kwargs) -> List[Any]:
+    """``engine.generate_from_pcm(clips[i:i + mb], **generate_kwargs)`` over micro-batches of :func:`microbatch_size`."""
     rows: List[Any] = []
-    mb = microbatch_size(engine.max_batch, num_beams, group)
+    mb = microbatch_size(engine.max_batch, generate_kwargs.get("num_beams", 1), group)
     for i in range(0, len(clips), mb):
-        rows.extend(engine.generate_from_pcm(clips[i:i + mb], task=task, language=language,
-                                             **_extra(return_timestamps, num_beams, token_timestamps, prompt_ids)))
+        rows.extend(engine.generate_from_pcm(clips[i:i + mb], **generate_kwargs))
     return rows
 
 
@@ -148,12 +130,12 @@ class WindowScheduler:
     def max_batch(self) -> int:
         return self.engines[0][0].max_batch
 
-    def run(self, clips: Sequence[np.ndarray], task: str = "transcribe", language: Optional[str] = None,
-            return_timestamps: bool = True, num_beams: int = 1, token_timestamps: bool = False,
-            group: Optional[int] = None, prompt_ids: Optional[Sequence[int]] = None) -> List[Any]:
-        """Token rows per window, in order.  ``prompt_ids``: the text prompt of every window (generate(prompt_ids=...)).  ``token_timestamps``: every row is ``(ids, times)`` (word timestamps);
-        ``group`` = the HF pipeline's batch_size: micro-batches then are HF's generate batches (the per-token times of
-        a row depend on the longest row of its batch, $TF/models/whisper/generation_whisper.py:241-381)."""
+    def run(self, clips: Sequence[np.ndarray], group: Optional[int] = None, **generate_kwargs) -> List[Any]:
+        """Token rows per window, in order.  ``generate_kwargs``: the generate options of every window, forwarded to
+        ``engine.generate_from_pcm`` untouched; ``num_beams`` (default 1) sizes the micro-batches.  ``group`` = the HF
+        pipeline's batch_size (word timestamps, where every row is ``(ids, times)``): micro-batches then are HF's
+        generate batches (the per-token times of a row depend on the longest row of its batch,
+        $TF/models/whisper/generation_whisper.py:241-381)."""
         t0 = time.perf_counter()
         n = len(clips)
         engines = self.flat_engines
@@ -164,12 +146,12 @@ class WindowScheduler:
         cap = min(e.max_batch for e in engines)
         # word timestamps: exactly the HF pipeline's batches; otherwise as few, equally sized micro-batches as keep
         # every context busy
+        num_beams = generate_kwargs.get("num_beams", 1)
         mb = microbatch_size(cap, num_beams, group) if group else \
             balanced_microbatch(n, len(engines), microbatch_size(cap, num_beams), min(MIN_MICROBATCH, max(1, cap // max(1, num_beams))))
         queue = WorkQueue(n, mb)
         results: List[Optional[List[int]]] = [None] * n
         errors: List[BaseException] = []
-        extra = _extra(return_timestamps, num_beams, token_timestamps, prompt_ids)
 
         def work(engine):
             try:
@@ -178,7 +160,7 @@ class WindowScheduler:
                     if item is None:
                         return
                     a, b = item
-                    results[a:b] = engine.generate_from_pcm(clips[a:b], task=task, language=language, **extra)
+                    results[a:b] = engine.generate_from_pcm(clips[a:b], **generate_kwargs)
             except BaseException as ex:  # surfaced on the calling thread
                 errors.append(ex)
 
@@ -200,12 +182,10 @@ class WindowScheduler:
                            "microbatches": list(queue.handed), "seconds": time.perf_counter() - t0}
         return [r for r in results]
 
-    def run_long(self, audio: np.ndarray, task: str = "transcribe", language: Optional[str] = None,
-                 num_beams: int = 1, prompt_ids: Optional[Sequence[int]] = None) -> List[int]:
+    def run_long(self, audio: np.ndarray, **generate_kwargs) -> List[int]:
         """Token row of ONE un-chunked long-form clip (> 30 s): HF's long-form generate is a sequential seek loop over the
-        clip's frames, so it runs on one engine context."""
-        kw = {} if prompt_ids is None else {"prompt_ids": list(prompt_ids)}
-        return self.engines[0][0].generate_long_from_pcm(audio, task=task, language=language, num_beams=num_beams, **kw)
+        clip's frames, so it runs on one engine context (``engine.generate_long_from_pcm(audio, **generate_kwargs)``)."""
+        return self.engines[0][0].generate_long_from_pcm(audio, **generate_kwargs)
 
     def close(self):
         self.engines = []
@@ -232,19 +212,18 @@ class DistributedWindowScheduler:
     def local_range(self, n: int, mb: Optional[int] = None) -> Tuple[int, int]:
         return (group_ranges(n, self.world_size, mb) if mb else partition(n, self.world_size))[self.rank]
 
-    def run_local(self, clips: Sequence[np.ndarray], task: str = "transcribe", language: Optional[str] = None,
-                  return_timestamps: bool = True, num_beams: int = 1, token_timestamps: bool = False,
-                  group: Optional[int] = None, prompt_ids: Optional[Sequence[int]] = None) -> List[Any]:
-        mb = microbatch_size(self.engine.max_batch, num_beams, group) if group else None
-        s, e = self.local_range(len(clips), mb)
+    def _group_mb(self, group: Optional[int], generate_kwargs: Dict[str, Any]) -> Optional[int]:
+        """Micro-batch size of word-timestamp jobs (:func:`group_ranges`); None otherwise."""
+        return microbatch_size(self.engine.max_batch, generate_kwargs.get("num_beams", 1), group) if group else None
+
+    def run_local(self, clips: Sequence[np.ndarray], group: Optional[int] = None, **generate_kwargs) -> List[Any]:
+        """Token rows of this rank's range of ``clips``; ``generate_kwargs`` are forwarded untouched."""
+        s, e = self.local_range(len(clips), self._group_mb(group, generate_kwargs))
         if e <= s:
             return []
         if hasattr(self.engine, "run"):          # a local WindowScheduler (engine contexts of this rank's GPU)
-            kw = {} if prompt_ids is None else {"prompt_ids": prompt_ids}
-            return self.engine.run(clips[s:e], task=task, language=language, return_timestamps=return_timestamps,
-                                   num_beams=num_beams, token_timestamps=token_timestamps, group=group, **kw)
-        return run_in_microbatches(self.engine, clips[s:e], task, language, return_timestamps, num_beams,
-                                   token_timestamps, group, prompt_ids)
+            return self.engine.run(clips[s:e], group=group, **generate_kwargs)
+        return run_in_microbatches(self.engine, clips[s:e], group, **generate_kwargs)
 
     def gather(self, local_rows: List[List[int]]) -> List[List[int]]:
         if self.world_size == 1:
@@ -257,24 +236,19 @@ class DistributedWindowScheduler:
             rows.extend(b)
         return rows
 
-    def run(self, clips: Sequence[np.ndarray], task: str = "transcribe", language: Optional[str] = None,
-            return_timestamps: bool = True, num_beams: int = 1, token_timestamps: bool = False,
-            group: Optional[int] = None, prompt_ids: Optional[Sequence[int]] = None) -> List[Any]:
+    def run(self, clips: Sequence[np.ndarray], group: Optional[int] = None, **generate_kwargs) -> List[Any]:
         t0 = time.perf_counter()
-        s, e = self.local_range(len(clips), microbatch_size(self.engine.max_batch, num_beams, group) if group else None)
-        rows = self.gather(self.run_local(clips, task, language, return_timestamps, num_beams, token_timestamps, group,
-                                          prompt_ids))
+        s, e = self.local_range(len(clips), self._group_mb(group, generate_kwargs))
+        rows = self.gather(self.run_local(clips, group, **generate_kwargs))
         self.last_stats = {"workers": self.world_size, "rank": self.rank, "local_range": (s, e),
                            "seconds": time.perf_counter() - t0}
         return rows
 
-    def run_long(self, audio: np.ndarray, task: str = "transcribe", language: Optional[str] = None,
-                 num_beams: int = 1, prompt_ids: Optional[Sequence[int]] = None) -> List[int]:
+    def run_long(self, audio: np.ndarray, **generate_kwargs) -> List[int]:
         """Un-chunked long-form input does not shard (one sequential seek loop): every rank computes the same row."""
-        kw = {} if prompt_ids is None else {"prompt_ids": list(prompt_ids)}
         if hasattr(self.engine, "run_long"):
-            return self.engine.run_long(audio, task=task, language=language, num_beams=num_beams, **kw)
-        return self.engine.generate_long_from_pcm(audio, task=task, language=language, num_beams=num_beams, **kw)
+            return self.engine.run_long(audio, **generate_kwargs)
+        return self.engine.generate_long_from_pcm(audio, **generate_kwargs)
 
     def close(self):
         if hasattr(self.engine, "close"):
