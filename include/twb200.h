@@ -76,6 +76,16 @@ int tw_logmel_n(const void* tables_dev, const float* pcm, int64_t pcm_stride, co
 int tw_logmel_long_n(const void* tables_dev, const float* pcm_long, int64_t hop_samples, int32_t n_windows,
                      const int32_t* frame_lo, const int32_t* frame_hi, const int32_t* out_row0, uint32_t* max_scratch,
                      void* out_bf16_t, int64_t total_frames, int32_t out_t_row_off, int32_t n_mels, void* stream);
+/* Whole-clip features of SEVERAL clips in one launch (plus one floor launch): the clips' buffers (each laid out as for
+ * tw_logmel_long) are concatenated in pcm; window b reads pcm + win_offset[b] (samples), belongs to clip win_clip[b] and
+ * writes its frames [frame_lo[b], frame_hi[b]) to rows out_row0[b].. of out_bf16_t (time-major [total_frames, n_mels]).
+ * Clip c owns rows [clip_row0[c], clip_row0[c + 1]) and gets its own max - 8 clamp (max_scratch: n_clips device
+ * uint32).  win_offset, clip_row0 (n_clips + 1 entries): device int64; the other arrays device int32.  A clip computed
+ * alone or together with others gives the same bits. */
+int tw_logmel_long_multi(const void* tables_dev, const float* pcm, const int64_t* win_offset, const int32_t* win_clip,
+                         int32_t n_windows, const int32_t* frame_lo, const int32_t* frame_hi, const int32_t* out_row0,
+                         int32_t n_clips, const int64_t* clip_row0, uint32_t* max_scratch, void* out_bf16_t,
+                         int64_t total_frames, int32_t n_mels, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * K4  LayerNorm over the last dimension, fp32 in -> bf16 out (eps as nn.LayerNorm, 1e-5).
@@ -139,6 +149,13 @@ int tw_attention_enc_set_trace(void* dev_buf_int64_x192);
 int tw_shift_frames(const void* src_bf16, void* dst_bf16, const int32_t* src_row, const int32_t* seek,
                     int32_t batch, int32_t frames, int32_t cols, int64_t batch_stride, int32_t row_off,
                     void* stream);
+/* The same gather for the long-form seek loop, every row from the whole-clip features of its own clip:
+ * dst[b, dst_row_off + t, :] = src_rows[b][seek[b] + t, :] for t < min(window, frames[b] - seek[b]), zeros up to window.
+ * src_rows: device array of batch pointers, each to 16-byte aligned time-major bf16 features [frames[b], cols];
+ * frames, seek: device int32 [batch]; dst: bf16, row b at dst_bf16 + b * dst_batch_stride (elements).  One launch. */
+int tw_gather_frames(const void* const* src_rows, const int32_t* frames, const int32_t* seek, int32_t batch,
+                     int32_t window, int32_t cols, void* dst_bf16, int64_t dst_batch_stride, int32_t dst_row_off,
+                     void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * K7 / K8  batched greedy decode step (<= 32 rows per call).  All per-row state lives on the

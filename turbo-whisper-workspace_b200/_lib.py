@@ -97,6 +97,10 @@ SIGNATURES = {
     "tw_attention_enc_set_trace": (C.c_int, [c_void_p]),
     "tw_shift_frames": (C.c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int64,
                                   c_int32, c_void_p]),
+    "tw_logmel_long_multi": (C.c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_void_p,
+                                       c_int32, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_void_p]),
+    "tw_gather_frames": (C.c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_void_p, c_int64, c_int32,
+                                   c_void_p]),
     "tw_resample": (C.c_int, [c_void_p, c_int32, c_int32, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_int32, c_int32,
                               c_int32, c_void_p]),
     "tw_prefill_embed": (C.c_int, [c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_int32, c_void_p]),

@@ -387,9 +387,13 @@ __global__ void __launch_bounds__(NT) logmel_kernel(const float* __restrict__ pc
 // OVERLAPPING 30 s windows that start `hop_samples` apart: a frame only depends on 400 samples, so every frame of a
 // window that does not touch the window's own reflect padding equals the clip's frame; window b contributes its frames
 // [frame_lo[b], frame_hi[b]) to rows out_row0[b].. of the clip's time-major output.  The clamp uses the maximum of the
-// WHOLE clip: this kernel stores un-floored values and raises ONE maximum, logmel_floor_kernel applies the floor.
+// WHOLE clip: this kernel stores un-floored values and raises the clip's maximum, logmel_floor_kernel applies the floor.
+// Several clips in one launch: window b reads pcm + win_off[b] and raises long_max[win_clip[b]] (NULL arrays: window b
+// starts at b * hop_samples and every window belongs to clip 0).
 template <int NMEL>
 __global__ void __launch_bounds__(NT) logmel_long_kernel(const float* __restrict__ pcm, long long hop_samples,
+                                                        const long long* __restrict__ win_off,
+                                                        const int* __restrict__ win_clip,
                                                         const MelTables<NMEL>* __restrict__ tab, const int* __restrict__ frame_lo,
                                                         const int* __restrict__ frame_hi, const int* __restrict__ out_row0,
                                                         unsigned int* __restrict__ long_max,
@@ -404,7 +408,7 @@ __global__ void __launch_bounds__(NT) logmel_long_kernel(const float* __restrict
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
 
     load_tables<NMEL>(tid, tab, s);
-    phase_load(tid, NT, pcm + (size_t)b * hop_samples, N_SAMPLES, f0, s.x);
+    phase_load(tid, NT, pcm + (win_off ? win_off[b] : (long long)b * hop_samples), N_SAMPLES, f0, s.x);
     __syncthreads();
 
     float2* wa = s.a[warp];
@@ -449,18 +453,23 @@ __global__ void __launch_bounds__(NT) logmel_long_kernel(const float* __restrict
         float mx = s.red[0][0];
 #pragma unroll
         for (int i = 1; i < NWARP; ++i) mx = fmaxf(mx, s.red[0][i]);
-        if (mx > -INFINITY) atomicMax(long_max, float_to_umono(mx));
+        if (mx > -INFINITY) atomicMax(long_max + (win_clip ? win_clip[b] : 0), float_to_umono(mx));
     }
 }
 
 // raise every value below the clip's floor (max - 8 in log10 units, compared after the bf16 rounding of the output, like
 // the floor pass of logmel_kernel).  It sees the output as a flat run of uint4, so one kernel serves both bin counts.
+// blockIdx.y = clip c, which owns the rows [clip_row[c], clip_row[c + 1]) (vec_per_row uint4 each) and the maximum
+// long_max[c] (clip_row NULL: one clip owning the whole run [0, n_vec)).
 __global__ void __launch_bounds__(256) logmel_floor_kernel(uint4* __restrict__ mel, long long n_vec,
+                                                          const long long* __restrict__ clip_row, int vec_per_row,
                                                           const unsigned int* __restrict__ long_max) {
-    const float floor_y = scaled_floor(umono_to_float(*long_max));
+    const int c = blockIdx.y;
+    const float floor_y = scaled_floor(umono_to_float(long_max[c]));
     const uint32_t floor_bf = pack_bf16x2(floor_y, floor_y);
     const float floor_bf_f = __uint_as_float(floor_bf << 16);
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n_vec; i += (long long)gridDim.x * blockDim.x) {
+    const long long v0 = clip_row ? clip_row[c] * vec_per_row : 0, v1 = clip_row ? clip_row[c + 1] * vec_per_row : n_vec;
+    for (long long i = v0 + (long long)blockIdx.x * blockDim.x + threadIdx.x; i < v1; i += (long long)gridDim.x * blockDim.x) {
         uint4 v = mel[i];
         uint32_t* w = reinterpret_cast<uint32_t*>(&v);
         bool changed = false;
@@ -562,8 +571,9 @@ int logmel_launch(const void* tables_dev, const float* pcm, int64_t pcm_stride, 
 }
 
 template <int NMEL>
-int logmel_long_launch(const void* tables_dev, const float* pcm_long, int64_t hop_samples, int32_t n_windows,
-                       const int32_t* frame_lo, const int32_t* frame_hi, const int32_t* out_row0, uint32_t* max_scratch,
+int logmel_long_launch(const void* tables_dev, const float* pcm_long, int64_t hop_samples, const int64_t* win_off,
+                       const int32_t* win_clip, int32_t n_windows, const int32_t* frame_lo, const int32_t* frame_hi,
+                       const int32_t* out_row0, int32_t n_clips, const int64_t* clip_row, uint32_t* max_scratch,
                        void* out_bf16_t, int64_t total_frames, int32_t out_t_row_off, cudaStream_t st) {
     static std::atomic<unsigned long long> attr_done{0};
     if (device_needs_setup(attr_done)) {
@@ -571,15 +581,17 @@ int logmel_long_launch(const void* tables_dev, const float* pcm_long, int64_t ho
                                            (int)sizeof(MelSmem<NMEL>)));
         mark_device_done(attr_done);
     }
-    TW_CUDA_CHECK(cudaMemsetAsync(max_scratch, 0, sizeof(uint32_t), st));     // below every real value in the ordered map
+    // zero is below every real value in the ordered map
+    TW_CUDA_CHECK(cudaMemsetAsync(max_scratch, 0, sizeof(uint32_t) * n_clips, st));
     logmel_long_kernel<NMEL><<<dim3(N_TILES, n_windows), NT, sizeof(MelSmem<NMEL>), st>>>(
-        pcm_long, (long long)hop_samples, (const MelTables<NMEL>*)tables_dev, frame_lo, frame_hi, out_row0, max_scratch,
-        (__nv_bfloat16*)out_bf16_t, out_t_row_off);
+        pcm_long, (long long)hop_samples, (const long long*)win_off, win_clip, (const MelTables<NMEL>*)tables_dev,
+        frame_lo, frame_hi, out_row0, max_scratch, (__nv_bfloat16*)out_bf16_t, out_t_row_off);
     TW_CUDA_CHECK(cudaGetLastError());
     const long long n_vec = (long long)total_frames * NMEL / 8;
     uint4* first = reinterpret_cast<uint4*>((__nv_bfloat16*)out_bf16_t + (size_t)out_t_row_off * NMEL);
-    const int blocks = (int)std::min<long long>((n_vec + 255) / 256, 148 * 8);
-    logmel_floor_kernel<<<blocks, 256, 0, st>>>(first, n_vec, max_scratch);
+    const int blocks = (int)std::max<long long>(1, std::min<long long>((n_vec / n_clips + 255) / 256, 148 * 8));
+    logmel_floor_kernel<<<dim3(blocks, n_clips), 256, 0, st>>>(first, n_vec, (const long long*)clip_row, NMEL / 8,
+                                                                max_scratch);
     TW_CUDA_CHECK(cudaGetLastError());
     return 0;
 }
@@ -639,10 +651,32 @@ extern "C" int tw_logmel_long_n(const void* tables_dev, const float* pcm_long, i
     if (n_windows == 0 || total_frames == 0) return 0;
     cudaStream_t st = (cudaStream_t)stream;
     return n_mels == 128
-        ? logmel_long_launch<128>(tables_dev, pcm_long, hop_samples, n_windows, frame_lo, frame_hi, out_row0, max_scratch,
-                                  out_bf16_t, total_frames, out_t_row_off, st)
-        : logmel_long_launch<80>(tables_dev, pcm_long, hop_samples, n_windows, frame_lo, frame_hi, out_row0, max_scratch,
-                                 out_bf16_t, total_frames, out_t_row_off, st);
+        ? logmel_long_launch<128>(tables_dev, pcm_long, hop_samples, nullptr, nullptr, n_windows, frame_lo, frame_hi,
+                                  out_row0, 1, nullptr, max_scratch, out_bf16_t, total_frames, out_t_row_off, st)
+        : logmel_long_launch<80>(tables_dev, pcm_long, hop_samples, nullptr, nullptr, n_windows, frame_lo, frame_hi,
+                                 out_row0, 1, nullptr, max_scratch, out_bf16_t, total_frames, out_t_row_off, st);
+}
+
+extern "C" int tw_logmel_long_multi(const void* tables_dev, const float* pcm, const int64_t* win_offset,
+                                    const int32_t* win_clip, int32_t n_windows, const int32_t* frame_lo,
+                                    const int32_t* frame_hi, const int32_t* out_row0, int32_t n_clips,
+                                    const int64_t* clip_row0, uint32_t* max_scratch, void* out_bf16_t,
+                                    int64_t total_frames, int32_t n_mels, void* stream) {
+    TW_REQUIRE(tables_dev && pcm && win_offset && win_clip && frame_lo && frame_hi && out_row0 && clip_row0 &&
+               max_scratch && out_bf16_t, "tw_logmel_long_multi: null argument");
+    TW_REQUIRE_N_MELS("tw_logmel_long_multi", n_mels);
+    if (tw::ensure_device(pcm)) return 1;
+    TW_REQUIRE(n_windows >= 0 && n_windows <= 65535, "tw_logmel_long_multi: %d windows out of range", n_windows);
+    TW_REQUIRE(n_clips >= 1 && n_clips <= 65535, "tw_logmel_long_multi: %d clips out of range", n_clips);
+    TW_REQUIRE(((uintptr_t)out_bf16_t & 15) == 0 && total_frames >= 0,
+               "tw_logmel_long_multi: the output must be 16-byte aligned");
+    if (n_windows == 0 || total_frames == 0) return 0;
+    cudaStream_t st = (cudaStream_t)stream;
+    return n_mels == 128
+        ? logmel_long_launch<128>(tables_dev, pcm, 1, win_offset, win_clip, n_windows, frame_lo, frame_hi, out_row0,
+                                  n_clips, clip_row0, max_scratch, out_bf16_t, total_frames, 0, st)
+        : logmel_long_launch<80>(tables_dev, pcm, 1, win_offset, win_clip, n_windows, frame_lo, frame_hi, out_row0,
+                                 n_clips, clip_row0, max_scratch, out_bf16_t, total_frames, 0, st);
 }
 
 extern "C" int tw_logmel_long(const void* tables_dev, const float* pcm_long, int64_t hop_samples, int32_t n_windows,

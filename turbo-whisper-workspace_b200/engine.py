@@ -15,7 +15,7 @@ import os
 
 import ctypes as C
 import threading
-from typing import Dict, List, Optional, Sequence
+from typing import Callable, Dict, List, Optional, Sequence, Union
 
 import numpy as np
 import torch
@@ -242,6 +242,91 @@ def init_rows(rows: torch.Tensor, max_len: int, g: Grammar, timestamps: bool, pr
         st["ts_hi"] = g.ts_begin + g.max_initial_ts
         st["begin"] = 1
     return tokens, forced, torch.from_numpy(st.view(np.int32).reshape(R, -1)), P
+
+
+def long_guard(frames: int) -> int:
+    """Seek iterations a long-form clip of ``frames`` mel frames may take before its loop counts as stuck (degenerate
+    timestamp output that never advances the seek)."""
+    return 64 + 4 * (int(frames) // N_FRAMES)
+
+
+class LongClip:
+    """One clip of a long-form call: its index in the call, frame count, device features, seek pointer, language
+    (-1 until detected on its first window), seek iterations run, generated ids (segments in order) and trace."""
+
+    def __init__(self, index: int, frames: int, feats, lang: int):
+        self.index, self.frames, self.feats, self.lang = index, int(frames), feats, lang
+        self.seek, self.iters = 0, 0
+        self.ids: List[int] = []
+        self.trace = {"iterations": []}
+
+
+class LongFormRows:
+    """Host bookkeeping of the long-form seek loop over many clips (no device work, unit-tested on the CPU): up to
+    ``capacity`` clips are active decode rows; a clip whose seek reaches its frame count leaves, and its row is
+    refilled at the next iteration from ``source`` (a callable returning ``(index, audio)`` or None when no clip is
+    pending) in the order the source hands clips out.  ``admit([(index, audio), ...]) -> [(frames, feats), ...]``
+    prepares the clips that enter at one refill together.  ``record``: keep every clip's seek-loop trace."""
+
+    def __init__(self, capacity: int, source: Callable[[], Optional[tuple]], admit: Callable[[list], list],
+                 lang: int = -1, record: bool = False):
+        if capacity < 1:
+            raise ValueError("a long-form call needs at least one decode row")
+        self.capacity, self.source, self.admit, self.lang, self.record = int(capacity), source, admit, lang, record
+        self.rows: List[LongClip] = []
+        self.done: Dict[int, LongClip] = {}
+        self.iterations = self.windows = 0
+        self._pending = True
+
+    def refill(self) -> List[LongClip]:
+        """Fill the free rows from the source; returns the active rows of the next iteration (empty: the call is over)
+        after counting the iteration against every row's guard."""
+        while self._pending and len(self.rows) < self.capacity:
+            items = []
+            while len(self.rows) + len(items) < self.capacity:
+                item = self.source()
+                if item is None:
+                    self._pending = False
+                    break
+                if item[0] in self.done or any(c.index == item[0] for c in self.rows) or \
+                        any(i == item[0] for i, _ in items):
+                    raise RuntimeError(f"long-form clip {item[0]} was handed out twice")
+                items.append(item)
+            if not items:
+                break
+            for (index, _), (frames, feats) in zip(items, self.admit(items)):
+                clip = LongClip(index, frames, feats, self.lang)
+                if clip.frames > 0:
+                    self.rows.append(clip)
+                else:
+                    clip.feats = None
+                    self.done[index] = clip
+        for c in self.rows:
+            c.iters += 1
+            if c.iters > long_guard(c.frames):
+                raise RuntimeError("whisper seek loop does not advance (degenerate timestamp output)")
+        if self.rows:
+            self.iterations += 1
+            self.windows += len(self.rows)
+        return list(self.rows)
+
+    def advance(self, clip: LongClip, segments: List[List[int]], adv: int, tokens: Optional[List[int]] = None,
+                beam: Optional[tuple] = None) -> None:
+        """Append one iteration's segments to ``clip`` and move its seek by ``adv`` frames; a clip whose seek reaches
+        its frame count leaves the active rows.  ``tokens`` (the decoder row) and ``beam`` (beam search: the search's
+        own (sum of log-probabilities, length) of the returned hypothesis) go to the trace."""
+        if self.record and tokens is not None:
+            entry = {"rows": [0], "seek": [clip.seek], "tokens": [list(tokens)]}
+            if beam is not None:
+                entry["beam"] = [beam]
+            clip.trace["iterations"].append(entry)
+        for sg in segments:
+            clip.ids.extend(sg)
+        clip.seek += adv
+        if clip.seek >= clip.frames:
+            self.rows.remove(clip)
+            clip.feats = None
+            self.done[clip.index] = clip
 
 
 class WhisperEngine:
@@ -1020,24 +1105,64 @@ class WhisperEngine:
 
     def generate_long_from_pcm(self, audio: np.ndarray, trace: Optional[dict] = None, **options) -> List[int]:
         """ONE clip longer than 30 s, un-chunked (the ASR pipeline without chunk_length_s,
-        $TF/pipelines/automatic_speech_recognition.py:446-454): features of the whole clip (tw_logmel_long) and HF's
-        long-form generate — the same seek loop as :meth:`generate`, over all n // 160 frames
-        ($TF/models/whisper/generation_whisper.py:654-658, :785-870); timestamps are mandatory (:1388-1394).  Sequential
-        by construction: one window is encoded and decoded per iteration.  Returns the generated ids (segments
-        concatenated; timestamp tokens restart in every 30 s segment, which `_decode_asr` undoes).
+        $TF/pipelines/automatic_speech_recognition.py:446-454): the one-clip call of :meth:`generate_long_batch`.
+        Returns the generated ids (segments concatenated; timestamp tokens restart in every 30 s segment, which
+        `_decode_asr` undoes).  ``trace`` receives the clip's seek-loop trace.
         ``options``: the generate options (see :meth:`generate`), checked before any device work; ``prompt_ids`` is
         prepended in every seek iteration (HF with condition_on_prev_tokens off)."""
-        opts = resolve_generate_options(self.dims, self.gen, long_form=True, **options)
+        # checked here as well so that an invalid call fails before anything else is touched
+        resolve_generate_options(self.dims, self.gen, long_form=True, **options)
+        traces = None if trace is None else {}
+        out = self.generate_long_batch([audio], trace=traces, **options)[0]
+        if trace is not None:
+            trace.update(traces[0])
+        return out
 
-        def run():
-            mel = self.logmel.long(audio)
+    def generate_long_batch(self, audios: Optional[Sequence[np.ndarray]] = None, *,
+                            source: Optional[Callable[[], Optional[tuple]]] = None, rows: Optional[int] = None,
+                            trace: Optional[dict] = None, **options) -> Union[List[List[int]], Dict[int, List[int]]]:
+        """Many un-chunked long-form clips decoded together: HF's batched long-form generate (every row has its own seek
+        pointer and frame count, $TF/models/whisper/generation_whisper.py:654-658, :785-870), with a clip's row refilled
+        by the next pending clip as soon as its seek reaches its frame count.  Up to ``rows`` (default and cap
+        max_batch // num_beams) clips are active; each iteration gathers the active rows' 30 s windows out of their
+        clips' whole-clip features in one launch (tw_gather_frames), encodes them and decodes them as one batch.  The
+        language of a clip is detected on its first window.
+        ``audios``: the clips (fp32 16 kHz), admitted longest first; returns their ids in input order.
+        ``source``: instead of ``audios``, a callable returning ``(index, audio)`` or None when no clip is pending
+        (several engine contexts may share one); returns {index: ids} of the clips this call took.
+        ``trace``: receives {index: seek-loop trace of that clip} (the format of :meth:`generate`'s trace).
+        ``options``: the generate options (see :meth:`generate`), checked before any device work."""
+        opts = resolve_generate_options(self.dims, self.gen, long_form=True, **options)
+        if (audios is None) == (source is None):
+            raise ValueError("generate_long_batch takes either `audios` or `source`")
+        if audios is not None:
+            order = sorted(range(len(audios)), key=lambda i: -int(np.asarray(audios[i]).size))
+            pending = iter([(i, audios[i]) for i in order])
+            source = lambda: next(pending, None)
+
+        staging: list = []
+
+        def admit(items):
+            # the clips entering together: one H2D copy, one log-mel and one floor launch; the staging buffers live
+            # until the next iteration's device-to-host copy has passed them
+            feats, keep = self.logmel.long_many([a for _, a in items])
+            staging.append(keep)
             self.stats["launches"] += 2
-            self.stats["h2d_bytes"] += int(np.asarray(audio).size) * 4
-            return self._seek(1, opts, trace=trace, long_mel=mel)[0]
+            self.stats["h2d_bytes"] += int(keep[0].numel()) * 4
+            return [(int(f.shape[0]), f) for f in feats]
+
+        cap = max(1, self.max_batch // opts.num_beams)
+        book = LongFormRows(min(cap, int(rows or cap)), source, admit, opts.lang_id, record=trace is not None)
         if self.stream is not None:
             with torch.cuda.stream(self.stream):
-                return run()
-        return run()
+                self._seek_long(book, opts, staging)
+        else:
+            self._seek_long(book, opts, staging)
+        if trace is not None:
+            trace.update({i: dict(c.trace, langs=[c.lang]) for i, c in book.done.items()})
+        if audios is not None:
+            return [book.done[i].ids for i in range(len(audios))]
+        return {i: c.ids for i, c in book.done.items()}
 
     def _strip(self, row: List[int]) -> List[int]:
         """generate_with_fallback's pad / eos stripping ($TF/...generation_whisper.py:1063-1086)."""
@@ -1076,22 +1201,93 @@ class WhisperEngine:
         if long_mel is not None and B != 1:
             raise ValueError("long-form generate takes one clip, needs timestamps and has no token timestamps")
         opts = resolve_generate_options(self.dims, self.gen, long_form=long_mel is not None, **options)
-        return self._seek(B, opts, trace=trace, num_frames=num_frames, long_mel=long_mel)
+        if long_mel is None:
+            return self._seek(B, opts, trace=trace, num_frames=num_frames)
+        clip = iter([(0, long_mel)])
+        book = LongFormRows(1, lambda: next(clip, None), lambda items: [(int(m.shape[0]), m) for _, m in items],
+                            opts.lang_id, record=trace is not None)
+        self._seek_long(book, opts)
+        if trace is not None:
+            trace.update(book.done[0].trace, langs=[book.done[0].lang])
+        return [book.done[0].ids]
+
+    def _decode_windows(self, n: int, mel: torch.Tensor, langs: List[int], opts: GenerateOptions,
+                        frames_keep: Optional[List[int]] = None) -> List[List[int]]:
+        """One seek iteration's device work for n windows whose time-major features are in ``mel``: encode, language
+        detection where ``langs[i]`` is -1 (``langs`` is updated in place), greedy decode or beam search.  Returns the
+        decoder rows (prompt included).  ``frames_keep``: token timestamps on (see :meth:`decode_beams`)."""
+        gen, timestamps, prompt_ids = self.gen, opts.timestamps, opts.prompt_ids
+        self.encode(n, mel)
+
+        def prompts():
+            return torch.tensor([[gen.decoder_start_token_id, langs[i], opts.task_id] for i in range(n)], dtype=torch.int32)
+        if (opts.num_beams > 1 or prompt_ids is not None) and any(v < 0 for v in langs):
+            # language detection first (one decoder position), as detect_language does before generate
+            first = self.decode(n, prompts(), n_steps=1, timestamps=timestamps)[:, 1].cpu().tolist()
+            for i in range(n):
+                if langs[i] < 0:
+                    langs[i] = int(first[i])
+        pr = prompts()
+        if opts.num_beams > 1:
+            best = self.decode_beams(n, pr, opts.num_beams, timestamps=timestamps, frames_keep=frames_keep,
+                                     prompt_ids=prompt_ids).cpu().tolist()
+            toks = [self.prompt_row(prompt_ids, pr[i], timestamps) + best[i] for i in range(n)]
+        else:
+            self._align_on = frames_keep is not None
+            try:
+                toks = self.decode(n, pr, timestamps=timestamps, prompt_ids=prompt_ids).cpu().tolist()
+            finally:
+                self._align_on = False
+        self.stats["d2h_bytes"] += n * self.max_len * 4
+        for i in range(n):
+            if langs[i] < 0:
+                langs[i] = toks[i][1]
+        return toks
+
+    def _seek_long(self, book: LongFormRows, opts: GenerateOptions, staging: Optional[list] = None) -> None:
+        """The long-form seek loop over the clips of ``book`` with the options already resolved.  ``staging``: buffers
+        of the clips' admission, released once an iteration's device-to-host copy has passed their launches."""
+        ts_begin, P = self.gen.timestamp_begin, opts.prompt_len
+        iters0, windows0 = book.iterations, book.windows
+        with torch.cuda.device(self.device):
+            while True:
+                rows = book.refill()
+                if not rows:
+                    break
+                n = len(rows)
+                nfr = [min(c.frames - c.seek, N_FRAMES) for c in rows]
+                # the window [seek, seek + 3000) of every row's whole-clip features, zeros past the clip's last frame
+                ops.gather_frames([c.feats for c in rows], [c.frames for c in rows], [c.seek for c in rows], self.mel_s,
+                                  window=N_FRAMES, row_off=1)
+                self.stats["launches"] += 1
+                self.stats["h2d_bytes"] += n * 16
+                langs = [c.lang for c in rows]
+                toks = self._decode_windows(n, self.mel_s, langs, opts)
+                if staging:
+                    staging.clear()      # the token copy above waited for every launch of this iteration
+                beam = self.last_beam if opts.num_beams > 1 else None
+                for i, c in enumerate(rows):
+                    c.lang = langs[i]
+                    segs, adv = retrieve_segment(self._strip(toks[i][P:]), nfr[i], ts_begin)
+                    book.advance(c, segs, adv, toks[i], None if beam is None else
+                                 (float(beam["sum_logprob"][i]), int(beam["length"][i])))
+        self.stats["long_iterations"] = self.stats.get("long_iterations", 0) + book.iterations - iters0
+        self.stats["long_windows"] = self.stats.get("long_windows", 0) + book.windows - windows0
+        self.stats["long_mean_rows"] = self.stats["long_windows"] / max(1, self.stats["long_iterations"])
 
     def _seek(self, B: int, opts: GenerateOptions, trace: Optional[dict] = None,
-              num_frames: Optional[Sequence[int]] = None, long_mel: Optional[torch.Tensor] = None) -> List[List[int]]:
-        """The seek loop of :meth:`generate` with the options already resolved."""
-        gen = self.gen
-        timestamps, num_beams, prompt_ids, P = opts.timestamps, opts.num_beams, opts.prompt_ids, opts.prompt_len
+              num_frames: Optional[Sequence[int]] = None) -> List[List[int]]:
+        """The short-form seek loop of :meth:`generate` with the options already resolved."""
+        num_beams, P = opts.num_beams, opts.prompt_len
         if opts.token_timestamps:
             if num_frames is None or len(num_frames) != B:
                 raise ValueError("token_timestamps needs num_frames for every row")
             self.enable_alignment()
         ts_out: List[List[float]] = [[] for _ in range(B)]
         ts_raw: List[List[float]] = [[] for _ in range(B)]
-        ts_begin = gen.timestamp_begin
+        ts_begin = self.gen.timestamp_begin
         seek = [0] * B
-        max_frames = [N_FRAMES] * B if long_mel is None else [int(long_mel.shape[0])]
+        max_frames = [N_FRAMES] * B
         langs = [opts.lang_id] * B
         out: List[List[int]] = [[] for _ in range(B)]
         it = 0
@@ -1112,15 +1308,7 @@ class WhisperEngine:
                 rows = [b for b in range(B) if seek[b] < max_frames[b]]
                 nfr = {b: min(max_frames[b] - seek[b], N_FRAMES) for b in rows}
                 n = len(rows)
-                if long_mel is not None:
-                    # the window [seek, seek + 3000) of the whole-clip features, zeros past the clip's last frame
-                    # (device-to-device copies: data movement, no arithmetic)
-                    k = nfr[0]
-                    self.mel_s[0, 1:1 + k].copy_(long_mel[seek[0]:seek[0] + k])
-                    if k < N_FRAMES:
-                        self.mel_s[0, 1 + k:1 + N_FRAMES].zero_()
-                    mel = self.mel_s
-                elif it == 1:
+                if it == 1:
                     mel = self.mel_t       # seek = 0 for every row: the window is the clip itself
                 else:
                     ops.shift_frames(self.mel_t, self.mel_s,
@@ -1128,29 +1316,11 @@ class WhisperEngine:
                                      src_row=torch.tensor(rows, dtype=torch.int32, device=self.device))
                     self.stats["launches"] += 1
                     mel = self.mel_s
-                self.encode(n, mel)
-                prompts = torch.tensor([[gen.decoder_start_token_id, langs[b], opts.task_id] for b in rows],
-                                       dtype=torch.int32)
-                if (num_beams > 1 or prompt_ids is not None) and any(langs[b] < 0 for b in rows):
-                    # language detection first (one decoder position), as detect_language does before generate
-                    first = self.decode(n, prompts, n_steps=1, timestamps=timestamps)[:, 1].cpu().tolist()
-                    for i, b in enumerate(rows):
-                        if langs[b] < 0:
-                            langs[b] = int(first[i])
-                    prompts = torch.tensor([[gen.decoder_start_token_id, langs[b], opts.task_id] for b in rows],
-                                           dtype=torch.int32)
-                if num_beams > 1:
-                    best = self.decode_beams(n, prompts, num_beams, timestamps=timestamps,
-                                             frames_keep=frames_keep(rows) if opts.token_timestamps else None,
-                                             prompt_ids=prompt_ids).cpu().tolist()
-                    toks = [self.prompt_row(prompt_ids, prompts[i], timestamps) + best[i] for i in range(n)]
-                else:
-                    self._align_on = opts.token_timestamps
-                    try:
-                        toks = self.decode(n, prompts, timestamps=timestamps, prompt_ids=prompt_ids).cpu().tolist()
-                    finally:
-                        self._align_on = False
-                self.stats["d2h_bytes"] += n * self.max_len * 4
+                row_langs = [langs[b] for b in rows]
+                toks = self._decode_windows(n, mel, row_langs, opts,
+                                            frames_keep(rows) if opts.token_timestamps else None)
+                for i, b in enumerate(rows):
+                    langs[b] = row_langs[i]
                 tok_frames = None
                 if opts.token_timestamps and num_beams > 1:
                     tok_frames = self.last_beam_frames
@@ -1160,8 +1330,6 @@ class WhisperEngine:
                     trace.setdefault("iterations", []).append({"rows": list(rows), "seek": [seek[b] for b in rows],
                                                                "tokens": [list(t) for t in toks]})
                 for i, b in enumerate(rows):
-                    if langs[b] < 0:
-                        langs[b] = toks[i][1]
                     s = self._strip(toks[i][P:])
                     segs, adv = retrieve_segment(s, nfr[b], ts_begin)
                     if tok_frames is not None:

@@ -107,6 +107,43 @@ class LogMel:
             torch.cuda.current_stream(self.device).synchronize()      # `pcm` / `ints` are freed when this returns
         return out
 
+    def long_many(self, audios):
+        """Whole-clip features of several clips: ONE host-to-device copy of their concatenated buffers
+        (:func:`longform_buffer`), one tw_logmel_long_multi launch and its floor launch, every clip with its own
+        max - 8 clamp — bit-identical to :meth:`long` per clip.  Returns (features, staging): cuda bf16
+        [n // 160, n_mels] per clip (views of one buffer) and the device / pinned staging tensors, which the caller
+        keeps until the stream has passed the launch (no synchronisation here)."""
+        lib = _lib.load()
+        plans = [longform_plan(int(np.asarray(a).size)) for a in audios]
+        sizes = [max(p["buffer_samples"], int(np.asarray(a).size) + 200) for a, p in zip(audios, plans)]
+        starts = np.concatenate([[0], np.cumsum(sizes)]).astype(np.int64)
+        rows = np.concatenate([[0], np.cumsum([p["frames"] for p in plans])]).astype(np.int64)
+        host = torch.empty(int(starts[-1]), dtype=torch.float32, pin_memory=True)
+        hv = host.numpy()
+        off, clip, lo, hi, row0 = [], [], [], [], []
+        for c, (a, p) in enumerate(zip(audios, plans)):
+            hv[starts[c]:starts[c + 1]] = longform_buffer(np.asarray(a, dtype=np.float32).reshape(-1), p)
+            off += [int(starts[c]) + k * p["hop_samples"] for k in range(len(p["lo"]))]
+            clip += [c] * len(p["lo"])
+            lo += p["lo"]
+            hi += p["hi"]
+            row0 += [int(rows[c]) + r for r in p["row0"]]
+        ints = torch.tensor([clip, lo, hi, row0], dtype=torch.int32).pin_memory()
+        longs = torch.from_numpy(np.concatenate([np.asarray(off, dtype=np.int64), rows])).pin_memory()
+        with torch.cuda.device(self.device):
+            pcm = host.to(self.device, non_blocking=True)
+            ints_d = ints.to(self.device, non_blocking=True)
+            longs_d = longs.to(self.device, non_blocking=True)
+            mx = torch.empty(len(audios), dtype=torch.int32, device=self.device)
+            out = torch.empty(int(rows[-1]), self.n_mels, dtype=torch.bfloat16, device=self.device)
+            nw = len(off)
+            check(lib.tw_logmel_long_multi(_ptr(self.tables), _ptr(pcm), _ptr(longs_d), _ptr(ints_d[0]), nw,
+                                           _ptr(ints_d[1]), _ptr(ints_d[2]), _ptr(ints_d[3]), len(audios),
+                                           _ptr(longs_d[nw:]), _ptr(mx), _ptr(out), int(rows[-1]), self.n_mels,
+                                           _stream()), "tw_logmel_long_multi")
+        feats = [out[int(rows[c]):int(rows[c + 1])] for c in range(len(audios))]
+        return feats, (host, ints, longs, pcm, ints_d, longs_d, mx, out)
+
 
 LONG_HOP_FRAMES = 2997      # frames 2 .. 2998 of a 30 s window do not touch its reflect padding
 
@@ -212,6 +249,27 @@ def shift_frames(src, dst, seek, src_row=None, frames: int = N_FRAMES, row_off: 
     with torch.cuda.device(src.device):
         check(lib.tw_shift_frames(_ptr(src), _ptr(dst), _ptr(src_row), _ptr(seek), B, frames, src.shape[2],
                                   src.stride(0), row_off, _stream()), "tw_shift_frames")
+    return dst
+
+
+def gather_frames(feats, frames, seek, dst, window: int = N_FRAMES, row_off: int = 1):
+    """dst[b, row_off+t] = feats[b][seek[b]+t] for t < min(window, frames[b] - seek[b]), zeros up to ``window``: one
+    launch (tw_gather_frames) over rows that each read their own clip's time-major bf16 features [frames, cols].
+    ``frames`` / ``seek``: host ints per row; ``dst``: bf16 [>= rows, >= row_off + window, cols]."""
+    lib = _lib.load()
+    _need_cuda(dst, *feats)
+    B = len(feats)
+    cols = dst.shape[2]
+    assert dst.dtype == torch.bfloat16 and dst.stride(2) == 1 and dst.stride(1) == cols and dst.shape[0] >= B
+    assert dst.shape[1] >= row_off + window and len(frames) == len(seek) == B
+    for f, n in zip(feats, frames):
+        assert f.dtype == torch.bfloat16 and f.is_contiguous() and f.device == dst.device and f.shape[-1] == cols
+        assert f.shape[0] >= n and f.data_ptr() % 16 == 0
+    with torch.cuda.device(dst.device):
+        ptrs = torch.tensor([f.data_ptr() for f in feats], dtype=torch.int64).to(dst.device)
+        ints = torch.tensor([list(frames), list(seek)], dtype=torch.int32).to(dst.device)
+        check(lib.tw_gather_frames(_ptr(ptrs), _ptr(ints[0]), _ptr(ints[1]), B, window, cols, _ptr(dst), dst.stride(0),
+                                   row_off, _stream()), "tw_gather_frames")
     return dst
 
 

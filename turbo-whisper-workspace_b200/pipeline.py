@@ -256,8 +256,10 @@ class B200WhisperPipeline:
                  scheduler=None, contexts_per_device: int = 4):
         """``scheduler``: any object with ``run(clips, task=, language=) -> token rows`` and ``last_stats``; every other
         generate option reaches ``run`` (and ``run_long``) as a keyword only when it differs from its default, which a
-        scheduler forwards to its engines untouched.  Defaults to a :class:`WindowScheduler` with one GPU engine per
-        entry of ``devices``."""
+        scheduler forwards to its engines untouched.  Un-chunked long-form inputs (> 30 s without chunk_length_s) go to
+        ``run_long(audio, **kw) -> token row``, one call per input; a scheduler may also provide
+        ``run_long_many(audios, **kw) -> token rows in input order``, which then receives all long inputs of a call
+        that has two or more.  Defaults to a :class:`WindowScheduler` with one GPU engine per entry of ``devices``."""
         self.dims = dims
         self.tokenizer = tokenizer
         self.generation = generation or GenerationSettings()
@@ -353,7 +355,13 @@ class B200WhisperPipeline:
             token_rows = [r for r, _ in token_rows]
         # long-form input is only reached with timestamps on and without word timestamps, so run_kw holds nothing that
         # long-form generate refuses
-        long_rows = {i: self.scheduler.run_long(p["longform"], **run_kw) for i, p in enumerate(prepared) if "longform" in p}
+        long_idx = [i for i, p in enumerate(prepared) if "longform" in p]
+        if len(long_idx) >= 2 and hasattr(self.scheduler, "run_long_many"):
+            # one batched seek loop over all long inputs, spread over the engine contexts
+            long_rows = dict(zip(long_idx, self.scheduler.run_long_many([prepared[i]["longform"] for i in long_idx],
+                                                                        **run_kw)))
+        else:
+            long_rows = {i: self.scheduler.run_long(prepared[i]["longform"], **run_kw) for i in long_idx}
         t2 = time.perf_counter()
         self.last_token_rows = token_rows      # the engines' rows of this call, window order (bench.py's output check)
         results, w0 = [], 0

@@ -96,6 +96,43 @@ class WorkQueue:
             return a, b
 
 
+def long_order(lengths: Sequence[int]) -> List[int]:
+    """Indices of long-form clips, longest first (ties in input order): the order in which clips are admitted, so
+    the longest seek loops start first and the short ones fill the rows that free up near the end."""
+    return sorted(range(len(lengths)), key=lambda i: (-int(lengths[i]), i))
+
+
+def long_partition(lengths: Sequence[int], n_workers: int) -> List[List[int]]:
+    """Deterministic length-balanced plan of long-form clips over workers: longest first, each clip to the worker with
+    the least assigned audio so far (ties: the lowest worker).  Every rank computes the same plan from the lengths."""
+    if n_workers < 1:
+        raise ValueError("n_workers must be >= 1")
+    load, plan = [0] * n_workers, [[] for _ in range(n_workers)]
+    for i in long_order(lengths):
+        w = min(range(n_workers), key=lambda k: (load[k], k))
+        plan[w].append(i)
+        load[w] += int(lengths[i])
+    return plan
+
+
+class LongQueue:
+    """Pending long-form clips of one call shared by engine contexts: ``take`` hands out ``(index, audio)`` (or None
+    once the queue is empty or the call has failed), each clip exactly once."""
+
+    def __init__(self, audios: Sequence[np.ndarray], order: Sequence[int]):
+        self.audios, self.order, self.pos = audios, list(order), 0
+        self.lock = threading.Lock()
+        self.failed = False
+
+    def take(self) -> Optional[Tuple[int, np.ndarray]]:
+        with self.lock:
+            if self.failed or self.pos >= len(self.order):
+                return None
+            i = self.order[self.pos]
+            self.pos += 1
+            return i, self.audios[i]
+
+
 class WindowScheduler:
     """One process; ``contexts_per_device`` engine contexts per local GPU, each driven by its own host thread and
     CUDA stream and sharing one copy of the weights.  All contexts of all devices pull micro-batches of consecutive
@@ -121,6 +158,7 @@ class WindowScheduler:
                                               own_stream=self.contexts_per_device > 1))
             self.engines.append(ctxs)
         self.last_stats: Dict[str, Any] = {}
+        self.last_long_stats: Dict[str, Any] = {}      # the last run_long_many call
 
     @property
     def flat_engines(self) -> List[Any]:
@@ -187,6 +225,51 @@ class WindowScheduler:
         clip's frames, so it runs on one engine context (``engine.generate_long_from_pcm(audio, **generate_kwargs)``)."""
         return self.engines[0][0].generate_long_from_pcm(audio, **generate_kwargs)
 
+    def run_long_many(self, audios: Sequence[np.ndarray], **generate_kwargs) -> List[List[int]]:
+        """Token rows of many un-chunked long-form clips, in input order.  The clips are dealt longest first over the
+        engine contexts (contexts of different devices first, as :meth:`run`), one each; the rest wait in ONE shared
+        queue, from which every context refills a decode row as soon as one of its clips finishes
+        (``engine.generate_long_batch(source=..., rows=...)``).  A context holds about ceil(n / contexts) active rows,
+        capped at max_batch // num_beams.  ``generate_kwargs`` are forwarded untouched."""
+        t0 = time.perf_counter()
+        n = len(audios)
+        order = [self.engines[d][c] for c in range(self.contexts_per_device) for d in range(len(self.devices))]
+        n_ctx = min(len(order), n)
+        results: List[Optional[List[int]]] = [None] * n
+        if n_ctx == 0:
+            self.last_long_stats = {"clips": 0, "contexts": 0, "rows": 0, "seconds": time.perf_counter() - t0}
+            return []
+        cap = microbatch_size(min(e.max_batch for e in order), generate_kwargs.get("num_beams", 1))
+        rows = min(cap, -(-n // n_ctx))
+        clips = long_order([np.asarray(a).size for a in audios])
+        queue = LongQueue(audios, clips[n_ctx:])
+        errors: List[BaseException] = []
+
+        def work(engine, first):
+            seed = iter([(first, audios[first])])
+
+            def source():
+                return next(seed, None) or queue.take()
+            try:
+                for i, ids in engine.generate_long_batch(source=source, rows=rows, **generate_kwargs).items():
+                    results[i] = ids
+            except BaseException as ex:  # surfaced on the calling thread
+                queue.failed = True
+                errors.append(ex)
+
+        threads = [threading.Thread(target=work, args=(order[k], clips[k]), daemon=True) for k in range(n_ctx)]
+        if len(threads) == 1:
+            threads[0].run()
+        else:
+            for t in threads:
+                t.start()
+            for t in threads:
+                t.join()
+        if errors:
+            raise errors[0]
+        self.last_long_stats = {"clips": n, "contexts": n_ctx, "rows": rows, "seconds": time.perf_counter() - t0}
+        return results
+
     def close(self):
         self.engines = []
 
@@ -249,6 +332,30 @@ class DistributedWindowScheduler:
         if hasattr(self.engine, "run_long"):
             return self.engine.run_long(audio, **generate_kwargs)
         return self.engine.generate_long_from_pcm(audio, **generate_kwargs)
+
+    def run_long_many(self, audios: Sequence[np.ndarray], **generate_kwargs) -> List[List[int]]:
+        """Token rows of many un-chunked long-form clips, in input order.  Every rank computes the same
+        :func:`long_partition` of the clips by length, runs its share on its local :class:`WindowScheduler` (or
+        engine), and the rows are gathered with ``all_gather_object``.  Must be called by every rank with the same
+        clips; ``generate_kwargs`` are forwarded untouched."""
+        mine = long_partition([np.asarray(a).size for a in audios], self.world_size)[self.rank]
+        local: List[List[int]] = []
+        if mine:
+            clips = [audios[i] for i in mine]
+            if hasattr(self.engine, "run_long_many"):
+                local = self.engine.run_long_many(clips, **generate_kwargs)
+            else:
+                local = self.engine.generate_long_batch(clips, **generate_kwargs)
+        pairs = list(zip(mine, local))
+        if self.world_size > 1:
+            import torch.distributed as dist
+            buckets: List[Any] = [None] * self.world_size
+            dist.all_gather_object(buckets, pairs, group=self.group)
+            pairs = [p for b in buckets for p in b]
+        rows: List[Optional[List[int]]] = [None] * len(audios)
+        for i, ids in pairs:
+            rows[i] = ids
+        return rows
 
     def close(self):
         if hasattr(self.engine, "close"):
